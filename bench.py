@@ -4,6 +4,7 @@ POMO = 100, x8 augmentation, synthetic uniform instances, seeded random-init wei
 (BASELINE.json configs[1]; the released checkpoints are not available offline).
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path
+    python bench.py ... --dump-outputs DIR                   # + the last timed step's costs, rewards and tours as .npy
     python bench.py --impl reference --steps K --warmup W    # the reference algorithm on host cores
                                                              # (CPU oracle port; the reference is Python
                                                              # and cannot travel to the GPU box)
@@ -43,6 +44,7 @@ FP32_PEAK_TFLOPS = SMS * LANES * 2 * 1.965e9 / 1e12
 PIPE_TENSOR_FLOP = 41536 * 2 * 3
 PIPE_FMA_OPS = 2 * (128 + 492 + 492 + 96 + 164) + 3232 + 656 + 303 + 3780 + 1200
 PIPE_XU_OPS = 8 * 101 + 4 * 41
+DUMP_BYTES = 64 << 20                  # --dump-outputs: all arrays together
 
 
 def ncu_traffic():
@@ -268,7 +270,8 @@ def run_ours(args):
         ev0.record()
         costs = []
         for s in range(args.warmup, total_steps):
-            costs.append(fn(s)[1].mean())
+            out = fn(s)
+            costs.append(out[1].mean())
         ev1.record()
         barrier()
         ms = ev0.elapsed_time(ev1)
@@ -279,10 +282,12 @@ def run_ours(args):
             t = torch.tensor([ms], device=dev)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             ms = float(t.item())
-        return ms, launches, events, clocks, float(torch.stack(costs).mean())
+        return ms, launches, events, clocks, float(torch.stack(costs).mean()), out
 
-    ms_dev, launches, events, clocks, mean_cost = timed(step_device)
-    ms_e2e, _, _, clocks_e2e, _ = timed(step_e2e)
+    ms_dev, launches, events, clocks, mean_cost, last = timed(step_device)
+    dump = sample_outputs(*last) if args.dump_outputs and rank == 0 else None
+    del last
+    ms_e2e, _, _, clocks_e2e, _, _ = timed(step_e2e)
 
     # rollout-kernel roofline numbers from the CUDA events recorded around each elg_rollout launch
     k_ms, aug_steps, row_steps, T_list = 0.0, 0, 0, []
@@ -382,9 +387,34 @@ def run_ours(args):
                                                     "TF32), %.1f s, T=%d; informative (SURVEY 8d), not the baseline" % (n_eager, dev, dt_g, T_g)}
             except Exception as e:
                 line["ref_cuda_eager"] = {"error": repr(e)[:200]}
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def sample_outputs(no_aug_cost, aug_cost, tours, rewards):
+    """What solve_batch() returned in the last timed step, as host arrays for --dump-outputs.  The costs are kept whole.
+    Tours and rewards of more aug-instances than fit in DUMP_BYTES are cut to a fixed seeded sample of aug-instances: a
+    prefix of one seeded permutation, so the sample of a longer rollout is a subset of that of a shorter one.  `rows`
+    lists the sampled aug-instances (row a * batch + i = augmentation a of instance i)."""
+    import torch
+    A, M, T = tours.shape
+    room = DUMP_BYTES - 2 * 4 * no_aug_cost.numel()
+    k = min(A, room // (4 * M * (T + 1) + 8))
+    rows = torch.randperm(A, generator=torch.Generator().manual_seed(0))[:k].sort()[0]
+    idx = rows.to(tours.device)
+    return {"no_aug_cost": no_aug_cost.float().cpu().numpy(), "aug_cost": aug_cost.float().cpu().numpy(),
+            "rewards": rewards[idx].float().cpu().numpy(), "tours": tours[idx].float().cpu().numpy(),
+            "rows": rows.double().numpy()}
+
+
+def write_outputs(dirname, arrays):
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------- training workload
@@ -609,7 +639,11 @@ def main():
     ap.add_argument("--train-batch", type=int, default=64, help="training instances per step per GPU")
     ap.add_argument("--chunk-steps", type=int, default=128, help="rollout steps per decode-backward launch")
     ap.add_argument("--cpu-train-sample", type=int, default=2, help="instances in the CPU training-step sample")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's instances) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "inference"):
+        ap.error("--dump-outputs applies to the CUDA inference path (--impl ours --workload inference)")
     if args.warmup < 3 and args.impl == "ours" and not os.environ.get("ELG_BENCH_ALLOW_SHORT"):
         args.warmup = 3
     if args.workload == "train":
