@@ -28,8 +28,9 @@ int check_desc(const elg_model_desc* d) {
               "kernels are built for local_att 32/4/8 (got %d/%d/%d)", d->local_emb, d->local_heads, d->local_qkv);
   ELG_REQUIRE(d->layers >= 1 && d->layers <= ELG_MAX_LAYERS, ELG_EUNSUPPORTED, "encoder_layer_num %d not in [1,%d]", d->layers, ELG_MAX_LAYERS);
   ELG_REQUIRE(d->ff > 0 && d->ff % 128 == 0, ELG_EUNSUPPORTED, "ff_hidden_dim must be a positive multiple of 128");
-  int kt = d->local_k + (d->problem == ELG_CVRP ? 1 : 0);
-  ELG_REQUIRE(d->local_k >= 1 && kt <= KT_MAX, ELG_EUNSUPPORTED, "local_size %d outside [1,%d]", d->local_k, KT_MAX - 1);
+  const int k_max = KT_MAX - (d->problem == ELG_CVRP ? 1 : 0);      // the cvrp local sequence also holds the depot
+  ELG_REQUIRE(d->local_k >= 1 && d->local_k <= k_max, ELG_EUNSUPPORTED, "local_size %d outside [1,%d] for %s", d->local_k,
+              k_max, d->problem == ELG_CVRP ? "cvrp" : "tsp");
   ELG_REQUIRE(d->flags & ELG_FLAG_DISTANCE_PENALTY, ELG_EUNSUPPORTED,
               "distance_penalty=False is not implemented (ensemble may be on or off)");
   return ELG_OK;

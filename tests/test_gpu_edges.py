@@ -4,6 +4,7 @@ import torch
 
 from helpers import compare_tours
 from oracle import elg_oracle as O
+from test_gpu_model_config import assert_kernel, expected_kernel, launched_kernels
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -24,17 +25,26 @@ def _run(kind, N, M, n, aug, gain=3.0, seed=1, attention="fp32"):
     ref_t, _, ref_r = O.rollout(W, prob, M, perm, "greedy")
     handle = engine.ModelHandle(kind, mp, sd, DEV, attention=attention)
     batch = engine.encode(handle, prob.xy.to(DEV), None if prob.demand is None else prob.demand.to(DEV))
-    tours16, reward, _, n_steps = engine.rollout(batch, M, perm.tolist())
+    (tours16, reward, _, n_steps), kernels = launched_kernels(lambda: engine.rollout(batch, M, perm.tolist()))
     T = int(n_steps.max())
-    return tours16[:, :, :T].long().cpu(), reward.cpu(), ref_t, ref_r, prob
+    return tours16[:, :, :T].long().cpu(), reward.cpu(), ref_t, ref_r, prob, kernels
+
+
+def _kernel(kind, N, M, n, aug, attention):
+    """The decode kernel the released configuration (local_size 40 / 30) runs this shape on."""
+    from elg_b200.synth import DEFAULT_MODEL_PARAMS
+    return expected_kernel(kind, DEFAULT_MODEL_PARAMS[kind]["local_size"][0], N + (1 if kind == "cvrp" else 0), attention, True,
+                           n * aug, M, torch.cuda.get_device_properties(DEV).multi_processor_count)
 
 
 @pytest.mark.parametrize("kind,N,M,n,aug", [
     ("cvrp", 5, 1, 3, 1),       # one POMO row, tiny instance (local neighbourhood smaller than k)
     ("cvrp", 7, 5, 2, 8),       # M not a multiple of 4
     ("cvrp", 45, 45, 1, 8),     # k = 40 < N: neighbour list truncation
-    ("cvrp", 111, 9, 1, 1),     # largest resident instance (N+1 = 112)
-    ("cvrp", 112, 9, 1, 1),     # smallest streaming instance (N+1 = 113)
+    ("cvrp", 107, 9, 1, 1),     # largest resident instance at k = 40 (N+1 = 108)
+    ("cvrp", 108, 9, 1, 1),     # smallest streaming instance at k = 40 (N+1 = 109)
+    ("cvrp", 111, 9, 1, 1),     # N+1 = 112: streaming at k = 40, the largest node count the resident kernels have slots for
+    ("cvrp", 112, 9, 1, 1),     # N+1 = 113: beyond the resident kernels' node slots
     ("tsp", 4, 4, 2, 1),
     ("tsp", 31, 31, 1, 8),      # k = 30 = N-1
     ("tsp", 112, 7, 1, 1),      # resident limit
@@ -42,7 +52,8 @@ def _run(kind, N, M, n, aug, gain=3.0, seed=1, attention="fp32"):
     ("tsp", 129, 129, 1, 1),    # 5 mask words, M > 128
 ])
 def test_ragged_shapes_match_oracle(kind, N, M, n, aug):
-    tours, reward, ref_t, ref_r, prob = _run(kind, N, M, n, aug)
+    tours, reward, ref_t, ref_r, prob, kernels = _run(kind, N, M, n, aug)
+    assert_kernel(kernels, _kernel(kind, N, M, n, aug, "fp32"))
     frac, same = compare_tours(tours, ref_t)
     assert frac >= 0.9, frac
     assert ((reward - ref_r).abs() / ref_r.abs())[same].max() < 1e-4
@@ -63,7 +74,8 @@ def test_ragged_shapes_match_oracle(kind, N, M, n, aug):
 ])
 def test_ragged_shapes_streamed_tensor_core_kernel(kind, N, M, n, aug):
     """Large instances on the streamed tensor-core kernel (rollout_stc.cu; attention = auto) against the oracle."""
-    tours, reward, ref_t, ref_r, prob = _run(kind, N, M, n, aug, attention="auto")
+    tours, reward, ref_t, ref_r, prob, kernels = _run(kind, N, M, n, aug, attention="auto")
+    assert_kernel(kernels, "rollout_stc_kernel<%d>" % (1 if kind == "cvrp" else 0))
     frac, same = compare_tours(tours, ref_t)
     assert frac >= 0.9, frac
     assert ((reward - ref_r).abs() / ref_r.abs())[same].max() < 1e-4
@@ -83,6 +95,8 @@ def test_streamed_kernel_is_the_one_that_runs():
     assert int(_lib.lib.elg_rollout_ws_bytes(desc, 8, 200, 201)) > 0 and int(_lib.lib.elg_rollout_ws_bytes(desc, 8, 100, 101)) == 0
     a = _run("cvrp", 150, 60, 1, 8, attention="auto")
     b = _run("cvrp", 150, 60, 1, 8, attention="fp32")
+    assert_kernel(a[5], "rollout_stc_kernel<1>")
+    assert_kernel(b[5], "rollout_kernel<1, 6, false>")
     frac, _ = compare_tours(a[0], b[0])
     assert frac >= 0.97, frac
 
@@ -93,14 +107,17 @@ def test_streamed_kernel_is_the_one_that_runs():
     ("cvrp", 15, 15, 2, 8),     # N+1 = 16: no padded key columns
     ("cvrp", 45, 45, 1, 8),     # k = 40 < N; rows in two TMEM lane quadrants
     ("cvrp", 70, 66, 1, 8),     # rows in three quadrants, M not a multiple of 4
-    ("cvrp", 111, 111, 1, 1),   # resident limit, 111 rows in one CTA
+    ("cvrp", 107, 107, 1, 1),   # resident limit at k = 40 (N+1 = 108), 107 rows in one CTA
     ("tsp", 4, 4, 2, 1),
     ("tsp", 31, 31, 1, 8),
     ("tsp", 100, 100, 1, 8),
     ("tsp", 112, 112, 1, 1),    # 112 nodes, 112 rows: every TMEM column of the S buffers in use
 ])
 def test_ragged_shapes_tensor_core_kernel(kind, N, M, n, aug):
-    tours, reward, ref_t, ref_r, prob = _run(kind, N, M, n, aug, attention="tensor")
+    tours, reward, ref_t, ref_r, prob, kernels = _run(kind, N, M, n, aug, attention="tensor")
+    want = _kernel(kind, N, M, n, aug, "tensor")
+    assert want.startswith("rollout_tc_kernel<")
+    assert_kernel(kernels, want)
     frac, same = compare_tours(tours, ref_t)
     assert frac >= 0.9, frac
     assert ((reward - ref_r).abs() / ref_r.abs())[same].max() < 1e-4
