@@ -16,7 +16,7 @@ FLAG_ENSEMBLE, FLAG_DISTANCE_PENALTY, FLAG_POSITIONAL = 1, 2, 4
 FLAG_ATTN_FP32, FLAG_ATTN_TENSOR = 8, 16
 MAX_LAYERS = 16
 NBR_STRIDE = 128
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 
 class ModelDesc(C.Structure):
@@ -67,6 +67,7 @@ SYMBOLS = {
     "elg_env_step": (_I, [_I, _P, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _P]),
     "elg_cur_feature": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P]),
     "elg_tour_length": (_I, [_P, _I, _P, _I, _I, _I, _I, _I, _P, _P]),
+    "elg_two_opt": (_I, [_I, _P, _I, _I, _P, _P, _I, _I, _I, _I, _P, _P, _P]),
     "elg_train_saved_bytes": (_SZ, [C.POINTER(ModelDesc), _I, _I]),
     "elg_encode_train": (_I, [C.POINTER(ModelDesc), _P, _P, C.POINTER(Tables), _I, _I, _P, _SZ, _P]),
     "elg_train_workspace_bytes": (_SZ, [C.POINTER(ModelDesc), _I, _I, _I, _I, _I]),

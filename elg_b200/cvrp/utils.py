@@ -1,4 +1,4 @@
-"""Drop-in for the reference's CVRP/utils.py: rollout, x8 augmentation, feasibility check, seeding.
+"""Drop-in for the reference's CVRP/utils.py: rollout, 2-opt, x8 augmentation, feasibility check, seeding.
 
 `rollout(model, env, eval_type)` keeps the reference signature and return convention
 (CVRP/utils.py:7-29): (solutions (B, M, T) int64, probs (B, T, M) | None, reward (B, M)).
@@ -11,7 +11,7 @@ import random
 import numpy as np
 import torch
 
-from .. import engine
+from .. import _lib, engine
 
 
 def rollout(model, env, eval_type='greedy'):
@@ -58,6 +58,44 @@ def _probs_from_logp(logp, T):
     underflows fp32 (an untrained CVRP100 policy has log-likelihoods around -360), so every step carries the geometric
     mean exp(logp / T) -- an expanded view, no memory.  The exact value is also kept as `model._last_logp`."""
     return torch.exp(logp / T)[:, None, :].expand(-1, T, -1)
+
+
+def batched_two_opt_torch(points, tour, max_iterations=1000, device=None):
+    """2-opt local search on depot-delimited CVRP tours (CVRP/utils.py:31-67), on the GPU (elg_two_opt).
+
+    points (N+1, 2) with the depot at row 0; tour (batch, T) node ids, depot visits as 0 (a rollout row); numpy or torch,
+    and the result comes back in the same type and dtype.  Returns (tour, iterations), iterations being the largest number
+    of moves any tour took.  device=None is the current CUDA device; there is no CPU path.
+
+    The reference tree is not part of this project; the signature is that of the DIFUSCO utility the cited lines are
+    understood to be.  Two deliberate differences: every tour stops on its own (the reference's loop couples the batch
+    and runs while any tour improves), and a move only reverses customers of one route, depot edges included, so every
+    route keeps its customers and its load.  The TSP function applied to these tours would reverse segments across depot
+    visits and could break capacity."""
+    return _two_opt_dropin("cvrp", points, tour, max_iterations, device)
+
+
+def _two_opt_dropin(problem, points, tour, max_iterations, device):
+    """Shared body of the cvrp / tsp batched_two_opt_torch: conversion in and out of numpy / torch, closed tsp tours."""
+    dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    if dev.type != "cuda":
+        raise _lib.ElgError("batched_two_opt_torch needs a CUDA device (got %s): elg_b200 has no CPU path" % dev)
+    as_numpy = isinstance(tour, np.ndarray)
+    t = torch.as_tensor(tour)
+    out_dtype, out_dev = t.dtype, t.device
+    t = t.to(dev, torch.int64)
+    xy = torch.as_tensor(points).to(dev, torch.float32)[None]
+    if problem == "tsp":
+        if t.dim() != 2 or t.shape[1] < 2 or not bool((t[:, -1] == t[:, 0]).all()):
+            raise ValueError("tsp tours must be (batch, N+1) closed tours (last node = first node)")
+        refined, _, iters = engine.two_opt("tsp", xy, t[:, :-1].contiguous(), max_iterations=max_iterations)
+        refined = torch.cat((refined, refined[:, :1]), dim=1)
+    else:
+        refined, _, iters = engine.two_opt("cvrp", xy, t, max_iterations=max_iterations)
+    n_iter = int(iters.max()) if iters.numel() else 0
+    if as_numpy:
+        return refined.cpu().numpy().astype(tour.dtype), n_iter
+    return refined.to(out_dev, out_dtype), n_iter
 
 
 def augment_xy_data_by_8_fold(problems):

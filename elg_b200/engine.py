@@ -310,6 +310,41 @@ def tour_length(xy, tours, rounding=False):
     return out
 
 
+def two_opt(problem, xy, tours, inst=None, max_iterations=1000, rounding=False):
+    """Best-improvement 2-opt local search (elg_two_opt; semantics in include/elg_b200.h), one launch for all tours.
+
+    xy (Bxy, N1, 2) coordinates; tours (R, L) int16 (the rollout's rows) or int64 node ids: tsp a permutation in positions
+    0..N1-1 that keeps its start node, cvrp a depot-delimited row whose moves stay inside one route; inst (R,) picks the xy
+    instance of every tour (default: tour r uses xy[r], or xy[0] when Bxy == 1); rounding rint()s every edge (library
+    metric).  Returns (tours int64 (R, L), length (R,) as tour_length measures it, iterations (R,) moves applied)."""
+    _require_cuda(xy, "xy")
+    _require_cuda(tours, "tours")
+    if tours.dim() != 2 or xy.dim() != 3 or xy.shape[2] != 2:
+        raise ValueError("tours must be (R, L) and xy (Bxy, N1, 2)")
+    if max_iterations < 0:
+        raise ValueError("max_iterations must be >= 0")
+    dev = tours.device
+    R, L = tours.shape
+    Bxy, N1 = int(xy.shape[0]), int(xy.shape[1])
+    n = L if problem == "cvrp" else min(N1, L)
+    if R and n:
+        lo, hi = torch.aminmax(tours[:, :n])
+        if int(lo) < 0 or int(hi) >= N1:
+            raise ValueError("tour node ids must lie in [0, %d)" % N1)
+    if inst is not None:
+        inst = torch.as_tensor(inst, device=dev).to(torch.int32).contiguous()
+        if inst.shape != (R,) or (R and (int(inst.min()) < 0 or int(inst.max()) >= Bxy)):
+            raise ValueError("inst must be (R,) indices into the %d xy instances" % Bxy)
+    t16 = tours.to(torch.int16, copy=True).contiguous()
+    length = torch.empty(R, dtype=torch.float32, device=dev)
+    iters = torch.empty(R, dtype=torch.int32, device=dev)
+    xy = xy.contiguous().float()
+    with torch.cuda.device(dev):
+        check(lib.elg_two_opt(ELG_CVRP if problem == "cvrp" else ELG_TSP, _ptr(xy), Bxy, N1, _ptr(inst), _ptr(t16), R, L,
+                              1 if rounding else 0, int(max_iterations), _ptr(iters), _ptr(length), _stream(dev)))
+    return t16.long(), length, iters
+
+
 # ---------------------------------------------------------------------------------------------- training path
 def encode_train(handle, xy, demand=None):
     """model.pre_forward for a training step: elg_encode that also keeps every layer's activations.

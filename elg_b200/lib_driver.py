@@ -5,6 +5,12 @@ TSP/test_tsplib.py:18-168) but are thin shells around the functions here:
     solve_instance(model, env, aug)      one greedy rollout of a loaded instance -> (best cost over aug x POMO, tours, rewards)
     run_set(entries, solve, ...)         the per-instance loop with timing and the record dicts of the result files
     gap_bins(results, edges, ...)        mean gap per size bin, as the reference prints them
+
+Optional 2-opt stage (config params.two_opt_iterations; absent or 0: nothing changes).  load_model records the setting on
+the model; solve_instance then refines the best POMO row of every aug-instance in the library metric (rounded unscaled
+coordinates) and returns the cost as an InstanceCost carrying the refined result; fill_record adds best_cost_2opt /
+gap_2opt / two_opt_seconds / two_opt_iterations to the record; run_set prints one extra line per instance and gap_bins
+one per size bin.  two_opt_refine is shared with the test.py drivers.
 """
 import json
 import os
@@ -12,6 +18,8 @@ import time
 
 import numpy as np
 import torch
+
+from . import engine
 
 
 def require_cuda(config):
@@ -32,7 +40,30 @@ def load_model(model_cls, config, device, model=None, needs_local=True):
     model = model.to(device)
     model.eval()
     model.requires_grad_(False)
+    model._elg_two_opt_iterations = config.get('params', {}).get('two_opt_iterations') or 0
     return model
+
+
+class InstanceCost(float):
+    """Best cost of one instance (a plain float to every caller).  `two_opt` is (refined cost, seconds, moves) when the
+    optional 2-opt stage ran, else None."""
+    two_opt = None
+
+
+def two_opt_refine(problem, xy, solutions, rewards, aug_factor, iterations, rounding):
+    """2-opt (engine.two_opt, one launch) of the best POMO row of every aug-instance of a greedy rollout.
+    xy (aug*n or 1, N1, 2) is the metric the cost is measured in: library runs pass the unscaled coordinates with
+    rounding, random instances the scaled ones without.  -> (refined cost per instance, best over its augmentations (n,);
+    seconds; moves applied per instance, summed over its augmentations (n,))"""
+    B = rewards.shape[0]
+    rows = solutions[torch.arange(B, device=solutions.device), rewards.argmax(dim=1)]
+    torch.cuda.synchronize()
+    t0 = time.time()
+    _, length, iters = engine.two_opt(problem, xy, rows, max_iterations=iterations, rounding=rounding)
+    torch.cuda.synchronize()
+    seconds = time.time() - t0
+    cost = length.reshape(aug_factor, B // aug_factor).min(dim=0)[0]
+    return cost, seconds, iters.reshape(aug_factor, B // aug_factor).sum(dim=0)
 
 
 def solve_instance(model, env, rollout, aug_factor, width):
@@ -42,7 +73,15 @@ def solve_instance(model, env, rollout, aug_factor, width):
     with torch.no_grad():
         solutions, _, rewards = rollout(model, env, 'greedy')
     best = -rewards.reshape(aug_factor, 1, width).max(dim=2)[0].max(dim=0)[0].float()
-    return float(best.cpu()[0]), solutions, rewards
+    cost = InstanceCost(best.cpu()[0])
+    iterations = getattr(model, '_elg_two_opt_iterations', 0)
+    if iterations:
+        cvrp = hasattr(env, 'unscaled_depot_node_xy')
+        refined, seconds, moves = two_opt_refine('cvrp' if cvrp else 'tsp',
+                                                 env.unscaled_depot_node_xy if cvrp else env._unscaled_dev,
+                                                 solutions, rewards, aug_factor, iterations, rounding=True)
+        cost.two_opt = (float(refined[0]), seconds, int(moves[0]))
+    return cost, solutions, rewards
 
 
 def run_set(entries, solve_one, repeat_times=1, echo_cost=False):
@@ -60,19 +99,39 @@ def run_set(entries, solve_one, repeat_times=1, echo_cost=False):
             print("Instance Name {}: gap {:.4f}".format(name, record['gap']))
             if echo_cost:
                 print("cost: {}".format(record['best_cost']))
+            if 'gap_2opt' in record:
+                print("Instance Name {}: gap after 2-opt {:.4f}".format(name, record['gap_2opt']))
     return results, total
 
 
 def fill_record(record, best_cost, scale, optimal):
     if record is not None:
-        record['best_cost'] = best_cost
+        record['best_cost'] = float(best_cost)
         record['scale'] = scale
         record['gap'] = (best_cost - optimal) / optimal
+        if getattr(best_cost, 'two_opt', None):
+            cost, seconds, moves = best_cost.two_opt
+            record['best_cost_2opt'] = cost
+            record['gap_2opt'] = (cost - optimal) / optimal
+            record['two_opt_seconds'] = seconds
+            record['two_opt_iterations'] = moves          # moves applied, summed over the augmentations
 
 
 def gap_bins(results, edges):
-    """edges: [(label, lo_exclusive, hi_inclusive)] on the instance scale -> {label: mean gap in %}, plus 'total'."""
-    gap = np.array([r['record'][-1]['gap'] for r in results])
+    """edges: [(label, lo_exclusive, hi_inclusive)] on the instance scale -> {label: mean gap in %}, plus 'total'.
+    When the records carry the 2-opt stage, also prints one line per bin and 'gap_2opt': {label: mean gap in %}."""
+    out = _bin_means(results, edges, 'gap')
+    if results and all('gap_2opt' in r['record'][-1] for r in results):
+        out['gap_2opt'] = _bin_means(results, edges, 'gap_2opt')
+        for label, mean in out['gap_2opt'].items():
+            if label != 'total':
+                print("Average gap after 2-opt on subset of {}: {:.2f}%".format(label, mean))
+        print("Average gap after 2-opt total: {:.2f}%".format(out['gap_2opt']['total']))
+    return out
+
+
+def _bin_means(results, edges, key):
+    gap = np.array([r['record'][-1][key] for r in results])
     scale = np.array([int(r['record'][-1]['scale']) for r in results])
     out = {}
     for label, lo, hi in edges:

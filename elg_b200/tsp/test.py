@@ -10,6 +10,7 @@ import torch
 
 from .TSPEnv import TSPEnv
 from .TSPModel import TSPModel
+from .. import lib_driver as drv
 from .utils import rollout
 
 
@@ -29,15 +30,24 @@ def solve_batch(model, env, batch, aug_factor):
     return no_aug_cost, aug_cost, solutions, rewards
 
 
-def test(dataloader, model, env, aug_factor):
+def test(dataloader, model, env, aug_factor, two_opt_iterations=0):
+    """two_opt_iterations > 0 (config params.two_opt_iterations) also refines the best POMO row of every aug-instance
+    with 2-opt in the reward metric and prints the refined cost after the reference's lines."""
     model.eval()
     model.requires_grad_(False)
     avg_cost_total, no_avg_cost_total, t = 0., 0., 0
+    two_opt_cost, two_opt_seconds, two_opt_moves = 0., 0., 0
     start = time.time()
     for batch in dataloader:
-        no_aug_cost, aug_cost, _, _ = solve_batch(model, env, batch, aug_factor)
+        no_aug_cost, aug_cost, solutions, rewards = solve_batch(model, env, batch, aug_factor)
         avg_cost_total += aug_cost.mean()
         no_avg_cost_total += no_aug_cost.mean()
+        if two_opt_iterations:
+            cost, seconds, moves = drv.two_opt_refine("tsp", env.problems, solutions, rewards, aug_factor, two_opt_iterations,
+                                                      rounding=False)
+            two_opt_cost += cost.mean()
+            two_opt_seconds += seconds
+            two_opt_moves += int(moves.sum())
         t += 1
     torch.cuda.synchronize()
     end = time.time()
@@ -45,6 +55,8 @@ def test(dataloader, model, env, aug_factor):
     no_avg_cost_total /= t
     print("Aug cost: {:.4f}".format(avg_cost_total))
     print("no aug Avg cost: {:.4f}, Wall-clock time: {:.2f}s".format(no_avg_cost_total, float(end - start)))
+    if two_opt_iterations:
+        print("2-opt Aug cost: {:.4f}, 2-opt time: {:.2f}s, moves: {}".format(two_opt_cost / t, two_opt_seconds, two_opt_moves))
     return avg_cost_total
 
 
@@ -71,4 +83,5 @@ if __name__ == "__main__":
         data = pickle.load(f)[:config['params']['test_size']]
     bs = config['params']['test_batch_size']
     batches = [torch.FloatTensor(data[i:i + bs]) for i in range(0, len(data), bs)]
-    test(batches, model, env, aug_factor=config['params']['aug_factor'])
+    test(batches, model, env, aug_factor=config['params']['aug_factor'],
+         two_opt_iterations=config['params'].get('two_opt_iterations') or 0)

@@ -1,11 +1,11 @@
-"""Drop-in for the reference's TSP/utils.py: rollout (TSP/utils.py:7-26), x8 augmentation, seeding."""
+"""Drop-in for the reference's TSP/utils.py: rollout (TSP/utils.py:7-26), 2-opt, x8 augmentation, seeding."""
 import random
 
 import numpy as np
 import torch
 
 from .. import engine
-from ..cvrp.utils import augment_xy_data_by_8_fold, seed_everything  # noqa: F401  (same functions in both sub-projects)
+from ..cvrp.utils import _two_opt_dropin, augment_xy_data_by_8_fold, seed_everything  # noqa: F401  (same functions in both sub-projects)
 
 
 def rollout(model, env, eval_type='greedy'):
@@ -40,6 +40,19 @@ def _fused_rollout(model, env, eval_type):
     probs = None if eval_type == 'greedy' else _probs_from_logp(logp, env.problem_size)
     model._last_logp = logp
     return solutions, probs, reward
+
+
+def batched_two_opt_torch(points, tour, max_iterations=1000, device=None):
+    """2-opt local search on closed TSP tours (TSP/utils.py:28-70), on the GPU (elg_two_opt).
+
+    points (N, 2); tour (batch, N+1) closed tours (last node = first node); numpy or torch, and the result comes back in
+    the same type and dtype.  Returns (tour, iterations), iterations being the largest number of moves any tour took.
+    Position 0 (the start node) never moves.  device=None is the current CUDA device; there is no CPU path.
+
+    The reference tree is not part of this project; the signature is that of the DIFUSCO utility the cited lines are
+    understood to be.  One deliberate difference: every tour stops on its own, where the reference's loop couples the
+    batch and runs while any tour improves."""
+    return _two_opt_dropin("tsp", points, tour, max_iterations, device)
 
 
 def check_feasible(pi):

@@ -29,7 +29,8 @@
 extern "C" {
 #endif
 
-#define ELG_ABI_VERSION 3   /* 2: training path, data generators; 3: elg_tables.et / .ws (streamed tensor-core decode) */
+#define ELG_ABI_VERSION 4   /* 2: training path, data generators; 3: elg_tables.et / .ws (streamed tensor-core decode);
+                               4: elg_two_opt */
 
 enum { ELG_TSP = 0, ELG_CVRP = 1 };
 enum { ELG_GREEDY = 0, ELG_SAMPLE = 1 };
@@ -222,6 +223,22 @@ int elg_cur_feature(const float* xy, const float* demand, const float* load, con
  * aug-instances as in TSPEnv.compute_unscaled_distance); round_edges applies rint() per edge. */
 int elg_tour_length(const float* xy, int Bxy, const int64_t* tours, int B, int M, int T, int N1, int round_edges,
                     float* out, void* stream);
+
+/* ---- 2-opt local search ------------------------------------------------------------------------
+ * Best-improvement 2-opt on R tours, refined in place; the counterpart of the reference's batched_two_opt_torch
+ * (TSP/utils.py:28-70, CVRP/utils.py:31-67), except that every tour stops on its own.
+ *   xy [Bxy][N1][2]   coordinates; inst [R] int32 picks the xy instance of each tour (NULL: r when Bxy == R, 0 when Bxy == 1)
+ *   tours [R][L]      int16 node ids.  tsp: positions 0..N1-1 hold a permutation, closed implicitly (L >= N1; positions
+ *                     N1.. are ignored and left as they are).  cvrp: a rollout row (depot visits as 0, trailing zero
+ *                     padding), closed implicitly, L <= 2*N1+2.
+ *   A move picks positions i < j, reverses positions i+1..j and gains d(t_i,t_j) + d(t_i+1,t_j+1) - d(t_i,t_i+1) -
+ *   d(t_j,t_j+1) (j+1 wraps to 0); d is the reward's segment length, rint()-ed per edge when round_edges is set.  Every
+ *   move evaluates all admissible pairs and applies the smallest gain (ties: lowest i*L + j) if it is below -1e-6, at most
+ *   max_iterations times.  tsp: admissible j >= i+2 except (0, N1-1), so position 0 never moves.  cvrp: admissible j >= i+2
+ *   with positions i+1..j all customers, so every move stays inside one route and every route keeps its customers (and its load).
+ *   iterations [R]    moves applied;  length [R]  closed length of the refined tour, summed as elg_tour_length sums it */
+int elg_two_opt(int problem, const float* xy, int Bxy, int N1, const int32_t* inst, int16_t* tours, int R, int L,
+                int round_edges, int max_iterations, int32_t* iterations, float* length, void* stream);
 
 /* ---- training path (REINFORCE with the POMO shared baseline) ----------------------------------
  * Replaces the body of the reference's training loop, CVRP/train.py:104-125 (TSP/train.py:100-122):
