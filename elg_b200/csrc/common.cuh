@@ -116,6 +116,37 @@ __device__ __forceinline__ float seglen(float dx, float dy) {
   return __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
 }
 
+// ---- local search (two_opt.cu, cvrp_ls.cu) ----------------------------------------------------
+constexpr float LS_MIN_GAIN = -1e-6f;  // a move is applied only if its gain is below this
+
+// d(a, b) of nodes a, b: the reward's seglen, rint()-ed under the library metric
+__device__ __forceinline__ float edge_len(const float2* __restrict__ xy, int a, int b, int round_edges) {
+  const float2 p = xy[a], q = xy[b];
+  const float d = seglen(p.x - q.x, p.y - q.y);
+  return round_edges ? rintf(d) : d;
+}
+
+// (gain, key) ordered by gain, then by key: torch.argmin's first-index tie-break
+__device__ __forceinline__ bool gain_better(float g, int key, float bg, int bkey) {
+  return g < bg || (g == bg && key < bkey);
+}
+
+// CTA-wide minimum of every thread's (bg, bkey) under gain_better, returned to every thread.  red_g / red_k hold one
+// entry per warp; a barrier must separate the reads here from the next writes to them.
+__device__ __forceinline__ void cta_min_gain(float& bg, int& bkey, float* red_g, int* red_k) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
+  for (int o = 16; o > 0; o >>= 1) {
+    const float g = __shfl_xor_sync(0xffffffffu, bg, o);
+    const int k = __shfl_xor_sync(0xffffffffu, bkey, o);
+    if (gain_better(g, k, bg, bkey)) { bg = g; bkey = k; }
+  }
+  if (lane == 0) { red_g[warp] = bg; red_k[warp] = bkey; }
+  __syncthreads();
+  bg = red_g[0]; bkey = red_k[0];
+  for (int w = 1; w < nwarps; ++w)
+    if (gain_better(red_g[w], red_k[w], bg, bkey)) { bg = red_g[w]; bkey = red_k[w]; }
+}
+
 // Swizzled column of the score matrix E' (row j): XOR the 16-byte chunk index with (j & 7) so
 // that 8 consecutive rows read by a quarter-warp hit 8 different bank groups.
 __host__ __device__ __forceinline__ int eswz(int j, int c) { return c ^ ((j & 7) << 2); }

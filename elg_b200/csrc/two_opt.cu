@@ -15,18 +15,6 @@
 namespace elg {
 
 constexpr int TWO_OPT_CHUNK = 16;          // pairs per diagonal chunk (one extra seglen per chunk)
-constexpr float TWO_OPT_MIN_GAIN = -1e-6f; // a move is applied only if its gain is below this
-
-__device__ __forceinline__ float two_opt_edge(const float2* __restrict__ xy, int a, int b, int round_edges) {
-  const float2 p = xy[a], q = xy[b];
-  const float d = seglen(p.x - q.x, p.y - q.y);
-  return round_edges ? rintf(d) : d;
-}
-
-// (gain, flat index) ordered by gain, then by index: torch.argmin's first-index tie-break
-__device__ __forceinline__ bool two_opt_better(float g, int idx, float bg, int bidx) {
-  return g < bg || (g == bg && idx < bidx);
-}
 
 template <int PROBLEM>
 __global__ void __launch_bounds__(512) two_opt_kernel(const float* __restrict__ xy_g, int Bxy, int N1,
@@ -42,7 +30,7 @@ __global__ void __launch_bounds__(512) two_opt_kernel(const float* __restrict__ 
   float* edge = reinterpret_cast<float*>(xy + N1);     // edge[p] = d(t_p, t_{p+1 mod n})
   int16_t* tour = reinterpret_cast<int16_t*>(edge + n);
   int16_t* lastdep = tour + n;                          // cvrp: last position <= p holding the depot, -1 if none
-  const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarps = nthr >> 5;
+  const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, warp = tid >> 5;
 
   for (int r = blockIdx.x; r < R; r += gridDim.x) {
     const int b = inst ? inst[r] : (Bxy == 1 ? 0 : r);
@@ -51,7 +39,7 @@ __global__ void __launch_bounds__(512) two_opt_kernel(const float* __restrict__ 
     for (int p = tid; p < N1; p += nthr) xy[p] = src[p];
     for (int p = tid; p < n; p += nthr) tour[p] = row[p];
     __syncthreads();
-    for (int p = tid; p < n; p += nthr) edge[p] = two_opt_edge(xy, tour[p], tour[p + 1 == n ? 0 : p + 1], round_edges);
+    for (int p = tid; p < n; p += nthr) edge[p] = edge_len(xy, tour[p], tour[p + 1 == n ? 0 : p + 1], round_edges);
 
     int dmax = n - 1;                                   // largest diagonal j - i worth sweeping
     if (PROBLEM == ELG_CVRP) {
@@ -94,30 +82,21 @@ __global__ void __launch_bounds__(512) two_opt_kernel(const float* __restrict__ 
         const int d = 2 + task % nd;
         const int i0 = (task / nd) * TWO_OPT_CHUNK, i1 = min(i0 + TWO_OPT_CHUNK, n - d);
         if (i0 >= i1) continue;
-        float dij = two_opt_edge(xy, tour[i0], tour[i0 + d], round_edges);
+        float dij = edge_len(xy, tour[i0], tour[i0 + d], round_edges);
         for (int i = i0; i < i1; ++i) {
           const int j = i + d, j1 = j + 1 == n ? 0 : j + 1;
-          const float dnext = two_opt_edge(xy, tour[i + 1], tour[j1], round_edges);
+          const float dnext = edge_len(xy, tour[i + 1], tour[j1], round_edges);
           const bool ok = PROBLEM == ELG_CVRP ? lastdep[j] <= i : !(i == 0 && j == n - 1);
           if (ok) {
             const float g = (dij - edge[i]) + (dnext - edge[j]);
             const int idx = i * L + j;
-            if (two_opt_better(g, idx, bg, bidx)) { bg = g; bidx = idx; }
+            if (gain_better(g, idx, bg, bidx)) { bg = g; bidx = idx; }
           }
           dij = dnext;
         }
       }
-      for (int o = 16; o > 0; o >>= 1) {
-        const float g = __shfl_xor_sync(0xffffffffu, bg, o);
-        const int idx = __shfl_xor_sync(0xffffffffu, bidx, o);
-        if (two_opt_better(g, idx, bg, bidx)) { bg = g; bidx = idx; }
-      }
-      if (lane == 0) { red_g[warp] = bg; red_i[warp] = bidx; }
-      __syncthreads();
-      bg = red_g[0]; bidx = red_i[0];
-      for (int w = 1; w < nwarps; ++w)
-        if (two_opt_better(red_g[w], red_i[w], bg, bidx)) { bg = red_g[w]; bidx = red_i[w]; }
-      if (!(bg < TWO_OPT_MIN_GAIN)) break;              // every thread reads the same reduction: uniform exit
+      cta_min_gain(bg, bidx, red_g, red_i);
+      if (!(bg < LS_MIN_GAIN)) break;                   // every thread reads the same reduction: uniform exit
       const int i = bidx / L, j = bidx % L;
       // reverse tour[i+1..j] and, with it, the edges strictly inside the segment, edge[i+1..j-1]
       for (int k = tid; k < (j - i) / 2; k += nthr) {
@@ -127,8 +106,8 @@ __global__ void __launch_bounds__(512) two_opt_kernel(const float* __restrict__ 
         const float e = edge[i + 1 + k]; edge[i + 1 + k] = edge[j - 1 - k]; edge[j - 1 - k] = e;
       }
       __syncthreads();
-      if (tid == 0) edge[i] = two_opt_edge(xy, tour[i], tour[i + 1], round_edges);
-      if (tid == 1) edge[j] = two_opt_edge(xy, tour[j], tour[j + 1 == n ? 0 : j + 1], round_edges);
+      if (tid == 0) edge[i] = edge_len(xy, tour[i], tour[i + 1], round_edges);
+      if (tid == 1) edge[j] = edge_len(xy, tour[j], tour[j + 1 == n ? 0 : j + 1], round_edges);
       ++moves;
       __syncthreads();
     }

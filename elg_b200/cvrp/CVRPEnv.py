@@ -3,7 +3,8 @@
 Public surface kept: CVRPEnv(multi_width, device), load_random_problems, load_vrplib_problem,
 reset, reset_width, pre_step, step, get_cur_feature, compute_unscaled_reward, and the attributes
 callers read (batch_size, problem_size, multi_width, depot_node_xy, depot_node_demand,
-selected_node_list, reset_state, step_state).  fp32 {0,-inf} masks are produced for API
+selected_node_list, reset_state, step_state).  `capacity` additionally keeps the vehicle capacity of a library
+instance (None for random problems, whose demands arrive already normalised); the drivers' local search needs it.  fp32 {0,-inf} masks are produced for API
 compatibility; the kernels work on 128-bit visited/mask words per row.
 """
 import torch
@@ -60,6 +61,7 @@ class CVRPEnv:
         self.depot_node_xy = None          # (batch, problem+1, 2)
         self.depot_node_demand = None      # (batch, problem+1)
         self.unscaled_depot_node_xy = None
+        self.capacity = None
         self.input_mask = None
         self.dist = None
         self.selected_count = None
@@ -88,6 +90,7 @@ class CVRPEnv:
         if aug_factor not in (1, 8):
             raise NotImplementedError
         self.vrplib = False
+        self.capacity = None
         loc = batch['loc'].to(self.device, non_blocking=True)
         demand = batch['demand'].to(self.device, non_blocking=True)
         depot = batch['depot'].to(self.device, non_blocking=True)
@@ -100,6 +103,7 @@ class CVRPEnv:
         if aug_factor not in (1, 8):
             raise NotImplementedError
         self.vrplib = True
+        self.capacity = instance['capacity']
         coord = torch.FloatTensor(instance['node_coord']).unsqueeze(0).to(self.device)
         demand = torch.FloatTensor(instance['demand']).unsqueeze(0).to(self.device) / instance['capacity']
         lo, hi = coord.min(dim=1, keepdim=True)[0], coord.max(dim=1, keepdim=True)[0]

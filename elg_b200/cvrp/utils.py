@@ -1,4 +1,5 @@
-"""Drop-in for the reference's CVRP/utils.py: rollout, 2-opt, x8 augmentation, feasibility check, seeding.
+"""Drop-in for the reference's CVRP/utils.py: rollout, 2-opt, x8 augmentation, feasibility check, seeding; plus the
+capacity-aware local search cvrp_local_search.
 
 `rollout(model, env, eval_type)` keeps the reference signature and return convention
 (CVRP/utils.py:7-29): (solutions (B, M, T) int64, probs (B, T, M) | None, reward (B, M)).
@@ -92,6 +93,30 @@ def _two_opt_dropin(problem, points, tour, max_iterations, device):
         refined = torch.cat((refined, refined[:, :1]), dim=1)
     else:
         refined, _, iters = engine.two_opt("cvrp", xy, t, max_iterations=max_iterations)
+    n_iter = int(iters.max()) if iters.numel() else 0
+    if as_numpy:
+        return refined.cpu().numpy().astype(tour.dtype), n_iter
+    return refined.to(out_dev, out_dtype), n_iter
+
+
+def cvrp_local_search(points, demand, capacity, tour, max_iterations=1000, device=None):
+    """Capacity-aware CVRP local search on the GPU (elg_cvrp_local_search): 2-opt inside a route, relocate, swap and
+    2-opt* between routes, best improvement, every tour stopping on its own.
+
+    points (N+1, 2) with the depot at row 0; demand (N+1,) normalised by the capacity as the environments hold it (depot
+    0); capacity the integer vehicle capacity; tour (batch, T) rollout rows (depot visits as 0, every customer once, every
+    route within capacity); numpy or torch, and the tour comes back in the same type and dtype, in canonical form (routes
+    in order, each preceded by one 0, zero padding to T).  Returns (tour, iterations), iterations being the largest number
+    of moves any tour took.  device=None is the current CUDA device; there is no CPU path."""
+    dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    if dev.type != "cuda":
+        raise _lib.ElgError("cvrp_local_search needs a CUDA device (got %s): elg_b200 has no CPU path" % dev)
+    as_numpy = isinstance(tour, np.ndarray)
+    t = torch.as_tensor(tour)
+    out_dtype, out_dev = t.dtype, t.device
+    xy = torch.as_tensor(points).to(dev, torch.float32)[None]
+    dem = torch.as_tensor(demand).to(dev, torch.float32)[None]
+    refined, _, iters = engine.cvrp_local_search(xy, t.to(dev, torch.int64), dem, capacity, max_iterations=max_iterations)
     n_iter = int(iters.max()) if iters.numel() else 0
     if as_numpy:
         return refined.cpu().numpy().astype(tour.dtype), n_iter

@@ -345,6 +345,63 @@ def two_opt(problem, xy, tours, inst=None, max_iterations=1000, rounding=False):
     return t16.long(), length, iters
 
 
+def cvrp_local_search(xy, tours, demand, capacity, inst=None, max_iterations=1000, rounding=False):
+    """Capacity-aware best-improvement CVRP local search (elg_cvrp_local_search; semantics in include/elg_b200.h): 2-opt
+    inside a route, relocate, swap and 2-opt* between routes, one launch for all rows.
+
+    xy (Bxy, N1, 2) coordinates; tours (R, L) rollout rows, int16 or int64, with every customer exactly once, position 0
+    the depot and every route within capacity; demand (Bxy, N1) normalised demands as CVRPEnv holds them (depot 0);
+    capacity the integer vehicle capacity: demands in units are rint(demand * capacity) and must lie within 1e-3 of it.
+    inst (R,) picks the xy / demand instance of every row (default: row r uses instance r, or 0 when Bxy == 1); rounding
+    rint()s every edge (library metric).  Returns (canonical tours int64 (R, L), length (R,) as tour_length measures it,
+    iterations (R,) moves applied)."""
+    if tours.dim() != 2 or xy.dim() != 3 or xy.shape[2] != 2 or demand.shape != xy.shape[:2]:
+        raise ValueError("tours must be (R, L), xy (Bxy, N1, 2) and demand (Bxy, N1)")
+    if max_iterations < 0:
+        raise ValueError("max_iterations must be >= 0")
+    if int(capacity) != capacity or capacity <= 0:
+        raise ValueError("capacity must be a positive integer (got %r)" % (capacity,))
+    capacity = int(capacity)
+    dev = tours.device
+    R, L = tours.shape
+    Bxy, N1 = int(xy.shape[0]), int(xy.shape[1])
+    scaled = demand.double() * capacity
+    units = torch.round(scaled)
+    if bool(((scaled - units).abs() > 1e-3).any()):
+        raise ValueError("demand * capacity must be integral (within 1e-3): demands are whole units of the capacity")
+    units = units.to(torch.int32).contiguous()
+    if inst is not None:
+        inst = torch.as_tensor(inst, device=dev).to(torch.int32).contiguous()
+        if inst.shape != (R,) or (R and (int(inst.min()) < 0 or int(inst.max()) >= Bxy)):
+            raise ValueError("inst must be (R,) indices into the %d xy instances" % Bxy)
+    elif Bxy not in (1, R):
+        raise ValueError("without inst, xy must hold 1 or R instances (got %d for %d rows)" % (Bxy, R))
+    if R:
+        t = tours.long()
+        if int(t.min()) < 0 or int(t.max()) >= N1 or bool((t[:, 0] != 0).any()):
+            raise ValueError("rows must hold node ids in [0, %d) with the depot at position 0" % N1)
+        counts = torch.zeros(R, N1, dtype=torch.int32, device=dev).scatter_add_(1, t, torch.ones_like(t, dtype=torch.int32))
+        if not bool((counts[:, 1:] == 1).all()):
+            raise ValueError("every row must visit each customer 1..%d exactly once" % (N1 - 1))
+        which = inst.long() if inst is not None else (torch.arange(R, device=dev) if Bxy > 1 else torch.zeros(R, dtype=torch.long, device=dev))
+        d = units[which].gather(1, t)
+        route = (t == 0).long().cumsum(1)
+        loads = torch.zeros(R, L + 1, dtype=torch.int64, device=dev).scatter_add_(1, route, d.long())
+        if int(loads.max()) > capacity:
+            raise ValueError("an input route exceeds the capacity %d" % capacity)
+    _require_cuda(xy, "xy")
+    _require_cuda(tours, "tours")
+    _require_cuda(units, "demand")
+    t16 = tours.to(torch.int16, copy=True).contiguous()
+    length = torch.empty(R, dtype=torch.float32, device=dev)
+    iters = torch.empty(R, dtype=torch.int32, device=dev)
+    xy = xy.contiguous().float()
+    with torch.cuda.device(dev):
+        check(lib.elg_cvrp_local_search(_ptr(xy), Bxy, N1, _ptr(units), capacity, _ptr(inst), _ptr(t16), R, L,
+                                        1 if rounding else 0, int(max_iterations), _ptr(iters), _ptr(length), _stream(dev)))
+    return t16.long(), length, iters
+
+
 # ---------------------------------------------------------------------------------------------- training path
 def encode_train(handle, xy, demand=None):
     """model.pre_forward for a training step: elg_encode that also keeps every layer's activations.

@@ -11,6 +11,12 @@ the model; solve_instance then refines the best POMO row of every aug-instance i
 coordinates) and returns the cost as an InstanceCost carrying the refined result; fill_record adds best_cost_2opt /
 gap_2opt / two_opt_seconds / two_opt_iterations to the record; run_set prints one extra line per instance and gap_bins
 one per size bin.  two_opt_refine is shared with the test.py drivers.
+
+Optional CVRP local search stage (config params.local_search_iterations; absent or 0: nothing changes), independent of
+the 2-opt stage and run on the same rows: solve_instance refines them with engine.cvrp_local_search in the library metric
+(with the capacity CVRPEnv.load_vrplib_problem recorded), InstanceCost.local_search carries the result, fill_record adds
+best_cost_ls / gap_ls / ls_seconds / ls_iterations, and run_set / gap_bins print their lines after the 2-opt ones.
+load_model rejects the key for a TSP model.
 """
 import json
 import os
@@ -32,6 +38,9 @@ def require_cuda(config):
 
 def load_model(model_cls, config, device, model=None, needs_local=True):
     """The reference's checkpoint protocol: add_local_policy BEFORE load_state_dict (CVRP/test.py:75-78)."""
+    from .cvrp.CVRPModel import CVRPModel
+    if not issubclass(model_cls, CVRPModel):
+        reject_local_search(config)
     if model is None:
         model = model_cls(**config['model_params'])
         if needs_local:
@@ -41,13 +50,30 @@ def load_model(model_cls, config, device, model=None, needs_local=True):
     model.eval()
     model.requires_grad_(False)
     model._elg_two_opt_iterations = config.get('params', {}).get('two_opt_iterations') or 0
+    model._elg_local_search_iterations = config.get('params', {}).get('local_search_iterations') or 0
     return model
 
 
+def reject_local_search(config):
+    """The TSP drivers: params.local_search_iterations is the CVRP local search, TSP tours have the 2-opt stage."""
+    if config.get('params', {}).get('local_search_iterations'):
+        raise ValueError("params.local_search_iterations is the capacity-aware CVRP local search; "
+                         "refine TSP tours with params.two_opt_iterations")
+
+
 class InstanceCost(float):
-    """Best cost of one instance (a plain float to every caller).  `two_opt` is (refined cost, seconds, moves) when the
-    optional 2-opt stage ran, else None."""
+    """Best cost of one instance (a plain float to every caller).  `two_opt` / `local_search` are (refined cost, seconds,
+    moves) when the optional stage ran, else None."""
     two_opt = None
+    local_search = None
+
+
+# optional refinement stages: (InstanceCost attribute, record key suffix, record key prefix, name in the printouts)
+_STAGES = (('two_opt', '2opt', 'two_opt', '2-opt'), ('local_search', 'ls', 'ls', 'local search'))
+
+
+def _best_rows(solutions, rewards):
+    return solutions[torch.arange(rewards.shape[0], device=solutions.device), rewards.argmax(dim=1)]
 
 
 def two_opt_refine(problem, xy, solutions, rewards, aug_factor, iterations, rounding):
@@ -55,13 +81,26 @@ def two_opt_refine(problem, xy, solutions, rewards, aug_factor, iterations, roun
     xy (aug*n or 1, N1, 2) is the metric the cost is measured in: library runs pass the unscaled coordinates with
     rounding, random instances the scaled ones without.  -> (refined cost per instance, best over its augmentations (n,);
     seconds; moves applied per instance, summed over its augmentations (n,))"""
-    B = rewards.shape[0]
-    rows = solutions[torch.arange(B, device=solutions.device), rewards.argmax(dim=1)]
+    rows = _best_rows(solutions, rewards)
+    return _timed_refine(lambda: engine.two_opt(problem, xy, rows, max_iterations=iterations, rounding=rounding), aug_factor)
+
+
+def local_search_refine(xy, demand, capacity, solutions, rewards, aug_factor, iterations, rounding):
+    """CVRP local search (engine.cvrp_local_search, one launch) of the best POMO row of every aug-instance of a greedy
+    rollout; demand (aug*n, N1) normalised as the environment holds it, capacity the integer capacity; otherwise as
+    two_opt_refine."""
+    rows = _best_rows(solutions, rewards)
+    return _timed_refine(lambda: engine.cvrp_local_search(xy, rows, demand, capacity, max_iterations=iterations,
+                                                          rounding=rounding), aug_factor)
+
+
+def _timed_refine(run, aug_factor):
     torch.cuda.synchronize()
     t0 = time.time()
-    _, length, iters = engine.two_opt(problem, xy, rows, max_iterations=iterations, rounding=rounding)
+    _, length, iters = run()
     torch.cuda.synchronize()
     seconds = time.time() - t0
+    B = length.shape[0]
     cost = length.reshape(aug_factor, B // aug_factor).min(dim=0)[0]
     return cost, seconds, iters.reshape(aug_factor, B // aug_factor).sum(dim=0)
 
@@ -81,6 +120,13 @@ def solve_instance(model, env, rollout, aug_factor, width):
                                                  env.unscaled_depot_node_xy if cvrp else env._unscaled_dev,
                                                  solutions, rewards, aug_factor, iterations, rounding=True)
         cost.two_opt = (float(refined[0]), seconds, int(moves[0]))
+    iterations = getattr(model, '_elg_local_search_iterations', 0)
+    if iterations:
+        if env.capacity is None:
+            raise ValueError("the local search stage needs the instance's capacity (CVRPEnv.load_vrplib_problem)")
+        refined, seconds, moves = local_search_refine(env.unscaled_depot_node_xy, env.depot_node_demand, env.capacity,
+                                                      solutions, rewards, aug_factor, iterations, rounding=True)
+        cost.local_search = (float(refined[0]), seconds, int(moves[0]))
     return cost, solutions, rewards
 
 
@@ -99,8 +145,9 @@ def run_set(entries, solve_one, repeat_times=1, echo_cost=False):
             print("Instance Name {}: gap {:.4f}".format(name, record['gap']))
             if echo_cost:
                 print("cost: {}".format(record['best_cost']))
-            if 'gap_2opt' in record:
-                print("Instance Name {}: gap after 2-opt {:.4f}".format(name, record['gap_2opt']))
+            for _, suffix, _, label in _STAGES:
+                if 'gap_' + suffix in record:
+                    print("Instance Name {}: gap after {} {:.4f}".format(name, label, record['gap_' + suffix]))
     return results, total
 
 
@@ -109,24 +156,28 @@ def fill_record(record, best_cost, scale, optimal):
         record['best_cost'] = float(best_cost)
         record['scale'] = scale
         record['gap'] = (best_cost - optimal) / optimal
-        if getattr(best_cost, 'two_opt', None):
-            cost, seconds, moves = best_cost.two_opt
-            record['best_cost_2opt'] = cost
-            record['gap_2opt'] = (cost - optimal) / optimal
-            record['two_opt_seconds'] = seconds
-            record['two_opt_iterations'] = moves          # moves applied, summed over the augmentations
+        for attr, suffix, prefix, _ in _STAGES:
+            if getattr(best_cost, attr, None):
+                cost, seconds, moves = getattr(best_cost, attr)
+                record['best_cost_' + suffix] = cost
+                record['gap_' + suffix] = (cost - optimal) / optimal
+                record[prefix + '_seconds'] = seconds
+                record[prefix + '_iterations'] = moves    # moves applied, summed over the augmentations
 
 
 def gap_bins(results, edges):
     """edges: [(label, lo_exclusive, hi_inclusive)] on the instance scale -> {label: mean gap in %}, plus 'total'.
-    When the records carry the 2-opt stage, also prints one line per bin and 'gap_2opt': {label: mean gap in %}."""
+    When the records carry an optional stage, also prints one line per bin and a total line for it, and adds
+    'gap_2opt' / 'gap_ls': {label: mean gap in %}."""
     out = _bin_means(results, edges, 'gap')
-    if results and all('gap_2opt' in r['record'][-1] for r in results):
-        out['gap_2opt'] = _bin_means(results, edges, 'gap_2opt')
-        for label, mean in out['gap_2opt'].items():
-            if label != 'total':
-                print("Average gap after 2-opt on subset of {}: {:.2f}%".format(label, mean))
-        print("Average gap after 2-opt total: {:.2f}%".format(out['gap_2opt']['total']))
+    for _, suffix, _, name in _STAGES:
+        key = 'gap_' + suffix
+        if results and all(key in r['record'][-1] for r in results):
+            out[key] = _bin_means(results, edges, key)
+            for label, mean in out[key].items():
+                if label != 'total':
+                    print("Average gap after {} on subset of {}: {:.2f}%".format(name, label, mean))
+            print("Average gap after {} total: {:.2f}%".format(name, out[key]['total']))
     return out
 
 

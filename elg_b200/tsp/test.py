@@ -76,6 +76,7 @@ if __name__ == "__main__":
     import yaml
     with open('config.yml', 'r', encoding='utf-8') as f:
         config = yaml.load(f.read(), Loader=yaml.FullLoader)
+    drv.reject_local_search(config)
     device = "cuda:{}".format(config['cuda_device_num'])
     model = load_model(config, device)
     env = TSPEnv(multi_width=config['params']['multiple_width'], device=device)

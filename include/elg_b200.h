@@ -30,7 +30,8 @@ extern "C" {
 #endif
 
 #define ELG_ABI_VERSION 4   /* 2: training path, data generators; 3: elg_tables.et / .ws (streamed tensor-core decode);
-                               4: elg_two_opt */
+                               4: elg_two_opt, then elg_cvrp_local_search (purely additive, so the version stays 4:
+                                  a library without it fails on the missing symbol when the binding loads) */
 
 enum { ELG_TSP = 0, ELG_CVRP = 1 };
 enum { ELG_GREEDY = 0, ELG_SAMPLE = 1 };
@@ -239,6 +240,30 @@ int elg_tour_length(const float* xy, int Bxy, const int64_t* tours, int B, int M
  *   iterations [R]    moves applied;  length [R]  closed length of the refined tour, summed as elg_tour_length sums it */
 int elg_two_opt(int problem, const float* xy, int Bxy, int N1, const int32_t* inst, int16_t* tours, int R, int L,
                 int round_edges, int max_iterations, int32_t* iterations, float* length, void* stream);
+
+/* ---- capacity-aware CVRP local search ------------------------------------------------------------
+ * Best-improvement local search on R CVRP solutions, refined in place; every row stops on its own.
+ *   xy [Bxy][N1][2], inst, round_edges, max_iterations, iterations [R], length [R]: as elg_two_opt
+ *   demand [Bxy][N1]  int32 demand units, demand[., 0] = 0; capacity in the same units.  A route is feasible iff the
+ *                     integer sum of its demands is <= capacity; there is no tolerance.  Input routes must be feasible.
+ *   tours [R][L]      int16 rollout rows: position 0 the depot, every customer 1..N1-1 exactly once, depot visits as 0,
+ *                     trailing zero padding, L <= 2*N1+2.  The output row is canonical even without a move: routes in
+ *                     their order, each preceded by one 0, no empty route, zero padding to L.
+ * A route is a maximal run of customers.  Positions refer to the current canonical row, P = 1 + last customer position:
+ *   type 0, 2-opt inside a route: reverse positions i+1..j (j >= i+2), all customers of one route.
+ *   type 1, relocate: move the customer at i onto the edge (t_j, t_j+1), j < P, j not i-1 or i; feasible within its
+ *           route, or if the target route's load + its demand <= capacity.  A route emptied by the move disappears.
+ *   type 2, swap: exchange the customers at i < j of two different routes; both new loads <= capacity.
+ *   type 3, 2-opt*: cut positions i < j (a route's depot position or a customer) of different routes A and B;
+ *           A' = A[..i] + B(j..] takes A's slot, B' = B[..j] + A(i..] takes B's; both loads <= capacity; an empty
+ *           result disappears, so two routes can merge.  No move opens a route.
+ * Gains are added minus removed edges of d (the reward's seglen, rint()-ed when round_edges is set).  Every iteration
+ * evaluates every admissible move and applies the smallest gain, ties to the lowest type*L^2 + i*L + j, if it is below
+ * -1e-6, at most max_iterations times.  length is the closed length of the returned row as elg_tour_length sums it.
+ * N1 <= 8192 (shared memory: 12*N1 + 8*L bytes). */
+int elg_cvrp_local_search(const float* xy, int Bxy, int N1, const int32_t* demand, int32_t capacity, const int32_t* inst,
+                          int16_t* tours, int R, int L, int round_edges, int max_iterations, int32_t* iterations,
+                          float* length, void* stream);
 
 /* ---- training path (REINFORCE with the POMO shared baseline) ----------------------------------
  * Replaces the body of the reference's training loop, CVRP/train.py:104-125 (TSP/train.py:100-122):
