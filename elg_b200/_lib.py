@@ -69,6 +69,7 @@ SYMBOLS = {
     "elg_tour_length": (_I, [_P, _I, _P, _I, _I, _I, _I, _I, _P, _P]),
     "elg_two_opt": (_I, [_I, _P, _I, _I, _P, _P, _I, _I, _I, _I, _P, _P, _P]),
     "elg_cvrp_local_search": (_I, [_P, _I, _I, _P, _I, _P, _P, _I, _I, _I, _I, _P, _P, _P]),
+    "elg_tsp_local_search": (_I, [_P, _I, _I, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P]),
     "elg_train_saved_bytes": (_SZ, [C.POINTER(ModelDesc), _I, _I]),
     "elg_encode_train": (_I, [C.POINTER(ModelDesc), _P, _P, C.POINTER(Tables), _I, _I, _P, _SZ, _P]),
     "elg_train_workspace_bytes": (_SZ, [C.POINTER(ModelDesc), _I, _I, _I, _I, _I]),

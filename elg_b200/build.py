@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libelg_b200.so")
 SOURCES = ["model.cu", "problems.cu", "encoder.cu", "rollout.cu", "rollout_tc.cu", "rollout_stc.cu", "selftest.cu", "train_decode.cu",
-           "train_bwd.cu", "generate.cu", "two_opt.cu", "cvrp_ls.cu"]
+           "train_bwd.cu", "generate.cu", "two_opt.cu", "cvrp_ls.cu", "tsp_ls.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--fmad=true"]
 

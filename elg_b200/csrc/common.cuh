@@ -116,7 +116,7 @@ __device__ __forceinline__ float seglen(float dx, float dy) {
   return __fsqrt_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)));
 }
 
-// ---- local search (two_opt.cu, cvrp_ls.cu) ----------------------------------------------------
+// ---- local search (two_opt.cu, cvrp_ls.cu, tsp_ls.cu) ----------------------------------------------------
 constexpr float LS_MIN_GAIN = -1e-6f;  // a move is applied only if its gain is below this
 
 // d(a, b) of nodes a, b: the reward's seglen, rint()-ed under the library metric
@@ -145,6 +145,13 @@ __device__ __forceinline__ void cta_min_gain(float& bg, int& bkey, float* red_g,
   bg = red_g[0]; bkey = red_k[0];
   for (int w = 1; w < nwarps; ++w)
     if (gain_better(red_g[w], red_k[w], bg, bkey)) { bg = red_g[w]; bkey = red_k[w]; }
+}
+
+// reverses row[a..b] with the threads of the CTA; the caller synchronises
+__device__ __forceinline__ void reverse_span(int16_t* row, int a, int b) {
+  for (int k = threadIdx.x; k < (b - a + 1) / 2; k += blockDim.x) {
+    const int16_t t = row[a + k]; row[a + k] = row[b - k]; row[b - k] = t;
+  }
 }
 
 // Swizzled column of the score matrix E' (row j): XOR the 16-byte chunk index with (j & 7) so

@@ -24,13 +24,6 @@ namespace elg {
 
 constexpr int CVRP_LS_CHUNK = 16;   // positions j per task
 
-// reverses row[a..b]; the caller synchronises
-__device__ __forceinline__ void reverse_span(int16_t* row, int a, int b) {
-  for (int k = threadIdx.x; k < (b - a + 1) / 2; k += blockDim.x) {
-    const int16_t t = row[a + k]; row[a + k] = row[b - k]; row[b - k] = t;
-  }
-}
-
 // rs and pref of positions lo..hi, where row[lo] == 0 and position hi+1 starts a route or is L.  One segmented scan over
 // contiguous per-thread slices: the carry of a slice is (last depot position in it or -1, demand after that depot).
 __device__ __forceinline__ void rebuild_routes(const int16_t* row, const int32_t* dem, int16_t* rs, int32_t* pref, int lo, int hi, int L,

@@ -89,6 +89,7 @@ if __name__ == "__main__":
     import yaml
     with open('config.yml', 'r', encoding='utf-8') as f:
         config = yaml.load(f.read(), Loader=yaml.FullLoader)
+    drv.reject_tsp_local_search(config)
     device = "cuda:{}".format(config['cuda_device_num'])
     model = load_model(config, device)
     env = CVRPEnv(multi_width=config['params']['multiple_width'], device=device)

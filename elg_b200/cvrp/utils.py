@@ -76,11 +76,13 @@ def batched_two_opt_torch(points, tour, max_iterations=1000, device=None):
     return _two_opt_dropin("cvrp", points, tour, max_iterations, device)
 
 
-def _two_opt_dropin(problem, points, tour, max_iterations, device):
-    """Shared body of the cvrp / tsp batched_two_opt_torch: conversion in and out of numpy / torch, closed tsp tours."""
+def _two_opt_dropin(problem, points, tour, max_iterations, device, max_segment=None):
+    """Shared body of the cvrp / tsp batched_two_opt_torch and, with max_segment set, of tsp.tsp_local_search (2-opt
+    and Or-opt): conversion in and out of numpy / torch, closed tsp tours."""
+    name = "batched_two_opt_torch" if max_segment is None else "tsp_local_search"
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     if dev.type != "cuda":
-        raise _lib.ElgError("batched_two_opt_torch needs a CUDA device (got %s): elg_b200 has no CPU path" % dev)
+        raise _lib.ElgError("%s needs a CUDA device (got %s): elg_b200 has no CPU path" % (name, dev))
     as_numpy = isinstance(tour, np.ndarray)
     t = torch.as_tensor(tour)
     out_dtype, out_dev = t.dtype, t.device
@@ -89,7 +91,11 @@ def _two_opt_dropin(problem, points, tour, max_iterations, device):
     if problem == "tsp":
         if t.dim() != 2 or t.shape[1] < 2 or not bool((t[:, -1] == t[:, 0]).all()):
             raise ValueError("tsp tours must be (batch, N+1) closed tours (last node = first node)")
-        refined, _, iters = engine.two_opt("tsp", xy, t[:, :-1].contiguous(), max_iterations=max_iterations)
+        if max_segment is None:
+            refined, _, iters = engine.two_opt("tsp", xy, t[:, :-1].contiguous(), max_iterations=max_iterations)
+        else:
+            refined, _, iters = engine.tsp_local_search(xy, t[:, :-1].contiguous(), max_iterations=max_iterations,
+                                                        max_segment=max_segment)
         refined = torch.cat((refined, refined[:, :1]), dim=1)
     else:
         refined, _, iters = engine.two_opt("cvrp", xy, t, max_iterations=max_iterations)

@@ -345,6 +345,50 @@ def two_opt(problem, xy, tours, inst=None, max_iterations=1000, rounding=False):
     return t16.long(), length, iters
 
 
+def tsp_local_search(xy, tours, inst=None, max_iterations=1000, max_segment=3, rounding=False):
+    """Best-improvement TSP local search with 2-opt and Or-opt moves (elg_tsp_local_search; semantics in
+    include/elg_b200.h), one launch for all tours.
+
+    xy (Bxy, N1, 2) coordinates; tours (R, L) int16 or int64 with a permutation of 0..N1-1 in positions 0..N1-1 (L >= N1;
+    the rest is left as it is); inst (R,) picks the xy instance of every tour (default: tour r uses xy[r], or xy[0] when
+    Bxy == 1); max_segment (0..3) the longest Or-opt segment, 0 being plain 2-opt; rounding rint()s every edge (library
+    metric).  Position 0 never moves.  Returns (tours int64 (R, L), length (R,) as tour_length measures it,
+    iterations (R,) moves applied)."""
+    if tours.dim() != 2 or xy.dim() != 3 or xy.shape[2] != 2:
+        raise ValueError("tours must be (R, L) and xy (Bxy, N1, 2)")
+    R, L = tours.shape
+    Bxy, N1 = int(xy.shape[0]), int(xy.shape[1])
+    if L < N1:
+        raise ValueError("tours need at least N1 = %d positions (got %d)" % (N1, L))
+    if max_iterations < 0:
+        raise ValueError("max_iterations must be >= 0")
+    if max_segment not in (0, 1, 2, 3):
+        raise ValueError("max_segment must be 0, 1, 2 or 3 (got %r)" % (max_segment,))
+    dev = tours.device
+    if inst is not None:
+        inst = torch.as_tensor(inst, device=dev).to(torch.int32).contiguous()
+        if inst.shape != (R,) or (R and (int(inst.min()) < 0 or int(inst.max()) >= Bxy)):
+            raise ValueError("inst must be (R,) indices into the %d xy instances" % Bxy)
+    elif Bxy not in (1, R):
+        raise ValueError("without inst, xy must hold 1 or R instances (got %d for %d rows)" % (Bxy, R))
+    if R and N1:
+        t = tours[:, :N1].long()
+        if int(t.min()) < 0 or int(t.max()) >= N1:
+            raise ValueError("tour node ids must lie in [0, %d)" % N1)
+        if not torch.equal(t.sort(1)[0], torch.arange(N1, device=dev).expand(R, -1)):
+            raise ValueError("positions 0..%d of every tour must hold a permutation of the nodes" % (N1 - 1))
+    _require_cuda(xy, "xy")
+    _require_cuda(tours, "tours")
+    t16 = tours.to(torch.int16, copy=True).contiguous()
+    length = torch.empty(R, dtype=torch.float32, device=dev)
+    iters = torch.empty(R, dtype=torch.int32, device=dev)
+    xy = xy.contiguous().float()
+    with torch.cuda.device(dev):
+        check(lib.elg_tsp_local_search(_ptr(xy), Bxy, N1, _ptr(inst), _ptr(t16), R, L, int(max_segment),
+                                       1 if rounding else 0, int(max_iterations), _ptr(iters), _ptr(length), _stream(dev)))
+    return t16.long(), length, iters
+
+
 def cvrp_local_search(xy, tours, demand, capacity, inst=None, max_iterations=1000, rounding=False):
     """Capacity-aware best-improvement CVRP local search (elg_cvrp_local_search; semantics in include/elg_b200.h): 2-opt
     inside a route, relocate, swap and 2-opt* between routes, one launch for all rows.

@@ -17,6 +17,12 @@ the 2-opt stage and run on the same rows: solve_instance refines them with engin
 (with the capacity CVRPEnv.load_vrplib_problem recorded), InstanceCost.local_search carries the result, fill_record adds
 best_cost_ls / gap_ls / ls_seconds / ls_iterations, and run_set / gap_bins print their lines after the 2-opt ones.
 load_model rejects the key for a TSP model.
+
+Optional TSP local search stage (config params.tsp_local_search_iterations; absent or 0: nothing changes): 2-opt and
+Or-opt moves (engine.tsp_local_search), independent of the 2-opt stage and run on the same rows in the library metric;
+InstanceCost.tsp_local_search carries the result, fill_record adds best_cost_tsp_ls / gap_tsp_ls / tsp_ls_seconds /
+tsp_ls_iterations, and run_set / gap_bins print their lines after the 2-opt ones.  load_model rejects the key for a CVRP
+model.
 """
 import json
 import os
@@ -41,6 +47,8 @@ def load_model(model_cls, config, device, model=None, needs_local=True):
     from .cvrp.CVRPModel import CVRPModel
     if not issubclass(model_cls, CVRPModel):
         reject_local_search(config)
+    else:
+        reject_tsp_local_search(config)
     if model is None:
         model = model_cls(**config['model_params'])
         if needs_local:
@@ -51,6 +59,7 @@ def load_model(model_cls, config, device, model=None, needs_local=True):
     model.requires_grad_(False)
     model._elg_two_opt_iterations = config.get('params', {}).get('two_opt_iterations') or 0
     model._elg_local_search_iterations = config.get('params', {}).get('local_search_iterations') or 0
+    model._elg_tsp_local_search_iterations = config.get('params', {}).get('tsp_local_search_iterations') or 0
     return model
 
 
@@ -61,15 +70,24 @@ def reject_local_search(config):
                          "refine TSP tours with params.two_opt_iterations")
 
 
+def reject_tsp_local_search(config):
+    """The CVRP drivers: params.tsp_local_search_iterations is the TSP search, CVRP rows have their own local search."""
+    if config.get('params', {}).get('tsp_local_search_iterations'):
+        raise ValueError("params.tsp_local_search_iterations is the TSP 2-opt + Or-opt local search; "
+                         "refine CVRP rows with params.local_search_iterations")
+
+
 class InstanceCost(float):
-    """Best cost of one instance (a plain float to every caller).  `two_opt` / `local_search` are (refined cost, seconds,
-    moves) when the optional stage ran, else None."""
+    """Best cost of one instance (a plain float to every caller).  `two_opt` / `local_search` / `tsp_local_search` are
+    (refined cost, seconds, moves) when the optional stage ran, else None."""
     two_opt = None
     local_search = None
+    tsp_local_search = None
 
 
 # optional refinement stages: (InstanceCost attribute, record key suffix, record key prefix, name in the printouts)
-_STAGES = (('two_opt', '2opt', 'two_opt', '2-opt'), ('local_search', 'ls', 'ls', 'local search'))
+_STAGES = (('two_opt', '2opt', 'two_opt', '2-opt'), ('local_search', 'ls', 'ls', 'local search'),
+           ('tsp_local_search', 'tsp_ls', 'tsp_ls', '2-opt + or-opt'))
 
 
 def _best_rows(solutions, rewards):
@@ -92,6 +110,14 @@ def local_search_refine(xy, demand, capacity, solutions, rewards, aug_factor, it
     rows = _best_rows(solutions, rewards)
     return _timed_refine(lambda: engine.cvrp_local_search(xy, rows, demand, capacity, max_iterations=iterations,
                                                           rounding=rounding), aug_factor)
+
+
+def tsp_local_search_refine(xy, solutions, rewards, aug_factor, iterations, rounding):
+    """TSP 2-opt + Or-opt local search (engine.tsp_local_search, one launch) of the best POMO row of every aug-instance
+    of a greedy rollout; as two_opt_refine."""
+    rows = _best_rows(solutions, rewards)
+    return _timed_refine(lambda: engine.tsp_local_search(xy, rows, max_iterations=iterations, rounding=rounding),
+                         aug_factor)
 
 
 def _timed_refine(run, aug_factor):
@@ -127,6 +153,11 @@ def solve_instance(model, env, rollout, aug_factor, width):
         refined, seconds, moves = local_search_refine(env.unscaled_depot_node_xy, env.depot_node_demand, env.capacity,
                                                       solutions, rewards, aug_factor, iterations, rounding=True)
         cost.local_search = (float(refined[0]), seconds, int(moves[0]))
+    iterations = getattr(model, '_elg_tsp_local_search_iterations', 0)
+    if iterations:
+        refined, seconds, moves = tsp_local_search_refine(env._unscaled_dev, solutions, rewards, aug_factor, iterations,
+                                                          rounding=True)
+        cost.tsp_local_search = (float(refined[0]), seconds, int(moves[0]))
     return cost, solutions, rewards
 
 
@@ -168,7 +199,7 @@ def fill_record(record, best_cost, scale, optimal):
 def gap_bins(results, edges):
     """edges: [(label, lo_exclusive, hi_inclusive)] on the instance scale -> {label: mean gap in %}, plus 'total'.
     When the records carry an optional stage, also prints one line per bin and a total line for it, and adds
-    'gap_2opt' / 'gap_ls': {label: mean gap in %}."""
+    'gap_2opt' / 'gap_ls' / 'gap_tsp_ls': {label: mean gap in %}."""
     out = _bin_means(results, edges, 'gap')
     for _, suffix, _, name in _STAGES:
         key = 'gap_' + suffix

@@ -30,13 +30,16 @@ def solve_batch(model, env, batch, aug_factor):
     return no_aug_cost, aug_cost, solutions, rewards
 
 
-def test(dataloader, model, env, aug_factor, two_opt_iterations=0):
+def test(dataloader, model, env, aug_factor, two_opt_iterations=0, tsp_local_search_iterations=0):
     """two_opt_iterations > 0 (config params.two_opt_iterations) also refines the best POMO row of every aug-instance
-    with 2-opt in the reward metric and prints the refined cost after the reference's lines."""
+    with 2-opt in the reward metric and prints the refined cost after the reference's lines.
+    tsp_local_search_iterations > 0 (params.tsp_local_search_iterations) does the same with the 2-opt + Or-opt local
+    search, independently of the 2-opt stage."""
     model.eval()
     model.requires_grad_(False)
     avg_cost_total, no_avg_cost_total, t = 0., 0., 0
     two_opt_cost, two_opt_seconds, two_opt_moves = 0., 0., 0
+    ls_cost, ls_seconds, ls_moves = 0., 0., 0
     start = time.time()
     for batch in dataloader:
         no_aug_cost, aug_cost, solutions, rewards = solve_batch(model, env, batch, aug_factor)
@@ -48,6 +51,12 @@ def test(dataloader, model, env, aug_factor, two_opt_iterations=0):
             two_opt_cost += cost.mean()
             two_opt_seconds += seconds
             two_opt_moves += int(moves.sum())
+        if tsp_local_search_iterations:
+            cost, seconds, moves = drv.tsp_local_search_refine(env.problems, solutions, rewards, aug_factor,
+                                                               tsp_local_search_iterations, rounding=False)
+            ls_cost += cost.mean()
+            ls_seconds += seconds
+            ls_moves += int(moves.sum())
         t += 1
     torch.cuda.synchronize()
     end = time.time()
@@ -57,6 +66,9 @@ def test(dataloader, model, env, aug_factor, two_opt_iterations=0):
     print("no aug Avg cost: {:.4f}, Wall-clock time: {:.2f}s".format(no_avg_cost_total, float(end - start)))
     if two_opt_iterations:
         print("2-opt Aug cost: {:.4f}, 2-opt time: {:.2f}s, moves: {}".format(two_opt_cost / t, two_opt_seconds, two_opt_moves))
+    if tsp_local_search_iterations:
+        print("2-opt + or-opt Aug cost: {:.4f}, 2-opt + or-opt time: {:.2f}s, moves: {}".format(ls_cost / t, ls_seconds,
+                                                                                                  ls_moves))
     return avg_cost_total
 
 
@@ -85,4 +97,5 @@ if __name__ == "__main__":
     bs = config['params']['test_batch_size']
     batches = [torch.FloatTensor(data[i:i + bs]) for i in range(0, len(data), bs)]
     test(batches, model, env, aug_factor=config['params']['aug_factor'],
-         two_opt_iterations=config['params'].get('two_opt_iterations') or 0)
+         two_opt_iterations=config['params'].get('two_opt_iterations') or 0,
+         tsp_local_search_iterations=config['params'].get('tsp_local_search_iterations') or 0)

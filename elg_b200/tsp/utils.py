@@ -1,4 +1,5 @@
-"""Drop-in for the reference's TSP/utils.py: rollout (TSP/utils.py:7-26), 2-opt, x8 augmentation, seeding."""
+"""Drop-in for the reference's TSP/utils.py: rollout (TSP/utils.py:7-26), 2-opt, x8 augmentation, seeding; plus the
+2-opt + Or-opt local search tsp_local_search."""
 import random
 
 import numpy as np
@@ -53,6 +54,17 @@ def batched_two_opt_torch(points, tour, max_iterations=1000, device=None):
     understood to be.  One deliberate difference: every tour stops on its own, where the reference's loop couples the
     batch and runs while any tour improves."""
     return _two_opt_dropin("tsp", points, tour, max_iterations, device)
+
+
+def tsp_local_search(points, tour, max_iterations=1000, max_segment=3, device=None):
+    """2-opt + Or-opt local search on closed TSP tours, on the GPU (elg_tsp_local_search): best improvement over 2-opt
+    and the moves of a segment of 1..max_segment consecutive nodes, forward or reversed, onto another edge; every tour
+    stops on its own.  max_segment = 0 is batched_two_opt_torch.
+
+    points (N, 2); tour (batch, N+1) closed tours (last node = first node); numpy or torch, and the result comes back in
+    the same type and dtype.  Returns (tour, iterations), iterations being the largest number of moves any tour took.
+    Position 0 (the start node) never moves.  device=None is the current CUDA device; there is no CPU path."""
+    return _two_opt_dropin("tsp", points, tour, max_iterations, device, max_segment=max_segment)
 
 
 def check_feasible(pi):

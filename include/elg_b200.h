@@ -30,8 +30,9 @@ extern "C" {
 #endif
 
 #define ELG_ABI_VERSION 4   /* 2: training path, data generators; 3: elg_tables.et / .ws (streamed tensor-core decode);
-                               4: elg_two_opt, then elg_cvrp_local_search (purely additive, so the version stays 4:
-                                  a library without it fails on the missing symbol when the binding loads) */
+                               4: elg_two_opt, then elg_cvrp_local_search, then elg_tsp_local_search (purely additive,
+                                  so the version stays 4: a library without one fails on the missing symbol when the
+                                  binding loads) */
 
 enum { ELG_TSP = 0, ELG_CVRP = 1 };
 enum { ELG_GREEDY = 0, ELG_SAMPLE = 1 };
@@ -240,6 +241,27 @@ int elg_tour_length(const float* xy, int Bxy, const int64_t* tours, int B, int M
  *   iterations [R]    moves applied;  length [R]  closed length of the refined tour, summed as elg_tour_length sums it */
 int elg_two_opt(int problem, const float* xy, int Bxy, int N1, const int32_t* inst, int16_t* tours, int R, int L,
                 int round_edges, int max_iterations, int32_t* iterations, float* length, void* stream);
+
+/* ---- TSP local search: 2-opt and Or-opt ------------------------------------------------------------
+ * Best-improvement local search on R TSP tours, refined in place; every tour stops on its own.
+ *   xy, Bxy, N1, inst, tours [R][L], round_edges, max_iterations, iterations [R]: as elg_two_opt with problem = ELG_TSP
+ *   (positions 0..N1-1 a permutation, closed implicitly; positions N1.. ignored and left as they are; position 0 never
+ *   moves).  d is the reward's seglen, rint()-ed per edge when round_edges is set; e_p = d(t_p, t_p+1), p+1 wrapping to 0.
+ * Move variants, keyed v*N1^2 + i*N1 + j:
+ *   v = 0, 2-opt, exactly the TSP move of elg_two_opt: i < j, j >= i+2, not (0, N1-1); reverses positions i+1..j;
+ *          gain (d(t_i,t_j) - e_i) + (d(t_i+1,t_j+1) - e_j).
+ *   v = 1..5, Or-opt: move the segment at positions i..i+s-1 onto the edge (t_j, t_j+1); v = 1: s = 1; v = 2 / 3: s = 2
+ *          forward / reversed; v = 4 / 5: s = 3 forward / reversed.  Admissible for 1 <= i, i+s-1 <= N1-1 and
+ *          j in 0..N1-1 outside {i-1, .., i+s-1} (either side of the segment); only s <= max_segment (0..3) is evaluated.
+ *          Gain ((d(t_i-1, t_i+s) - e_i-1) - e_i+s-1) + ((d(t_j, a) - e_j) + d(b, t_j+1)), i+s wrapping to 0, with
+ *          (a, b) = (t_i, t_i+s-1) forward and (t_i+s-1, t_i) reversed.
+ * Gains are fp32 in the order written.  Every iteration evaluates every admissible variant and applies the smallest gain,
+ * ties to the lowest key, if it is below -1e-6, at most max_iterations times.  max_segment = 0 is elg_two_opt(ELG_TSP)
+ * bit for bit.  length is the closed length of the returned tour as elg_tour_length sums it.
+ * N1 <= 8192 (shared memory: 14*N1 bytes). */
+int elg_tsp_local_search(const float* xy, int Bxy, int N1, const int32_t* inst, int16_t* tours, int R, int L,
+                         int max_segment, int round_edges, int max_iterations, int32_t* iterations, float* length,
+                         void* stream);
 
 /* ---- capacity-aware CVRP local search ------------------------------------------------------------
  * Best-improvement local search on R CVRP solutions, refined in place; every row stops on its own.
