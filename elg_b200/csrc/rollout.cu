@@ -29,6 +29,50 @@
 
 namespace elg {
 
+// Sampled decision of one row (one warp; node j = lane + 32 ch of the row's masked logits lg, N1 <= 128), the draw
+// elg_rollout and elg_decode_step document: u = ((x >> 8) + 0.5) 2^-24, x the first word of Philox4x32-10 at counter
+// (grow lo, grow hi, step lo, step hi) and key (seed lo, seed hi); the pick is the first node in index order with p > 0
+// and running sum >= u * total.  The total (butterfly) and the running sums (scan) round differently, so at u = 1 the
+// last running sum can end one ulp below u * total: the last node of positive probability is then the pick.
+// samp / selp are written only when the row has a node of positive probability.
+__device__ __forceinline__ void sample_row(const float (&lg)[4], float best, unsigned long long seed, unsigned long long grow,
+                                           unsigned long long step, int lane, int& samp, float& selp) {
+  float bv = best;
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) bv = fmaxf(bv, __shfl_xor_sync(FULL, bv, off));
+  float pr[4], tot = 0.f;
+#pragma unroll
+  for (int ch = 0; ch < 4; ++ch) { pr[ch] = lg[ch] == -INFINITY ? 0.f : expf(lg[ch] - bv); tot += pr[ch]; }
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) tot += __shfl_xor_sync(FULL, tot, off);
+  const uint4 rnd = philox4x32(make_uint4((uint32_t)grow, (uint32_t)(grow >> 32), (uint32_t)step, (uint32_t)(step >> 32)),
+                               make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+  const float target = ((rnd.x >> 8) + 0.5f) * (1.f / 16777216.f) * tot;
+  float run = 0.f, pickp = 0.f;
+  int pick = -1, last = -1;
+#pragma unroll
+  for (int ch = 0; ch < 4; ++ch) {
+    float inc = pr[ch];
+#pragma unroll
+    for (int off = 1; off < 32; off <<= 1) {
+      const float nb = __shfl_up_sync(FULL, inc, off);
+      if (lane >= off) inc += nb;
+    }
+    const float cum = run + inc;
+    const uint32_t hit = __ballot_sync(FULL, pr[ch] > 0.f && cum >= target);
+    const uint32_t pos = __ballot_sync(FULL, pr[ch] > 0.f);
+    if (pick < 0 && pos) {          // the first hit, else this chunk's last node of positive probability
+      const int src = hit ? __ffs(hit) - 1 : 31 - __clz(pos);
+      last = src + 32 * ch;
+      pickp = __shfl_sync(FULL, pr[ch], src);
+      if (hit) pick = last;
+    }
+    run += __shfl_sync(FULL, inc, 31);
+  }
+  if (pick < 0) pick = last;
+  if (pick >= 0) { samp = pick; selp = pickp / tot; }
+}
+
 // ---- shared-memory layout (offsets in floats) ---------------------------------------------------
 struct SmemLayout {
   int k, v, e, o, eb, xy, dem, wl, u, tt, a, vpe, pw, pb, zw, zb;
@@ -701,41 +745,9 @@ __global__ void __launch_bounds__(RT, 1) rollout_kernel(const RolloutArgs A) {
                   for (int ch = 0; ch < 4; ++ch)
                     if (lane + 32 * ch < N1) lo[lane + 32 * ch] = lg[ch];
                 }
-                if (A.mode == ELG_SAMPLE) {       // host guarantees N1 <= 128 (one chunk) in this mode
-                  float bv = best[i];
-#pragma unroll
-                  for (int off = 16; off > 0; off >>= 1) bv = fmaxf(bv, __shfl_xor_sync(FULL, bv, off));
-                  float pr[4], tot = 0.f;
-#pragma unroll
-                  for (int ch = 0; ch < 4; ++ch) { pr[ch] = lg[ch] == -INFINITY ? 0.f : expf(lg[ch] - bv); tot += pr[ch]; }
-#pragma unroll
-                  for (int off = 16; off > 0; off >>= 1) tot += __shfl_xor_sync(FULL, tot, off);
-                  const unsigned long long grow = (unsigned long long)b * A.M + row0 + r;
-                  const unsigned long long stp = A.single_step ? A.step_id : (unsigned long long)t;
-                  const uint4 rnd = philox4x32(make_uint4((uint32_t)grow, (uint32_t)(grow >> 32), (uint32_t)stp, (uint32_t)(stp >> 32)),
-                                               make_uint2((uint32_t)A.seed, (uint32_t)(A.seed >> 32)));
-                  const float target = ((rnd.x >> 8) + 0.5f) * (1.f / 16777216.f) * tot;
-                  float run = 0.f, pickp = 0.f;
-                  int pick = -1;
-#pragma unroll
-                  for (int ch = 0; ch < 4; ++ch) {
-                    float inc = pr[ch];
-#pragma unroll
-                    for (int off = 1; off < 32; off <<= 1) {
-                      const float nb = __shfl_up_sync(FULL, inc, off);
-                      if (lane >= off) inc += nb;
-                    }
-                    const float cum = run + inc;
-                    const uint32_t hit = __ballot_sync(FULL, pr[ch] > 0.f && cum >= target);
-                    if (pick < 0 && hit) {
-                      const int src = __ffs(hit) - 1;
-                      pick = src + 32 * ch;
-                      pickp = __shfl_sync(FULL, pr[ch], src);
-                    }
-                    run += __shfl_sync(FULL, inc, 31);
-                  }
-                  if (pick >= 0) { samp[i] = pick; selp[i] = pickp / tot; }
-                }
+                if (A.mode == ELG_SAMPLE)         // host guarantees N1 <= 128 (one chunk) in this mode
+                  sample_row(lg, best[i], A.seed, (unsigned long long)b * A.M + row0 + r,
+                             A.single_step ? A.step_id : (unsigned long long)t, lane, samp[i], selp[i]);
               }
             }
           }
@@ -812,41 +824,9 @@ __global__ void __launch_bounds__(RT, 1) rollout_kernel(const RolloutArgs A) {
                   for (int ch = 0; ch < 4; ++ch)
                     if (c0n + lane + 32 * ch < N1) lo[c0n + lane + 32 * ch] = lg[ch];
                 }
-                if (A.mode == ELG_SAMPLE) {       // host guarantees N1 <= 128 (one chunk) in this mode
-                  float bv = best[i];
-#pragma unroll
-                  for (int off = 16; off > 0; off >>= 1) bv = fmaxf(bv, __shfl_xor_sync(FULL, bv, off));
-                  float pr[4], tot = 0.f;
-#pragma unroll
-                  for (int ch = 0; ch < 4; ++ch) { pr[ch] = lg[ch] == -INFINITY ? 0.f : expf(lg[ch] - bv); tot += pr[ch]; }
-#pragma unroll
-                  for (int off = 16; off > 0; off >>= 1) tot += __shfl_xor_sync(FULL, tot, off);
-                  const unsigned long long grow = (unsigned long long)b * A.M + row0 + r;
-                  const unsigned long long stp = A.single_step ? A.step_id : (unsigned long long)t;
-                  const uint4 rnd = philox4x32(make_uint4((uint32_t)grow, (uint32_t)(grow >> 32), (uint32_t)stp, (uint32_t)(stp >> 32)),
-                                               make_uint2((uint32_t)A.seed, (uint32_t)(A.seed >> 32)));
-                  const float target = ((rnd.x >> 8) + 0.5f) * (1.f / 16777216.f) * tot;
-                  float run = 0.f, pickp = 0.f;
-                  int pick = -1;
-#pragma unroll
-                  for (int ch = 0; ch < 4; ++ch) {
-                    float inc = pr[ch];
-#pragma unroll
-                    for (int off = 1; off < 32; off <<= 1) {
-                      const float nb = __shfl_up_sync(FULL, inc, off);
-                      if (lane >= off) inc += nb;
-                    }
-                    const float cum = run + inc;
-                    const uint32_t hit = __ballot_sync(FULL, pr[ch] > 0.f && cum >= target);
-                    if (pick < 0 && hit) {
-                      const int src = __ffs(hit) - 1;
-                      pick = src + 32 * ch;
-                      pickp = __shfl_sync(FULL, pr[ch], src);
-                    }
-                    run += __shfl_sync(FULL, inc, 31);
-                  }
-                  if (pick >= 0) { samp[i] = pick; selp[i] = pickp / tot; }
-                }
+                if (A.mode == ELG_SAMPLE)         // host guarantees N1 <= 128 (one chunk) in this mode
+                  sample_row(lg, best[i], A.seed, (unsigned long long)b * A.M + row0 + r,
+                             A.single_step ? A.step_id : (unsigned long long)t, lane, samp[i], selp[i]);
               }
             }
             __syncwarp();
@@ -866,7 +846,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_kernel(const RolloutArgs A) {
               if (ov > bv || (ov == bv && oi < bi)) { bv = ov; bi = oi; }
             }
             int choice = live ? bi : 0;
-            if (A.mode == ELG_SAMPLE && live && samp[i] >= 0) choice = samp[i];     // else (rounding fell off the end): the mode
+            if (A.mode == ELG_SAMPLE && live && samp[i] >= 0) choice = samp[i];     // else (no node of positive probability): the mode
             sel[i] = choice;
           }
         }

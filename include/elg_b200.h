@@ -182,7 +182,13 @@ int elg_encode(const elg_model_desc* desc, const float* weights, const float* de
  *   logp [B][M]          sample mode: sum of log-probabilities of the sampled actions (may be NULL)
  *   work_counter         one zero-initialised int32 (dynamic CTA scheduler)
  * elg_rollout_tiles() returns the number of row tiles per aug-instance used for (B, M, N1);
- * elg_nbr_bytes() / elg_e_bytes() the sizes of elg_tables.nbr / .e.  Sampling mode needs N1 <= 128. */
+ * elg_nbr_bytes() / elg_e_bytes() the sizes of elg_tables.nbr / .e.  Sampling mode needs N1 <= 128.
+ * Sampled decision (elg_rollout and elg_decode_step, mode = ELG_SAMPLE) of row m of aug-instance b: x = word 0 of
+ * Philox4x32-10 with counter (grow lo, grow hi, step lo, step hi), grow = b*M + m, and key (seed lo, seed hi);
+ * u = ((x >> 8) + 0.5f) * 2^-24 in fp32, in [2^-25, 1]; the pick is the first node in node-index order with p > 0 and
+ * running sum of p >= u * sum of p (inverse CDF of softmax(logits)), or the last node with p > 0 when fp32 rounding
+ * leaves every running sum below u * sum.  elg_rollout uses the tour position t as the step (cvrp: t = 0 depot and
+ * t = 1 start node are forced, sampled from t = 2; tsp: sampled from t = 1); elg_decode_step uses its step argument. */
 int elg_rollout_tiles(const elg_model_desc* desc, int B, int M, int N1);
 int elg_rollout_resident(const elg_model_desc* desc, int N1);   /* 1 = resident variant, 0 = streaming, <0 = error */
 size_t elg_nbr_bytes(const elg_model_desc* desc, int B, int N1);
