@@ -154,6 +154,58 @@ __device__ __forceinline__ void reverse_span(int16_t* row, int a, int b) {
   }
 }
 
+// xy instance of row r: inst[r], else 0 when one instance is shared by all rows, else r
+__device__ __forceinline__ int ls_instance(const int32_t* __restrict__ inst, int Bxy, int r) {
+  return inst ? inst[r] : (Bxy == 1 ? 0 : r);
+}
+
+// Result of row r: the n positions of `tour` back to `row`; length[r] = edge[0..n-1] summed in the order of
+// tour_length_kernel (sequential from the edge leaving position 0, on thread 0); iterations[r] = moves.  tour and edge
+// must be final (behind a barrier); the closing barrier lets the next row reuse shared memory.  nthr is the kernel's
+// blockDim.x: reading it again here costs tsp_ls_kernel a register.
+__device__ __forceinline__ void ls_store_row(const int16_t* tour, const float* edge, int n, int16_t* __restrict__ row,
+                                             int r, int moves, float* __restrict__ length,
+                                             int32_t* __restrict__ iterations, int nthr) {
+  for (int p = threadIdx.x; p < n; p += nthr) row[p] = tour[p];
+  if (threadIdx.x == 0) {
+    float sum = 0.f;
+    for (int p = 0; p < n; ++p) sum += edge[p];
+    length[r] = sum;
+    iterations[r] = moves;
+  }
+  __syncthreads();
+}
+
+// The checks every local-search entry point makes; `what` names the search in the messages.
+inline int ls_check_args(const char* what, const float* xy, int Bxy, int N1, const int32_t* inst, const int16_t* tours,
+                         int R, int max_iterations, const int32_t* iterations, const float* length) {
+  ELG_REQUIRE(N1 > 0 && R >= 0 && Bxy > 0, ELG_EINVAL, "bad sizes N1=%d R=%d Bxy=%d", N1, R, Bxy);
+  ELG_REQUIRE(N1 <= ELG_MAX_NODES, ELG_EUNSUPPORTED, "%s supports up to %d nodes (got %d)", what, ELG_MAX_NODES, N1);
+  ELG_REQUIRE(max_iterations >= 0, ELG_EINVAL, "max_iterations must be >= 0 (got %d)", max_iterations);
+  ELG_REQUIRE(xy && tours && iterations && length, ELG_EINVAL, "NULL pointer");
+  ELG_REQUIRE(inst || Bxy == 1 || Bxy == R, ELG_EINVAL, "without inst the xy batch must be 1 or R (Bxy=%d, R=%d)", Bxy, R);
+  return ELG_OK;
+}
+
+// Persistent launch of a local-search kernel over R rows: one CTA per row at a time, 256 threads for rows of at most
+// 512 positions and 512 above, as many CTAs as fit on the device (at most R).
+template <typename... Params, typename... Args>
+int ls_launch(void (*kernel)(Params...), size_t smem, int positions, int R, void* stream, const char* what, int N1, int L,
+              Args... args) {
+  if (R == 0) return ELG_OK;
+  const int threads = positions <= 512 ? 256 : 512;
+  ELG_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int dev = 0, sms = 0, per_sm = 0;
+  ELG_CUDA_OK(cudaGetDevice(&dev));
+  ELG_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  ELG_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
+  ELG_REQUIRE(per_sm > 0, ELG_EUNSUPPORTED, "%s: %zu bytes of shared memory do not fit (N1=%d, L=%d)", what, smem, N1, L);
+  const int grid = (int)((long long)R < (long long)sms * per_sm ? R : sms * per_sm);
+  kernel<<<grid, threads, smem, (cudaStream_t)stream>>>(args...);
+  ELG_LAUNCH_OK();
+  return ELG_OK;
+}
+
 // Swizzled column of the score matrix E' (row j): XOR the 16-byte chunk index with (j & 7) so
 // that 8 consecutive rows read by a quarter-warp hit 8 different bank groups.
 __host__ __device__ __forceinline__ int eswz(int j, int c) { return c ^ ((j & 7) << 2); }

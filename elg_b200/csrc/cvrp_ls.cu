@@ -80,7 +80,7 @@ __global__ void __launch_bounds__(512, 1) cvrp_ls_kernel(const float* __restrict
   const int LL = L * L;
 
   for (int r = blockIdx.x; r < R; r += gridDim.x) {
-    const int b = inst ? inst[r] : (Bxy == 1 ? 0 : r);
+    const int b = ls_instance(inst, Bxy, r);
     const float2* src_xy = reinterpret_cast<const float2*>(xy_g) + (long long)b * N1;
     const int32_t* src_dem = dem_g + (long long)b * N1;
     int16_t* grow = tours + (long long)r * L;
@@ -195,20 +195,11 @@ __global__ void __launch_bounds__(512, 1) cvrp_ls_kernel(const float* __restrict
       ++moves;
     }
 
-    // closed length in the summation order of tour_length_kernel: sequential from the edge leaving position 0
-    float* edge = reinterpret_cast<float*>(pref);       // the prefixes are not needed any more
-    for (int p = tid; p < L; p += nthr) {
-      edge[p] = edge_len(xy, row[p], row[p + 1 == L ? 0 : p + 1], round_edges);
-      grow[p] = row[p];
-    }
+    // the row has no edge array: its edges go where the prefixes were, which are not needed any more
+    float* edge = reinterpret_cast<float*>(pref);
+    for (int p = tid; p < L; p += nthr) edge[p] = edge_len(xy, row[p], row[p + 1 == L ? 0 : p + 1], round_edges);
     __syncthreads();
-    if (tid == 0) {
-      float sum = 0.f;
-      for (int p = 0; p < L; ++p) sum += edge[p];
-      length[r] = sum;
-      iterations[r] = moves;
-    }
-    __syncthreads();                                    // shared memory is reused by the next row
+    ls_store_row(row, edge, L, grow, r, moves, length, iterations, nthr);
   }
 }
 
@@ -225,29 +216,12 @@ extern "C" {
 int elg_cvrp_local_search(const float* xy, int Bxy, int N1, const int32_t* demand, int32_t capacity, const int32_t* inst,
                           int16_t* tours, int R, int L, int round_edges, int max_iterations, int32_t* iterations,
                           float* length, void* stream) {
-  ELG_REQUIRE(N1 > 0 && R >= 0 && Bxy > 0, ELG_EINVAL, "bad sizes N1=%d R=%d Bxy=%d", N1, R, Bxy);
-  ELG_REQUIRE(N1 <= ELG_MAX_NODES, ELG_EUNSUPPORTED, "cvrp local search supports up to %d nodes (got %d)", ELG_MAX_NODES,
-              N1);
+  if (int e = ls_check_args("cvrp local search", xy, Bxy, N1, inst, tours, R, max_iterations, iterations, length)) return e;
   ELG_REQUIRE(L > 0 && L <= 2 * N1 + 2, ELG_EINVAL, "rows need 0 < L <= 2*N1+2 (L=%d, N1=%d)", L, N1);
   ELG_REQUIRE(capacity > 0, ELG_EINVAL, "capacity must be > 0 (got %d)", capacity);
-  ELG_REQUIRE(max_iterations >= 0, ELG_EINVAL, "max_iterations must be >= 0 (got %d)", max_iterations);
-  ELG_REQUIRE(xy && demand && tours && iterations && length, ELG_EINVAL, "NULL pointer");
-  ELG_REQUIRE(inst || Bxy == 1 || Bxy == R, ELG_EINVAL, "without inst the xy batch must be 1 or R (Bxy=%d, R=%d)", Bxy, R);
-  if (R == 0) return ELG_OK;
-  const size_t smem = cvrp_ls_smem_bytes(N1, L);
-  const int threads = L <= 512 ? 256 : 512;
-  ELG_CUDA_OK(cudaFuncSetAttribute(cvrp_ls_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int dev = 0, sms = 0, per_sm = 0;
-  ELG_CUDA_OK(cudaGetDevice(&dev));
-  ELG_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  ELG_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, cvrp_ls_kernel, threads, smem));
-  ELG_REQUIRE(per_sm > 0, ELG_EUNSUPPORTED, "cvrp local search: %zu bytes of shared memory do not fit (N1=%d, L=%d)", smem,
-              N1, L);
-  const int grid = (int)((long long)R < (long long)sms * per_sm ? R : sms * per_sm);
-  cvrp_ls_kernel<<<grid, threads, smem, (cudaStream_t)stream>>>(xy, Bxy, N1, demand, capacity, inst, tours, R, L,
-                                                                round_edges, max_iterations, iterations, length);
-  ELG_LAUNCH_OK();
-  return ELG_OK;
+  ELG_REQUIRE(demand, ELG_EINVAL, "NULL pointer");
+  return ls_launch(cvrp_ls_kernel, cvrp_ls_smem_bytes(N1, L), L, R, stream, "cvrp local search", N1, L, xy, Bxy, N1,
+                   demand, capacity, inst, tours, R, L, round_edges, max_iterations, iterations, length);
 }
 
 }  // extern "C"

@@ -45,8 +45,7 @@ __global__ void __launch_bounds__(512, 2) tsp_ls_kernel(const float* __restrict_
   const int tasks = N1 * nch;
 
   for (int r = blockIdx.x; r < R; r += gridDim.x) {
-    const int b = inst ? inst[r] : (Bxy == 1 ? 0 : r);
-    const float2* src = reinterpret_cast<const float2*>(xy_g) + (long long)b * N1;
+    const float2* src = reinterpret_cast<const float2*>(xy_g) + (long long)ls_instance(inst, Bxy, r) * N1;
     int16_t* row = tours + (long long)r * L;
     for (int p = tid; p < N1; p += nthr) xy[p] = src[p];
     for (int p = tid; p < N1; p += nthr) tour[p] = row[p];
@@ -60,8 +59,7 @@ __global__ void __launch_bounds__(512, 2) tsp_ls_kernel(const float* __restrict_
       int bk = 0x7fffffff;
       for (int task = tid; task < tasks; task += nthr) {
         const int i = task % N1, c = task / N1;
-        const int j0 = max(c * TSP_LS_CHUNK, max_segment ? 0 : i + 2), j1 = min(c * TSP_LS_CHUNK + TSP_LS_CHUNK, N1);
-        if (j0 >= j1) continue;
+        const int j0 = c * TSP_LS_CHUNK, j1 = min(j0 + TSP_LS_CHUNK, N1);
         const float2 p0 = xy[tour[i]], p1 = xy[tour[min(i + 1, N1 - 1)]], p2 = xy[tour[min(i + 2, N1 - 1)]];
         const float e_i = edge[i];
         // removal part of the Or-opt variants: segment i..i+s-1 taken out, t_i-1 joined to t_i+s
@@ -124,15 +122,7 @@ __global__ void __launch_bounds__(512, 2) tsp_ls_kernel(const float* __restrict_
       __syncthreads();
     }
 
-    for (int p = tid; p < N1; p += nthr) row[p] = tour[p];
-    if (tid == 0) {
-      // the summation order of tour_length_kernel: sequential from the edge leaving position 0
-      float sum = 0.f;
-      for (int p = 0; p < N1; ++p) sum += edge[p];
-      length[r] = sum;
-      iterations[r] = moves;
-    }
-    __syncthreads();                                    // shared memory is reused by the next tour
+    ls_store_row(tour, edge, N1, row, r, moves, length, iterations, nthr);
   }
 }
 
@@ -147,28 +137,13 @@ extern "C" {
 int elg_tsp_local_search(const float* xy, int Bxy, int N1, const int32_t* inst, int16_t* tours, int R, int L,
                          int max_segment, int round_edges, int max_iterations, int32_t* iterations, float* length,
                          void* stream) {
-  ELG_REQUIRE(N1 > 0 && R >= 0 && Bxy > 0, ELG_EINVAL, "bad sizes N1=%d R=%d Bxy=%d", N1, R, Bxy);
-  ELG_REQUIRE(N1 <= ELG_MAX_NODES, ELG_EUNSUPPORTED, "tsp local search supports up to %d nodes (got %d)", ELG_MAX_NODES,
-              N1);
+  if (int e = ls_check_args("tsp local search", xy, Bxy, N1, inst, tours, R, max_iterations, iterations, length)) return e;
   ELG_REQUIRE(L >= N1, ELG_EINVAL, "tours need L >= N1 (L=%d, N1=%d)", L, N1);
   ELG_REQUIRE(max_segment >= 0 && max_segment <= 3, ELG_EINVAL, "max_segment must be in 0..3 (got %d)", max_segment);
-  ELG_REQUIRE(max_iterations >= 0, ELG_EINVAL, "max_iterations must be >= 0 (got %d)", max_iterations);
-  ELG_REQUIRE(xy && tours && iterations && length, ELG_EINVAL, "NULL pointer");
-  ELG_REQUIRE(inst || Bxy == 1 || Bxy == R, ELG_EINVAL, "without inst the xy batch must be 1 or R (Bxy=%d, R=%d)", Bxy, R);
-  if (R == 0) return ELG_OK;
-  const size_t smem = tsp_ls_smem_bytes(N1);
-  const int threads = N1 <= 512 ? 256 : 512;
-  ELG_CUDA_OK(cudaFuncSetAttribute(tsp_ls_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int dev = 0, sms = 0, per_sm = 0;
-  ELG_CUDA_OK(cudaGetDevice(&dev));
-  ELG_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  ELG_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, tsp_ls_kernel, threads, smem));
-  ELG_REQUIRE(per_sm > 0, ELG_EUNSUPPORTED, "tsp local search: %zu bytes of shared memory do not fit (N1=%d)", smem, N1);
-  const int grid = (int)((long long)R < (long long)sms * per_sm ? R : sms * per_sm);
-  tsp_ls_kernel<<<grid, threads, smem, (cudaStream_t)stream>>>(xy, Bxy, N1, inst, tours, R, L, max_segment, round_edges,
-                                                               max_iterations, iterations, length);
-  ELG_LAUNCH_OK();
-  return ELG_OK;
+  if (max_segment == 0)                                 // plain 2-opt: the 2-opt kernel sweeps it with fewer distances
+    return elg_two_opt(ELG_TSP, xy, Bxy, N1, inst, tours, R, L, round_edges, max_iterations, iterations, length, stream);
+  return ls_launch(tsp_ls_kernel, tsp_ls_smem_bytes(N1), N1, R, stream, "tsp local search", N1, L, xy, Bxy, N1, inst,
+                   tours, R, L, max_segment, round_edges, max_iterations, iterations, length);
 }
 
 }  // extern "C"

@@ -33,8 +33,7 @@ __global__ void __launch_bounds__(512) two_opt_kernel(const float* __restrict__ 
   const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, warp = tid >> 5;
 
   for (int r = blockIdx.x; r < R; r += gridDim.x) {
-    const int b = inst ? inst[r] : (Bxy == 1 ? 0 : r);
-    const float2* src = reinterpret_cast<const float2*>(xy_g) + (long long)b * N1;
+    const float2* src = reinterpret_cast<const float2*>(xy_g) + (long long)ls_instance(inst, Bxy, r) * N1;
     int16_t* row = tours + (long long)r * L;
     for (int p = tid; p < N1; p += nthr) xy[p] = src[p];
     for (int p = tid; p < n; p += nthr) tour[p] = row[p];
@@ -112,15 +111,7 @@ __global__ void __launch_bounds__(512) two_opt_kernel(const float* __restrict__ 
       __syncthreads();
     }
 
-    for (int p = tid; p < n; p += nthr) row[p] = tour[p];
-    if (tid == 0) {
-      // the summation order of tour_length_kernel: sequential from the edge leaving position 0
-      float sum = 0.f;
-      for (int p = 0; p < n; ++p) sum += edge[p];
-      length[r] = sum;
-      iterations[r] = moves;
-    }
-    __syncthreads();                                    // shared memory is reused by the next tour
+    ls_store_row(tour, edge, n, row, r, moves, length, iterations, nthr);
   }
 }
 
@@ -138,30 +129,13 @@ extern "C" {
 int elg_two_opt(int problem, const float* xy, int Bxy, int N1, const int32_t* inst, int16_t* tours, int R, int L,
                 int round_edges, int max_iterations, int32_t* iterations, float* length, void* stream) {
   ELG_REQUIRE(problem == ELG_TSP || problem == ELG_CVRP, ELG_EINVAL, "unknown problem %d", problem);
-  ELG_REQUIRE(N1 > 0 && R >= 0 && Bxy > 0, ELG_EINVAL, "bad sizes N1=%d R=%d Bxy=%d", N1, R, Bxy);
-  ELG_REQUIRE(N1 <= ELG_MAX_NODES, ELG_EUNSUPPORTED, "2-opt supports up to %d nodes (got %d)", ELG_MAX_NODES, N1);
+  if (int e = ls_check_args("2-opt", xy, Bxy, N1, inst, tours, R, max_iterations, iterations, length)) return e;
   ELG_REQUIRE(problem == ELG_CVRP || L >= N1, ELG_EINVAL, "tsp tours need L >= N1 (L=%d, N1=%d)", L, N1);
   ELG_REQUIRE(problem == ELG_TSP || (L > 0 && L <= 2 * N1 + 2), ELG_EINVAL,
               "cvrp tours need 0 < L <= 2*N1+2 (L=%d, N1=%d)", L, N1);
-  ELG_REQUIRE(max_iterations >= 0, ELG_EINVAL, "max_iterations must be >= 0 (got %d)", max_iterations);
-  ELG_REQUIRE(xy && tours && iterations && length, ELG_EINVAL, "NULL pointer");
-  ELG_REQUIRE(inst || Bxy == 1 || Bxy == R, ELG_EINVAL, "without inst the xy batch must be 1 or R (Bxy=%d, R=%d)", Bxy, R);
-  if (R == 0) return ELG_OK;
-  const size_t smem = two_opt_smem_bytes(problem, N1, L);
-  const int n = problem == ELG_CVRP ? L : N1;
-  const int threads = n <= 512 ? 256 : 512;
-  auto kernel = problem == ELG_CVRP ? two_opt_kernel<ELG_CVRP> : two_opt_kernel<ELG_TSP>;
-  ELG_CUDA_OK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int dev = 0, sms = 0, per_sm = 0;
-  ELG_CUDA_OK(cudaGetDevice(&dev));
-  ELG_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  ELG_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
-  ELG_REQUIRE(per_sm > 0, ELG_EUNSUPPORTED, "2-opt: %zu bytes of shared memory do not fit (N1=%d, L=%d)", smem, N1, L);
-  const int grid = (int)((long long)R < (long long)sms * per_sm ? R : sms * per_sm);
-  kernel<<<grid, threads, smem, (cudaStream_t)stream>>>(xy, Bxy, N1, inst, tours, R, L, round_edges, max_iterations,
-                                                        iterations, length);
-  ELG_LAUNCH_OK();
-  return ELG_OK;
+  return ls_launch(problem == ELG_CVRP ? two_opt_kernel<ELG_CVRP> : two_opt_kernel<ELG_TSP>,
+                   two_opt_smem_bytes(problem, N1, L), problem == ELG_CVRP ? L : N1, R, stream, "2-opt", N1, L, xy, Bxy,
+                   N1, inst, tours, R, L, round_edges, max_iterations, iterations, length);
 }
 
 }  // extern "C"

@@ -39,26 +39,21 @@ def test(dataloader, model, env, aug_factor, two_opt_iterations=0, local_search_
         raise ValueError("the local search stage needs the capacity the demands are normalised by")
     model.eval()
     model.requires_grad_(False)
+    stages = drv.enabled_stages({'two_opt_iterations': two_opt_iterations,
+                                 'local_search_iterations': local_search_iterations})
+    totals = [[0., 0., 0] for _ in stages]              # cost, seconds, moves per enabled stage
     avg_cost_total, no_avg_cost_total, t = 0., 0., 0
-    two_opt_cost, two_opt_seconds, two_opt_moves = 0., 0., 0
-    ls_cost, ls_seconds, ls_moves = 0., 0., 0
     start = time.time()
     for batch in dataloader:
         no_aug_cost, aug_cost, solutions, rewards = solve_batch(model, env, batch, aug_factor)
         avg_cost_total += aug_cost.mean()
         no_avg_cost_total += no_aug_cost.mean()
-        if two_opt_iterations:
-            cost, seconds, moves = drv.two_opt_refine("cvrp", env.depot_node_xy, solutions, rewards, aug_factor, two_opt_iterations,
-                                                      rounding=False)
-            two_opt_cost += cost.mean()
-            two_opt_seconds += seconds
-            two_opt_moves += int(moves.sum())
-        if local_search_iterations:
-            cost, seconds, moves = drv.local_search_refine(env.depot_node_xy, env.depot_node_demand, capacity, solutions,
-                                                           rewards, aug_factor, local_search_iterations, rounding=False)
-            ls_cost += cost.mean()
-            ls_seconds += seconds
-            ls_moves += int(moves.sum())
+        for (stage, iterations), total in zip(stages, totals):
+            cost, seconds, moves = drv.refine(stage, "cvrp", env.depot_node_xy, solutions, rewards, aug_factor, iterations,
+                                              False, env.depot_node_demand, capacity)
+            total[0] += cost.mean()
+            total[1] += seconds
+            total[2] += int(moves.sum())
         t += 1
     torch.cuda.synchronize()
     end = time.time()
@@ -66,10 +61,8 @@ def test(dataloader, model, env, aug_factor, two_opt_iterations=0, local_search_
     no_avg_cost_total /= t
     print("Aug cost: {:.4f}".format(avg_cost_total))
     print("no aug Avg cost: {:.4f}, Wall-clock time: {:.2f}s".format(no_avg_cost_total, float(end - start)))
-    if two_opt_iterations:
-        print("2-opt Aug cost: {:.4f}, 2-opt time: {:.2f}s, moves: {}".format(two_opt_cost / t, two_opt_seconds, two_opt_moves))
-    if local_search_iterations:
-        print("local search Aug cost: {:.4f}, local search time: {:.2f}s, moves: {}".format(ls_cost / t, ls_seconds, ls_moves))
+    for (stage, _), (cost, seconds, moves) in zip(stages, totals):
+        print("{0} Aug cost: {1:.4f}, {0} time: {2:.2f}s, moves: {3}".format(stage.label, cost / t, seconds, moves))
     return avg_cost_total
 
 
@@ -89,7 +82,7 @@ if __name__ == "__main__":
     import yaml
     with open('config.yml', 'r', encoding='utf-8') as f:
         config = yaml.load(f.read(), Loader=yaml.FullLoader)
-    drv.reject_tsp_local_search(config)
+    drv.reject('cvrp', config)
     device = "cuda:{}".format(config['cuda_device_num'])
     model = load_model(config, device)
     env = CVRPEnv(multi_width=config['params']['multiple_width'], device=device)

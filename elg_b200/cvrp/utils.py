@@ -73,36 +73,24 @@ def batched_two_opt_torch(points, tour, max_iterations=1000, device=None):
     and runs while any tour improves), and a move only reverses customers of one route, depot edges included, so every
     route keeps its customers and its load.  The TSP function applied to these tours would reverse segments across depot
     visits and could break capacity."""
-    return _two_opt_dropin("cvrp", points, tour, max_iterations, device)
+    return _dropin("batched_two_opt_torch", points, tour, device,
+                   lambda xy, t: engine.two_opt("cvrp", xy, t, max_iterations=max_iterations))
 
 
-def _two_opt_dropin(problem, points, tour, max_iterations, device, max_segment=None):
-    """Shared body of the cvrp / tsp batched_two_opt_torch and, with max_segment set, of tsp.tsp_local_search (2-opt
-    and Or-opt): conversion in and out of numpy / torch, closed tsp tours."""
-    name = "batched_two_opt_torch" if max_segment is None else "tsp_local_search"
+def _dropin(name, points, tour, device, search):
+    """Shared body of the drop-in searches of both sub-projects (name: the calling function): the CUDA device
+    (device=None: the current one), numpy / torch in and out.  search(xy (1, N, 2) fp32, tours int64), both on that
+    device, -> (tours, length, iterations) of the engine; returns (tours in the input's type and dtype, the largest move
+    count)."""
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     if dev.type != "cuda":
         raise _lib.ElgError("%s needs a CUDA device (got %s): elg_b200 has no CPU path" % (name, dev))
-    as_numpy = isinstance(tour, np.ndarray)
     t = torch.as_tensor(tour)
-    out_dtype, out_dev = t.dtype, t.device
-    t = t.to(dev, torch.int64)
-    xy = torch.as_tensor(points).to(dev, torch.float32)[None]
-    if problem == "tsp":
-        if t.dim() != 2 or t.shape[1] < 2 or not bool((t[:, -1] == t[:, 0]).all()):
-            raise ValueError("tsp tours must be (batch, N+1) closed tours (last node = first node)")
-        if max_segment is None:
-            refined, _, iters = engine.two_opt("tsp", xy, t[:, :-1].contiguous(), max_iterations=max_iterations)
-        else:
-            refined, _, iters = engine.tsp_local_search(xy, t[:, :-1].contiguous(), max_iterations=max_iterations,
-                                                        max_segment=max_segment)
-        refined = torch.cat((refined, refined[:, :1]), dim=1)
-    else:
-        refined, _, iters = engine.two_opt("cvrp", xy, t, max_iterations=max_iterations)
+    refined, _, iters = search(torch.as_tensor(points).to(dev, torch.float32)[None], t.to(dev, torch.int64))
     n_iter = int(iters.max()) if iters.numel() else 0
-    if as_numpy:
+    if isinstance(tour, np.ndarray):
         return refined.cpu().numpy().astype(tour.dtype), n_iter
-    return refined.to(out_dev, out_dtype), n_iter
+    return refined.to(t.device, t.dtype), n_iter
 
 
 def cvrp_local_search(points, demand, capacity, tour, max_iterations=1000, device=None):
@@ -114,19 +102,8 @@ def cvrp_local_search(points, demand, capacity, tour, max_iterations=1000, devic
     route within capacity); numpy or torch, and the tour comes back in the same type and dtype, in canonical form (routes
     in order, each preceded by one 0, zero padding to T).  Returns (tour, iterations), iterations being the largest number
     of moves any tour took.  device=None is the current CUDA device; there is no CPU path."""
-    dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
-    if dev.type != "cuda":
-        raise _lib.ElgError("cvrp_local_search needs a CUDA device (got %s): elg_b200 has no CPU path" % dev)
-    as_numpy = isinstance(tour, np.ndarray)
-    t = torch.as_tensor(tour)
-    out_dtype, out_dev = t.dtype, t.device
-    xy = torch.as_tensor(points).to(dev, torch.float32)[None]
-    dem = torch.as_tensor(demand).to(dev, torch.float32)[None]
-    refined, _, iters = engine.cvrp_local_search(xy, t.to(dev, torch.int64), dem, capacity, max_iterations=max_iterations)
-    n_iter = int(iters.max()) if iters.numel() else 0
-    if as_numpy:
-        return refined.cpu().numpy().astype(tour.dtype), n_iter
-    return refined.to(out_dev, out_dtype), n_iter
+    return _dropin("cvrp_local_search", points, tour, device, lambda xy, t: engine.cvrp_local_search(
+        xy, t, torch.as_tensor(demand).to(xy.device, torch.float32)[None], capacity, max_iterations=max_iterations))
 
 
 def augment_xy_data_by_8_fold(problems):

@@ -310,6 +310,55 @@ def tour_length(xy, tours, rounding=False):
     return out
 
 
+class _LocalSearch:
+    """Checks and set-up shared by two_opt, tsp_local_search and cvrp_local_search.  The constructor checks the shapes,
+    max_iterations, inst (R indices into the Bxy instances; without it xy must hold 1 or R instances) and the node ids of
+    the tours: in every position (whole_row, CVRP rows) or in positions 0..N1-1 (TSP tours).  The caller adds its own
+    checks and then calls run()."""
+
+    def __init__(self, xy, tours, inst, max_iterations, whole_row):
+        if tours.dim() != 2 or xy.dim() != 3 or xy.shape[2] != 2:
+            raise ValueError("tours must be (R, L) and xy (Bxy, N1, 2)")
+        if max_iterations < 0:
+            raise ValueError("max_iterations must be >= 0")
+        self.R, self.L = tours.shape
+        self.Bxy, self.N1 = int(xy.shape[0]), int(xy.shape[1])
+        if inst is not None:
+            inst = torch.as_tensor(inst, device=tours.device).to(torch.int32).contiguous()
+            if inst.shape != (self.R,) or (self.R and (int(inst.min()) < 0 or int(inst.max()) >= self.Bxy)):
+                raise ValueError("inst must be (R,) indices into the %d xy instances" % self.Bxy)
+        elif self.Bxy not in (1, self.R):
+            raise ValueError("without inst, xy must hold 1 or R instances (got %d for %d rows)" % (self.Bxy, self.R))
+        ids = tours if whole_row else tours[:, :self.N1]
+        if ids.numel():
+            lo, hi = torch.aminmax(ids)
+            if int(lo) < 0 or int(hi) >= self.N1:
+                raise ValueError("tour node ids must lie in [0, %d)" % self.N1)
+        self.xy, self.tours, self.inst = xy, tours, inst
+
+    def per_row(self, x):
+        """(Bxy, ...) per-instance tensor -> (R, ...), row r taking its instance's entry"""
+        return x[self.inst.long()] if self.inst is not None else x.expand(self.R, *x.shape[1:])
+
+    def run(self, launch, demand=None):
+        """Checks that the tensors are on a CUDA device, then calls launch(xy, inst, tours, iterations, length, stream)
+        with the pointers of fp32 xy, int32 inst (NULL without it), an int16 working copy of the tours and the output
+        buffers, under the tours' device; its return code goes through check().  -> (tours int64 (R, L), length (R,),
+        iterations (R,))"""
+        _require_cuda(self.xy, "xy")
+        _require_cuda(self.tours, "tours")
+        if demand is not None:
+            _require_cuda(demand, "demand")
+        dev = self.tours.device
+        t16 = self.tours.to(torch.int16, copy=True).contiguous()
+        length = torch.empty(self.R, dtype=torch.float32, device=dev)
+        iters = torch.empty(self.R, dtype=torch.int32, device=dev)
+        xy = self.xy.contiguous().float()
+        with torch.cuda.device(dev):
+            check(launch(_ptr(xy), _ptr(self.inst), _ptr(t16), _ptr(iters), _ptr(length), _stream(dev)))
+        return t16.long(), length, iters
+
+
 def two_opt(problem, xy, tours, inst=None, max_iterations=1000, rounding=False):
     """Best-improvement 2-opt local search (elg_two_opt; semantics in include/elg_b200.h), one launch for all tours.
 
@@ -317,32 +366,10 @@ def two_opt(problem, xy, tours, inst=None, max_iterations=1000, rounding=False):
     0..N1-1 that keeps its start node, cvrp a depot-delimited row whose moves stay inside one route; inst (R,) picks the xy
     instance of every tour (default: tour r uses xy[r], or xy[0] when Bxy == 1); rounding rint()s every edge (library
     metric).  Returns (tours int64 (R, L), length (R,) as tour_length measures it, iterations (R,) moves applied)."""
-    _require_cuda(xy, "xy")
-    _require_cuda(tours, "tours")
-    if tours.dim() != 2 or xy.dim() != 3 or xy.shape[2] != 2:
-        raise ValueError("tours must be (R, L) and xy (Bxy, N1, 2)")
-    if max_iterations < 0:
-        raise ValueError("max_iterations must be >= 0")
-    dev = tours.device
-    R, L = tours.shape
-    Bxy, N1 = int(xy.shape[0]), int(xy.shape[1])
-    n = L if problem == "cvrp" else min(N1, L)
-    if R and n:
-        lo, hi = torch.aminmax(tours[:, :n])
-        if int(lo) < 0 or int(hi) >= N1:
-            raise ValueError("tour node ids must lie in [0, %d)" % N1)
-    if inst is not None:
-        inst = torch.as_tensor(inst, device=dev).to(torch.int32).contiguous()
-        if inst.shape != (R,) or (R and (int(inst.min()) < 0 or int(inst.max()) >= Bxy)):
-            raise ValueError("inst must be (R,) indices into the %d xy instances" % Bxy)
-    t16 = tours.to(torch.int16, copy=True).contiguous()
-    length = torch.empty(R, dtype=torch.float32, device=dev)
-    iters = torch.empty(R, dtype=torch.int32, device=dev)
-    xy = xy.contiguous().float()
-    with torch.cuda.device(dev):
-        check(lib.elg_two_opt(ELG_CVRP if problem == "cvrp" else ELG_TSP, _ptr(xy), Bxy, N1, _ptr(inst), _ptr(t16), R, L,
-                              1 if rounding else 0, int(max_iterations), _ptr(iters), _ptr(length), _stream(dev)))
-    return t16.long(), length, iters
+    s = _LocalSearch(xy, tours, inst, max_iterations, whole_row=problem == "cvrp")
+    return s.run(lambda xy_p, inst_p, t_p, it_p, len_p, stream: lib.elg_two_opt(
+        ELG_CVRP if problem == "cvrp" else ELG_TSP, xy_p, s.Bxy, s.N1, inst_p, t_p, s.R, s.L, 1 if rounding else 0,
+        int(max_iterations), it_p, len_p, stream))
 
 
 def tsp_local_search(xy, tours, inst=None, max_iterations=1000, max_segment=3, rounding=False):
@@ -354,39 +381,17 @@ def tsp_local_search(xy, tours, inst=None, max_iterations=1000, max_segment=3, r
     Bxy == 1); max_segment (0..3) the longest Or-opt segment, 0 being plain 2-opt; rounding rint()s every edge (library
     metric).  Position 0 never moves.  Returns (tours int64 (R, L), length (R,) as tour_length measures it,
     iterations (R,) moves applied)."""
-    if tours.dim() != 2 or xy.dim() != 3 or xy.shape[2] != 2:
-        raise ValueError("tours must be (R, L) and xy (Bxy, N1, 2)")
-    R, L = tours.shape
-    Bxy, N1 = int(xy.shape[0]), int(xy.shape[1])
-    if L < N1:
-        raise ValueError("tours need at least N1 = %d positions (got %d)" % (N1, L))
-    if max_iterations < 0:
-        raise ValueError("max_iterations must be >= 0")
     if max_segment not in (0, 1, 2, 3):
         raise ValueError("max_segment must be 0, 1, 2 or 3 (got %r)" % (max_segment,))
-    dev = tours.device
-    if inst is not None:
-        inst = torch.as_tensor(inst, device=dev).to(torch.int32).contiguous()
-        if inst.shape != (R,) or (R and (int(inst.min()) < 0 or int(inst.max()) >= Bxy)):
-            raise ValueError("inst must be (R,) indices into the %d xy instances" % Bxy)
-    elif Bxy not in (1, R):
-        raise ValueError("without inst, xy must hold 1 or R instances (got %d for %d rows)" % (Bxy, R))
-    if R and N1:
-        t = tours[:, :N1].long()
-        if int(t.min()) < 0 or int(t.max()) >= N1:
-            raise ValueError("tour node ids must lie in [0, %d)" % N1)
-        if not torch.equal(t.sort(1)[0], torch.arange(N1, device=dev).expand(R, -1)):
-            raise ValueError("positions 0..%d of every tour must hold a permutation of the nodes" % (N1 - 1))
-    _require_cuda(xy, "xy")
-    _require_cuda(tours, "tours")
-    t16 = tours.to(torch.int16, copy=True).contiguous()
-    length = torch.empty(R, dtype=torch.float32, device=dev)
-    iters = torch.empty(R, dtype=torch.int32, device=dev)
-    xy = xy.contiguous().float()
-    with torch.cuda.device(dev):
-        check(lib.elg_tsp_local_search(_ptr(xy), Bxy, N1, _ptr(inst), _ptr(t16), R, L, int(max_segment),
-                                       1 if rounding else 0, int(max_iterations), _ptr(iters), _ptr(length), _stream(dev)))
-    return t16.long(), length, iters
+    s = _LocalSearch(xy, tours, inst, max_iterations, whole_row=False)
+    R, L, N1 = s.R, s.L, s.N1
+    if L < N1:
+        raise ValueError("tours need at least N1 = %d positions (got %d)" % (N1, L))
+    if R and N1 and not torch.equal(tours[:, :N1].long().sort(1)[0], torch.arange(N1, device=tours.device).expand(R, -1)):
+        raise ValueError("positions 0..%d of every tour must hold a permutation of the nodes" % (N1 - 1))
+    return s.run(lambda xy_p, inst_p, t_p, it_p, len_p, stream: lib.elg_tsp_local_search(
+        xy_p, s.Bxy, N1, inst_p, t_p, R, L, int(max_segment), 1 if rounding else 0, int(max_iterations), it_p, len_p,
+        stream))
 
 
 def cvrp_local_search(xy, tours, demand, capacity, inst=None, max_iterations=1000, rounding=False):
@@ -399,51 +404,33 @@ def cvrp_local_search(xy, tours, demand, capacity, inst=None, max_iterations=100
     inst (R,) picks the xy / demand instance of every row (default: row r uses instance r, or 0 when Bxy == 1); rounding
     rint()s every edge (library metric).  Returns (canonical tours int64 (R, L), length (R,) as tour_length measures it,
     iterations (R,) moves applied)."""
-    if tours.dim() != 2 or xy.dim() != 3 or xy.shape[2] != 2 or demand.shape != xy.shape[:2]:
-        raise ValueError("tours must be (R, L), xy (Bxy, N1, 2) and demand (Bxy, N1)")
-    if max_iterations < 0:
-        raise ValueError("max_iterations must be >= 0")
+    s = _LocalSearch(xy, tours, inst, max_iterations, whole_row=True)
+    R, L, N1 = s.R, s.L, s.N1
+    if demand.shape != xy.shape[:2]:
+        raise ValueError("demand must be (Bxy, N1)")
     if int(capacity) != capacity or capacity <= 0:
         raise ValueError("capacity must be a positive integer (got %r)" % (capacity,))
     capacity = int(capacity)
-    dev = tours.device
-    R, L = tours.shape
-    Bxy, N1 = int(xy.shape[0]), int(xy.shape[1])
     scaled = demand.double() * capacity
     units = torch.round(scaled)
     if bool(((scaled - units).abs() > 1e-3).any()):
         raise ValueError("demand * capacity must be integral (within 1e-3): demands are whole units of the capacity")
     units = units.to(torch.int32).contiguous()
-    if inst is not None:
-        inst = torch.as_tensor(inst, device=dev).to(torch.int32).contiguous()
-        if inst.shape != (R,) or (R and (int(inst.min()) < 0 or int(inst.max()) >= Bxy)):
-            raise ValueError("inst must be (R,) indices into the %d xy instances" % Bxy)
-    elif Bxy not in (1, R):
-        raise ValueError("without inst, xy must hold 1 or R instances (got %d for %d rows)" % (Bxy, R))
     if R:
         t = tours.long()
-        if int(t.min()) < 0 or int(t.max()) >= N1 or bool((t[:, 0] != 0).any()):
-            raise ValueError("rows must hold node ids in [0, %d) with the depot at position 0" % N1)
-        counts = torch.zeros(R, N1, dtype=torch.int32, device=dev).scatter_add_(1, t, torch.ones_like(t, dtype=torch.int32))
+        if bool((t[:, 0] != 0).any()):
+            raise ValueError("rows must hold the depot at position 0")
+        counts = torch.zeros(R, N1, dtype=torch.int32, device=t.device).scatter_add_(1, t, torch.ones_like(t, dtype=torch.int32))
         if not bool((counts[:, 1:] == 1).all()):
             raise ValueError("every row must visit each customer 1..%d exactly once" % (N1 - 1))
-        which = inst.long() if inst is not None else (torch.arange(R, device=dev) if Bxy > 1 else torch.zeros(R, dtype=torch.long, device=dev))
-        d = units[which].gather(1, t)
         route = (t == 0).long().cumsum(1)
-        loads = torch.zeros(R, L + 1, dtype=torch.int64, device=dev).scatter_add_(1, route, d.long())
+        loads = torch.zeros(R, L + 1, dtype=torch.int64, device=t.device).scatter_add_(1, route,
+                                                                                         s.per_row(units).gather(1, t).long())
         if int(loads.max()) > capacity:
             raise ValueError("an input route exceeds the capacity %d" % capacity)
-    _require_cuda(xy, "xy")
-    _require_cuda(tours, "tours")
-    _require_cuda(units, "demand")
-    t16 = tours.to(torch.int16, copy=True).contiguous()
-    length = torch.empty(R, dtype=torch.float32, device=dev)
-    iters = torch.empty(R, dtype=torch.int32, device=dev)
-    xy = xy.contiguous().float()
-    with torch.cuda.device(dev):
-        check(lib.elg_cvrp_local_search(_ptr(xy), Bxy, N1, _ptr(units), capacity, _ptr(inst), _ptr(t16), R, L,
-                                        1 if rounding else 0, int(max_iterations), _ptr(iters), _ptr(length), _stream(dev)))
-    return t16.long(), length, iters
+    return s.run(lambda xy_p, inst_p, t_p, it_p, len_p, stream: lib.elg_cvrp_local_search(
+        xy_p, s.Bxy, N1, _ptr(units), capacity, inst_p, t_p, R, L, 1 if rounding else 0, int(max_iterations), it_p,
+        len_p, stream), demand=units)
 
 
 # ---------------------------------------------------------------------------------------------- training path

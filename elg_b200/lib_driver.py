@@ -6,27 +6,19 @@ TSP/test_tsplib.py:18-168) but are thin shells around the functions here:
     run_set(entries, solve, ...)         the per-instance loop with timing and the record dicts of the result files
     gap_bins(results, edges, ...)        mean gap per size bin, as the reference prints them
 
-Optional 2-opt stage (config params.two_opt_iterations; absent or 0: nothing changes).  load_model records the setting on
-the model; solve_instance then refines the best POMO row of every aug-instance in the library metric (rounded unscaled
-coordinates) and returns the cost as an InstanceCost carrying the refined result; fill_record adds best_cost_2opt /
-gap_2opt / two_opt_seconds / two_opt_iterations to the record; run_set prints one extra line per instance and gap_bins
-one per size bin.  two_opt_refine is shared with the test.py drivers.
-
-Optional CVRP local search stage (config params.local_search_iterations; absent or 0: nothing changes), independent of
-the 2-opt stage and run on the same rows: solve_instance refines them with engine.cvrp_local_search in the library metric
-(with the capacity CVRPEnv.load_vrplib_problem recorded), InstanceCost.local_search carries the result, fill_record adds
-best_cost_ls / gap_ls / ls_seconds / ls_iterations, and run_set / gap_bins print their lines after the 2-opt ones.
-load_model rejects the key for a TSP model.
-
-Optional TSP local search stage (config params.tsp_local_search_iterations; absent or 0: nothing changes): 2-opt and
-Or-opt moves (engine.tsp_local_search), independent of the 2-opt stage and run on the same rows in the library metric;
-InstanceCost.tsp_local_search carries the result, fill_record adds best_cost_tsp_ls / gap_tsp_ls / tsp_ls_seconds /
-tsp_ls_iterations, and run_set / gap_bins print their lines after the 2-opt ones.  load_model rejects the key for a CVRP
-model.
+Optional refinement stages (STAGES; a config key absent or 0: nothing changes): 2-opt (params.two_opt_iterations, both
+problems), the capacity-aware CVRP local search (params.local_search_iterations, with the capacity
+CVRPEnv.load_vrplib_problem recorded) and the TSP 2-opt + Or-opt local search (params.tsp_local_search_iterations).
+load_model records the settings on the model and rejects a key the problem does not accept; solve_instance then refines
+the best POMO row of every aug-instance with every enabled stage, independently and in the library metric (rounded
+unscaled coordinates), and returns the cost as an InstanceCost carrying each stage's result; fill_record adds the
+stage's best_cost_ / gap_ / _seconds / _iterations keys to the record, and run_set / gap_bins print one extra line per
+instance and per size bin, in the order of STAGES.  refine is shared with the test.py drivers.
 """
 import json
 import os
 import time
+from collections import namedtuple
 
 import numpy as np
 import torch
@@ -45,10 +37,7 @@ def require_cuda(config):
 def load_model(model_cls, config, device, model=None, needs_local=True):
     """The reference's checkpoint protocol: add_local_policy BEFORE load_state_dict (CVRP/test.py:75-78)."""
     from .cvrp.CVRPModel import CVRPModel
-    if not issubclass(model_cls, CVRPModel):
-        reject_local_search(config)
-    else:
-        reject_tsp_local_search(config)
+    reject('cvrp' if issubclass(model_cls, CVRPModel) else 'tsp', config)
     if model is None:
         model = model_cls(**config['model_params'])
         if needs_local:
@@ -57,24 +46,8 @@ def load_model(model_cls, config, device, model=None, needs_local=True):
     model = model.to(device)
     model.eval()
     model.requires_grad_(False)
-    model._elg_two_opt_iterations = config.get('params', {}).get('two_opt_iterations') or 0
-    model._elg_local_search_iterations = config.get('params', {}).get('local_search_iterations') or 0
-    model._elg_tsp_local_search_iterations = config.get('params', {}).get('tsp_local_search_iterations') or 0
+    model._elg_stage_iterations = {stage.key: config.get('params', {}).get(stage.key) or 0 for stage in STAGES}
     return model
-
-
-def reject_local_search(config):
-    """The TSP drivers: params.local_search_iterations is the CVRP local search, TSP tours have the 2-opt stage."""
-    if config.get('params', {}).get('local_search_iterations'):
-        raise ValueError("params.local_search_iterations is the capacity-aware CVRP local search; "
-                         "refine TSP tours with params.two_opt_iterations")
-
-
-def reject_tsp_local_search(config):
-    """The CVRP drivers: params.tsp_local_search_iterations is the TSP search, CVRP rows have their own local search."""
-    if config.get('params', {}).get('tsp_local_search_iterations'):
-        raise ValueError("params.tsp_local_search_iterations is the TSP 2-opt + Or-opt local search; "
-                         "refine CVRP rows with params.local_search_iterations")
 
 
 class InstanceCost(float):
@@ -85,45 +58,53 @@ class InstanceCost(float):
     tsp_local_search = None
 
 
-# optional refinement stages: (InstanceCost attribute, record key suffix, record key prefix, name in the printouts)
-_STAGES = (('two_opt', '2opt', 'two_opt', '2-opt'), ('local_search', 'ls', 'ls', 'local search'),
-           ('tsp_local_search', 'tsp_ls', 'tsp_ls', '2-opt + or-opt'))
+def _cvrp_local_search(problem, xy, rows, demand, capacity, iterations, rounding):
+    if capacity is None:
+        raise ValueError("the local search stage needs the instance's capacity (CVRPEnv.load_vrplib_problem)")
+    return engine.cvrp_local_search(xy, rows, demand, capacity, max_iterations=iterations, rounding=rounding)
 
 
-def _best_rows(solutions, rewards):
-    return solutions[torch.arange(rewards.shape[0], device=solutions.device), rewards.argmax(dim=1)]
+# An optional refinement stage: config key (under params), problems that accept it, InstanceCost attribute, record key
+# suffix and prefix, name in the printouts, rejection message for the other problem, and the engine call
+# run(problem, xy, rows, demand, capacity, iterations, rounding) -> (tours, length, moves).
+Stage = namedtuple('Stage', 'key problems attr suffix prefix label rejection run')
+STAGES = (
+    Stage('two_opt_iterations', ('tsp', 'cvrp'), 'two_opt', '2opt', 'two_opt', '2-opt', None,
+          lambda problem, xy, rows, demand, capacity, iterations, rounding:
+          engine.two_opt(problem, xy, rows, max_iterations=iterations, rounding=rounding)),
+    Stage('local_search_iterations', ('cvrp',), 'local_search', 'ls', 'ls', 'local search',
+          "params.local_search_iterations is the capacity-aware CVRP local search; "
+          "refine TSP tours with params.two_opt_iterations", _cvrp_local_search),
+    Stage('tsp_local_search_iterations', ('tsp',), 'tsp_local_search', 'tsp_ls', 'tsp_ls', '2-opt + or-opt',
+          "params.tsp_local_search_iterations is the TSP 2-opt + Or-opt local search; "
+          "refine CVRP rows with params.local_search_iterations",
+          lambda problem, xy, rows, demand, capacity, iterations, rounding:
+          engine.tsp_local_search(xy, rows, max_iterations=iterations, rounding=rounding)),
+)
 
 
-def two_opt_refine(problem, xy, solutions, rewards, aug_factor, iterations, rounding):
-    """2-opt (engine.two_opt, one launch) of the best POMO row of every aug-instance of a greedy rollout.
-    xy (aug*n or 1, N1, 2) is the metric the cost is measured in: library runs pass the unscaled coordinates with
-    rounding, random instances the scaled ones without.  -> (refined cost per instance, best over its augmentations (n,);
-    seconds; moves applied per instance, summed over its augmentations (n,))"""
-    rows = _best_rows(solutions, rewards)
-    return _timed_refine(lambda: engine.two_opt(problem, xy, rows, max_iterations=iterations, rounding=rounding), aug_factor)
+def reject(problem, config):
+    """Raises ValueError for a stage key in config['params'] that the problem ('tsp' / 'cvrp') does not accept."""
+    for stage in STAGES:
+        if problem not in stage.problems and config.get('params', {}).get(stage.key):
+            raise ValueError(stage.rejection)
 
 
-def local_search_refine(xy, demand, capacity, solutions, rewards, aug_factor, iterations, rounding):
-    """CVRP local search (engine.cvrp_local_search, one launch) of the best POMO row of every aug-instance of a greedy
-    rollout; demand (aug*n, N1) normalised as the environment holds it, capacity the integer capacity; otherwise as
-    two_opt_refine."""
-    rows = _best_rows(solutions, rewards)
-    return _timed_refine(lambda: engine.cvrp_local_search(xy, rows, demand, capacity, max_iterations=iterations,
-                                                          rounding=rounding), aug_factor)
+def enabled_stages(iterations):
+    """{config key: iterations} -> [(stage, iterations)] of the stages with iterations > 0, in the order of STAGES"""
+    return [(stage, iterations[stage.key]) for stage in STAGES if iterations.get(stage.key)]
 
 
-def tsp_local_search_refine(xy, solutions, rewards, aug_factor, iterations, rounding):
-    """TSP 2-opt + Or-opt local search (engine.tsp_local_search, one launch) of the best POMO row of every aug-instance
-    of a greedy rollout; as two_opt_refine."""
-    rows = _best_rows(solutions, rewards)
-    return _timed_refine(lambda: engine.tsp_local_search(xy, rows, max_iterations=iterations, rounding=rounding),
-                         aug_factor)
-
-
-def _timed_refine(run, aug_factor):
+def refine(stage, problem, xy, solutions, rewards, aug_factor, iterations, rounding, demand=None, capacity=None):
+    """One stage (one launch) on the best POMO row of every aug-instance of a greedy rollout.  xy (aug*n or 1, N1, 2) is
+    the metric the cost is measured in: library runs pass the unscaled coordinates with rounding, random instances the
+    scaled ones without; the CVRP local search also takes demand (aug*n, N1), normalised as the environment holds it, and
+    the integer capacity.  -> (refined cost per instance, best over its augmentations (n,); seconds; moves applied per
+    instance, summed over its augmentations (n,))"""
+    rows = solutions[torch.arange(rewards.shape[0], device=solutions.device), rewards.argmax(dim=1)]
     torch.cuda.synchronize()
     t0 = time.time()
-    _, length, iters = run()
+    _, length, iters = stage.run(problem, xy, rows, demand, capacity, iterations, rounding)
     torch.cuda.synchronize()
     seconds = time.time() - t0
     B = length.shape[0]
@@ -139,25 +120,15 @@ def solve_instance(model, env, rollout, aug_factor, width):
         solutions, _, rewards = rollout(model, env, 'greedy')
     best = -rewards.reshape(aug_factor, 1, width).max(dim=2)[0].max(dim=0)[0].float()
     cost = InstanceCost(best.cpu()[0])
-    iterations = getattr(model, '_elg_two_opt_iterations', 0)
-    if iterations:
-        cvrp = hasattr(env, 'unscaled_depot_node_xy')
-        refined, seconds, moves = two_opt_refine('cvrp' if cvrp else 'tsp',
-                                                 env.unscaled_depot_node_xy if cvrp else env._unscaled_dev,
-                                                 solutions, rewards, aug_factor, iterations, rounding=True)
-        cost.two_opt = (float(refined[0]), seconds, int(moves[0]))
-    iterations = getattr(model, '_elg_local_search_iterations', 0)
-    if iterations:
-        if env.capacity is None:
-            raise ValueError("the local search stage needs the instance's capacity (CVRPEnv.load_vrplib_problem)")
-        refined, seconds, moves = local_search_refine(env.unscaled_depot_node_xy, env.depot_node_demand, env.capacity,
-                                                      solutions, rewards, aug_factor, iterations, rounding=True)
-        cost.local_search = (float(refined[0]), seconds, int(moves[0]))
-    iterations = getattr(model, '_elg_tsp_local_search_iterations', 0)
-    if iterations:
-        refined, seconds, moves = tsp_local_search_refine(env._unscaled_dev, solutions, rewards, aug_factor, iterations,
-                                                          rounding=True)
-        cost.tsp_local_search = (float(refined[0]), seconds, int(moves[0]))
+    cvrp = hasattr(env, 'unscaled_depot_node_xy')
+    for stage, iterations in enabled_stages(getattr(model, '_elg_stage_iterations', {})):
+        if cvrp:
+            refined, seconds, moves = refine(stage, 'cvrp', env.unscaled_depot_node_xy, solutions, rewards, aug_factor,
+                                             iterations, True, env.depot_node_demand, env.capacity)
+        else:
+            refined, seconds, moves = refine(stage, 'tsp', env._unscaled_dev, solutions, rewards, aug_factor, iterations,
+                                             True)
+        setattr(cost, stage.attr, (float(refined[0]), seconds, int(moves[0])))
     return cost, solutions, rewards
 
 
@@ -176,9 +147,9 @@ def run_set(entries, solve_one, repeat_times=1, echo_cost=False):
             print("Instance Name {}: gap {:.4f}".format(name, record['gap']))
             if echo_cost:
                 print("cost: {}".format(record['best_cost']))
-            for _, suffix, _, label in _STAGES:
-                if 'gap_' + suffix in record:
-                    print("Instance Name {}: gap after {} {:.4f}".format(name, label, record['gap_' + suffix]))
+            for stage in STAGES:
+                if 'gap_' + stage.suffix in record:
+                    print("Instance Name {}: gap after {} {:.4f}".format(name, stage.label, record['gap_' + stage.suffix]))
     return results, total
 
 
@@ -187,13 +158,13 @@ def fill_record(record, best_cost, scale, optimal):
         record['best_cost'] = float(best_cost)
         record['scale'] = scale
         record['gap'] = (best_cost - optimal) / optimal
-        for attr, suffix, prefix, _ in _STAGES:
-            if getattr(best_cost, attr, None):
-                cost, seconds, moves = getattr(best_cost, attr)
-                record['best_cost_' + suffix] = cost
-                record['gap_' + suffix] = (cost - optimal) / optimal
-                record[prefix + '_seconds'] = seconds
-                record[prefix + '_iterations'] = moves    # moves applied, summed over the augmentations
+        for stage in STAGES:
+            if getattr(best_cost, stage.attr, None):
+                cost, seconds, moves = getattr(best_cost, stage.attr)
+                record['best_cost_' + stage.suffix] = cost
+                record['gap_' + stage.suffix] = (cost - optimal) / optimal
+                record[stage.prefix + '_seconds'] = seconds
+                record[stage.prefix + '_iterations'] = moves    # moves applied, summed over the augmentations
 
 
 def gap_bins(results, edges):
@@ -201,14 +172,14 @@ def gap_bins(results, edges):
     When the records carry an optional stage, also prints one line per bin and a total line for it, and adds
     'gap_2opt' / 'gap_ls' / 'gap_tsp_ls': {label: mean gap in %}."""
     out = _bin_means(results, edges, 'gap')
-    for _, suffix, _, name in _STAGES:
-        key = 'gap_' + suffix
+    for stage in STAGES:
+        key = 'gap_' + stage.suffix
         if results and all(key in r['record'][-1] for r in results):
             out[key] = _bin_means(results, edges, key)
             for label, mean in out[key].items():
                 if label != 'total':
-                    print("Average gap after {} on subset of {}: {:.2f}%".format(name, label, mean))
-            print("Average gap after {} total: {:.2f}%".format(name, out[key]['total']))
+                    print("Average gap after {} on subset of {}: {:.2f}%".format(stage.label, label, mean))
+            print("Average gap after {} total: {:.2f}%".format(stage.label, out[key]['total']))
     return out
 
 

@@ -6,7 +6,7 @@ import numpy as np
 import torch
 
 from .. import engine
-from ..cvrp.utils import _two_opt_dropin, augment_xy_data_by_8_fold, seed_everything  # noqa: F401  (same functions in both sub-projects)
+from ..cvrp.utils import _dropin, augment_xy_data_by_8_fold, seed_everything  # noqa: F401  (same functions in both sub-projects)
 
 
 def rollout(model, env, eval_type='greedy'):
@@ -53,7 +53,8 @@ def batched_two_opt_torch(points, tour, max_iterations=1000, device=None):
     The reference tree is not part of this project; the signature is that of the DIFUSCO utility the cited lines are
     understood to be.  One deliberate difference: every tour stops on its own, where the reference's loop couples the
     batch and runs while any tour improves."""
-    return _two_opt_dropin("tsp", points, tour, max_iterations, device)
+    return _dropin("batched_two_opt_torch", points, tour, device,
+                   _closed(lambda xy, t: engine.two_opt("tsp", xy, t, max_iterations=max_iterations)))
 
 
 def tsp_local_search(points, tour, max_iterations=1000, max_segment=3, device=None):
@@ -64,7 +65,18 @@ def tsp_local_search(points, tour, max_iterations=1000, max_segment=3, device=No
     points (N, 2); tour (batch, N+1) closed tours (last node = first node); numpy or torch, and the result comes back in
     the same type and dtype.  Returns (tour, iterations), iterations being the largest number of moves any tour took.
     Position 0 (the start node) never moves.  device=None is the current CUDA device; there is no CPU path."""
-    return _two_opt_dropin("tsp", points, tour, max_iterations, device, max_segment=max_segment)
+    return _dropin("tsp_local_search", points, tour, device, _closed(
+        lambda xy, t: engine.tsp_local_search(xy, t, max_iterations=max_iterations, max_segment=max_segment)))
+
+
+def _closed(search):
+    """search(xy, tours) of the engine -> the same on closed tours (batch, N+1), last node = first node"""
+    def closed_search(xy, t):
+        if t.dim() != 2 or t.shape[1] < 2 or not bool((t[:, -1] == t[:, 0]).all()):
+            raise ValueError("tsp tours must be (batch, N+1) closed tours (last node = first node)")
+        refined, length, iters = search(xy, t[:, :-1].contiguous())
+        return torch.cat((refined, refined[:, :1]), dim=1), length, iters
+    return closed_search
 
 
 def check_feasible(pi):

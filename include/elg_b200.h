@@ -262,8 +262,8 @@ int elg_two_opt(int problem, const float* xy, int Bxy, int N1, const int32_t* in
  *          Gain ((d(t_i-1, t_i+s) - e_i-1) - e_i+s-1) + ((d(t_j, a) - e_j) + d(b, t_j+1)), i+s wrapping to 0, with
  *          (a, b) = (t_i, t_i+s-1) forward and (t_i+s-1, t_i) reversed.
  * Gains are fp32 in the order written.  Every iteration evaluates every admissible variant and applies the smallest gain,
- * ties to the lowest key, if it is below -1e-6, at most max_iterations times.  max_segment = 0 is elg_two_opt(ELG_TSP)
- * bit for bit.  length is the closed length of the returned tour as elg_tour_length sums it.
+ * ties to the lowest key, if it is below -1e-6, at most max_iterations times.  max_segment = 0 runs
+ * elg_two_opt(ELG_TSP).  length is the closed length of the returned tour as elg_tour_length sums it.
  * N1 <= 8192 (shared memory: 14*N1 bytes). */
 int elg_tsp_local_search(const float* xy, int Bxy, int N1, const int32_t* inst, int16_t* tours, int R, int L,
                          int max_segment, int round_edges, int max_iterations, int32_t* iterations, float* length,

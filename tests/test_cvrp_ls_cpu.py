@@ -265,6 +265,6 @@ def test_stage_needs_cvrp_and_a_capacity():
     cfg = {"use_cuda": True, "cuda_device_num": 0, "params": {"aug_factor": 8, "local_search_iterations": 10}}
     with pytest.raises(ValueError, match="two_opt_iterations"):
         drv.load_model(TSPModel, cfg, "cpu")                    # what TSPLib_Tester calls
-    drv.reject_local_search({"params": {"local_search_iterations": 0}})
+    drv.reject("tsp", {"params": {"local_search_iterations": 0}})
     with pytest.raises(ValueError, match="capacity"):
         cvrp_test([], None, None, 8, local_search_iterations=10)

@@ -4,7 +4,6 @@ drivers' opt-in stage) against the CPU oracle (tests/cvrp_ls_oracle.py).
 Under the rounded library metric every edge is an integer, so gains are exact in fp32 and fp64 alike and the kernel must
 make the oracle's moves exactly.  Under the scaled metric the kernel's fp32 gains can order near-ties differently from
 the oracle's fp64 gains, so there only the invariants are exact."""
-import json
 import os
 import random
 
@@ -13,62 +12,15 @@ import pytest
 import torch
 
 import cvrp_ls_oracle as LS
+from local_search_helpers import DEV, ROOT, cfg, greedy_rows, model, setx_rows
 
 pytestmark = pytest.mark.gpu
-DEV = "cuda:0"
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "tests", "golden", "lib")
-
-
-def _cfg(ls_iterations=None):
-    from elg_b200.synth import DEFAULT_MODEL_PARAMS
-    cfg = {"name": "ELG", "use_cuda": True, "cuda_device_num": 0, "vrplib_set": "X", "load_checkpoint": None,
-           "params": {"aug_factor": 8}, "model_params": dict(DEFAULT_MODEL_PARAMS["cvrp"])}
-    if ls_iterations is not None:
-        cfg["params"]["local_search_iterations"] = ls_iterations
-    return cfg
-
-
-def _model(wseed, gain):
-    from elg_b200.cvrp import CVRPModel
-    from elg_b200.synth import synthetic_state_dict
-    m = CVRPModel(**_cfg()["model_params"])
-    m.decoder.add_local_policy(DEV)
-    m.load_state_dict(synthetic_state_dict("cvrp", seed=wseed, gain=gain))
-    return m
-
-
-def _setx_rows(name):
-    """Greedy rollout of one Set-X instance through its driver -> (unscaled xy x8 (8, N1, 2), normalised demand (8, N1),
-    integer capacity, best rows (8, L))."""
-    from elg_b200 import engine
-    from elg_b200.cvrp.test_vrplib import VRPLib_Tester
-    with open(os.path.join(LIB, "setx_ref.json")) as f:
-        ref = json.load(f)
-    z = np.load(os.path.join(LIB, "setx_inputs.npz"))
-    tester = VRPLib_Tester(_cfg(), model=_model(ref["wseed"], ref["gain"]))
-    cap, opt = z[name + "/capopt"]
-    inst = {"node_coord": z[name + "/coord"].astype(np.float64), "demand": z[name + "/demand"].astype(np.float64),
-            "capacity": float(cap), "depot": np.array([0])}
-    random.seed(ref["seed"])
-    sols, rewards = tester.test_on_one_ins(name=name, result_dict={}, instance=inst, solution=float(opt))
-    c = torch.tensor(z[name + "/coord"], dtype=torch.float32)[None].to(DEV)
-    dem = torch.tensor(z[name + "/demand"], dtype=torch.float32)[None].to(DEV) / float(cap)
-    xy, dem = engine.load_problems("cvrp", c[:, 1:], c[:, 0], dem[:, 1:], aug=8)
-    return xy, dem, int(cap), sols[torch.arange(8, device=DEV), rewards.argmax(1)]
 
 
 def _greedy_rows(N, n, seed):
-    """Greedy rollout of n random CVRP instances x 8 -> (xy, normalised demand, integer capacity, best rows)."""
-    from elg_b200 import engine
-    from elg_b200.synth import synthetic_cvrp_batch
+    """Greedy rows of n random CVRP instances x 8 -> (xy, normalised demand, integer capacity, best rows)."""
     cap = {100: 50, 1000: 250}[N]
-    b = synthetic_cvrp_batch(n, N, seed=seed, capacity=float(cap))
-    xy, dem = engine.load_problems("cvrp", b["loc"].to(DEV), b["depot"].to(DEV), b["demand"].to(DEV), aug=8)
-    from elg_b200.synth import DEFAULT_MODEL_PARAMS, synthetic_state_dict
-    h = engine.ModelHandle("cvrp", DEFAULT_MODEL_PARAMS["cvrp"], synthetic_state_dict("cvrp", seed=1234, gain=3.0), DEV)
-    tours16, reward, _, n_steps = engine.rollout(engine.encode(h, xy, dem), N, random.Random(seed).sample(range(N), N))
-    rows = tours16[torch.arange(xy.shape[0], device=DEV), reward.argmax(1), :int(n_steps.max())].long()
+    xy, dem, rows = greedy_rows("cvrp", N, n, seed, capacity=float(cap))
     return xy, dem, cap, rows
 
 
@@ -97,7 +49,7 @@ def _check_invariants(xy, dem, rows, out, length, rounding=False):
                                                 ("X-n298-k31", 3, 1000), ("X-n1001-k43", 2, 6)])
 def test_rounded_metric_identical_to_oracle(name, rows_used, cap):
     from elg_b200 import engine
-    xy, dem, capacity, rows = _setx_rows(name)
+    xy, dem, capacity, rows = setx_rows(name)
     xy, dem, rows = xy[:rows_used], dem[:rows_used], rows[:rows_used]
     out, length, iters = engine.cvrp_local_search(xy, rows, dem, capacity, max_iterations=cap, rounding=True)
     ref_t, ref_len, ref_it = _oracle(xy, dem, capacity, rows, cap, True)
@@ -233,10 +185,10 @@ def test_vrplib_driver_with_the_stage(tmp_path, capsys):
     from elg_b200.cvrp.test_vrplib import VRPLib_Tester
     out = {}
     for iters in (None, 300):
-        cfg = _cfg(iters)
-        cfg["vrplib_path"] = os.path.join(ROOT, "tests", "golden", "vrplib")
+        config = cfg("cvrp") if iters is None else cfg("cvrp", local_search_iterations=iters)
+        config["vrplib_path"] = os.path.join(ROOT, "tests", "golden", "vrplib")
         random.seed(1)
-        results = VRPLib_Tester(cfg, model=_model(3, 3.0)).test_on_vrplib(out_dir=str(tmp_path / str(iters)))
+        results = VRPLib_Tester(config, model=model("cvrp", 3, 3.0)).test_on_vrplib(out_dir=str(tmp_path / str(iters)))
         out[iters] = (capsys.readouterr().out, [r["record"][0] for r in results[:-1]])
     plain, recs = out[None]
     assert "local search" not in plain and not any(k.endswith("_ls") or k.startswith("ls_") for r in recs for k in r)
@@ -258,13 +210,13 @@ def test_test_py_with_the_stage(capsys):
     from elg_b200.cvrp.test import test
     from elg_b200.synth import synthetic_cvrp_batch
     batch = {k: v.to(DEV) for k, v in synthetic_cvrp_batch(4, 20, seed=8, capacity=30.).items()}
-    model = _model(21, 3.0).to(DEV)
+    m = model("cvrp", 21, 3.0).to(DEV)
     env = CVRPEnv(20, DEV)
     random.seed(5)
-    avg = test([batch], model, env, 8)
+    avg = test([batch], m, env, 8)
     plain = capsys.readouterr().out
     random.seed(5)
-    avg2 = test([batch], model, env, 8, local_search_iterations=100, capacity=30)
+    avg2 = test([batch], m, env, 8, local_search_iterations=100, capacity=30)
     out = capsys.readouterr().out
     assert "local search" not in plain and out.startswith(plain.split("Wall-clock")[0]) and float(avg2) == float(avg)
     line = [l for l in out.splitlines() if l.startswith("local search Aug cost: ")]

@@ -4,7 +4,6 @@ elg_b200.tsp.tsp_local_search, the drivers' opt-in stage) against the CPU oracle
 Under the rounded library metric every edge is an integer, so gains are exact in fp32 and fp64 alike and the kernel must
 make the oracle's moves exactly.  Under the scaled metric fp32 gains can order near-ties differently from fp64 ones, so
 there the invariants are checked instead.  max_segment = 0 must be elg_two_opt bit for bit in both metrics."""
-import json
 import os
 import random
 
@@ -13,12 +12,9 @@ import pytest
 import torch
 
 import tsp_ls_oracle as LS
-from test_gpu_two_opt import _greedy_rows, _lib_rows
+from local_search_helpers import DEV, LIB, greedy_rows, lib_rows, model, tsplib_driver
 
 pytestmark = pytest.mark.gpu
-DEV = "cuda:0"
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "tests", "golden", "lib")
 
 
 def _check_invariants(xy, rows, out, length, iters, max_iterations, optimum_rows=None):
@@ -40,7 +36,7 @@ def _check_invariants(xy, rows, out, length, iters, max_iterations, optimum_rows
 @pytest.mark.parametrize("name,cap", [("eil51", 1000), ("kroA100", 1000), ("a280", 30), ("rat575", 20), ("pr1002", 4)])
 def test_rounded_metric_identical_to_oracle(name, cap):
     from elg_b200 import engine
-    xy, rows, _, _ = _lib_rows("tsplib", name)
+    xy, rows, _, _ = lib_rows("tsplib", name)
     out, length, iters = engine.tsp_local_search(xy, rows, max_iterations=cap, rounding=True)
     ref_t, ref_len, ref_it = LS.tsp_local_search(xy.cpu(), rows.cpu(), cap, rounding=True)
     assert torch.equal(iters.cpu().long(), ref_it)
@@ -54,12 +50,12 @@ def test_rounded_metric_identical_to_oracle(name, cap):
 
 def test_max_segment_zero_is_two_opt():
     from elg_b200 import engine
-    xy, _, rows = _greedy_rows("tsp", 100, 64, seed=3)                     # scaled metric
+    xy, _, rows = greedy_rows("tsp", 100, 64, seed=3)                     # scaled metric
     a = engine.tsp_local_search(xy, rows, max_segment=0)
     b = engine.two_opt("tsp", xy, rows)
     assert all(torch.equal(x, y) for x, y in zip(a, b)) and int(a[2].sum()) > 0
     for name in ("eil51", "a280"):                                         # rounded metric
-        xy, rows, _, _ = _lib_rows("tsplib", name)
+        xy, rows, _, _ = lib_rows("tsplib", name)
         a = engine.tsp_local_search(xy, rows, max_segment=0, rounding=True)
         b = engine.two_opt("tsp", xy, rows, rounding=True)
         assert all(torch.equal(x, y) for x, y in zip(a, b)) and int(a[2].sum()) > 0
@@ -67,7 +63,7 @@ def test_max_segment_zero_is_two_opt():
 
 def test_shorter_segments_match_the_oracle():
     from elg_b200 import engine
-    xy, rows, _, _ = _lib_rows("tsplib", "kroA100")
+    xy, rows, _, _ = lib_rows("tsplib", "kroA100")
     for ms in (1, 2):
         out, length, iters = engine.tsp_local_search(xy, rows, max_segment=ms, rounding=True)
         ref = LS.tsp_local_search(xy.cpu(), rows.cpu(), 1000, max_segment=ms, rounding=True)
@@ -78,7 +74,7 @@ def test_shorter_segments_match_the_oracle():
 
 def test_tsp100_x8000_invariants():
     from elg_b200 import engine
-    xy, _, rows = _greedy_rows("tsp", 100, 1000, seed=100)
+    xy, _, rows = greedy_rows("tsp", 100, 1000, seed=100)
     out, length, iters = engine.tsp_local_search(xy, rows)
     _check_invariants(xy, rows, out, length, iters, 1000, optimum_rows=range(0, 8000, 40))
     two = engine.two_opt("tsp", xy, rows)[1]
@@ -87,7 +83,7 @@ def test_tsp100_x8000_invariants():
 
 def test_tsp1000_x8_invariants():
     from elg_b200 import engine
-    xy, _, rows = _greedy_rows("tsp", 1000, 1, seed=1000)
+    xy, _, rows = greedy_rows("tsp", 1000, 1, seed=1000)
     out, length, iters = engine.tsp_local_search(xy, rows, max_iterations=3000)
     _check_invariants(xy, rows, out, length, iters, 3000)
     assert int(iters.min()) > 0
@@ -156,7 +152,7 @@ def test_too_many_nodes_fails_loudly():
 
 def test_deterministic_and_idempotent():
     from elg_b200 import engine
-    xy, _, rows = _greedy_rows("tsp", 200, 16, seed=5)
+    xy, _, rows = greedy_rows("tsp", 200, 16, seed=5)
     a = engine.tsp_local_search(xy, rows)
     b = engine.tsp_local_search(xy, rows.to(torch.int16))
     assert all(torch.equal(x, y) for x, y in zip(a, b))
@@ -170,7 +166,7 @@ def test_deterministic_and_idempotent():
 def test_dropin_numpy_and_torch():
     from elg_b200 import engine
     from elg_b200.tsp import tsp_local_search
-    xy, _, rows = _greedy_rows("tsp", 50, 1, seed=9)
+    xy, _, rows = greedy_rows("tsp", 50, 1, seed=9)
     pts = xy[0]                                                            # augmentation 0 = the instance itself
     want, _, it = engine.tsp_local_search(pts[None], rows, max_iterations=500)
     closed = torch.cat((rows, rows[:, :1]), 1)
@@ -189,42 +185,22 @@ def test_dropin_numpy_and_torch():
 
 # ------------------------------------------------------------------------------------------------ 6. drivers
 
-def _tsplib_driver(name, params):
-    """The TSPLIB driver on one instance with extra config params -> (record, unscaled xy, best rows)."""
-    from elg_b200.synth import DEFAULT_MODEL_PARAMS, synthetic_state_dict
-    from elg_b200.tsp import TSPModel
-    from elg_b200.tsp.test_tsplib import TSPLib_Tester
-    with open(os.path.join(LIB, "tsplib_ref.json")) as f:
-        ref = json.load(f)
-    z = np.load(os.path.join(LIB, "tsplib_inputs.npz"))
-    cfg = {"name": "ELG", "use_cuda": True, "cuda_device_num": 0, "load_checkpoint": None,
-           "params": dict(aug_factor=8, **params), "model_params": dict(DEFAULT_MODEL_PARAMS["tsp"])}
-    m = TSPModel(**cfg["model_params"])
-    m.decoder.add_local_policy(DEV)
-    m.load_state_dict(synthetic_state_dict("tsp", seed=ref["wseed"], gain=ref["gain"]))
-    random.seed(ref["seed"])
-    res = {}
-    sols, rewards = TSPLib_Tester(cfg, model=m).test_on_one_ins(name, res, [z[name + "/coord"], float(z[name + "/opt"])])
-    return res, sols[torch.arange(rewards.shape[0], device=DEV), rewards.argmax(1)]
-
-
 def test_library_driver_refines_with_or_opt():
-    xy, rows, res_off, opt = _lib_rows("tsplib", "eil51")
-    res, rows_on = _tsplib_driver("eil51", {"tsp_local_search_iterations": 200})
+    xy, rows, res_off, opt = lib_rows("tsplib", "eil51")
+    res, rows_on = tsplib_driver("eil51", {"tsp_local_search_iterations": 200})
     assert torch.equal(rows_on, rows) and res["best_cost"] == res_off["best_cost"]
     assert not any("tsp_ls" in k for k in res_off)
     _, ref_len, ref_it = LS.tsp_local_search(xy.cpu(), rows.cpu(), 200, rounding=True)
     assert res["best_cost_tsp_ls"] == float(ref_len.min()) <= res["best_cost"]
     assert res["gap_tsp_ls"] == (res["best_cost_tsp_ls"] - opt) / opt
     assert res["tsp_ls_iterations"] == int(ref_it.sum()) > 0 and res["tsp_ls_seconds"] > 0
-    both, _ = _tsplib_driver("eil51", {"two_opt_iterations": 200, "tsp_local_search_iterations": 200})
+    both, _ = tsplib_driver("eil51", {"two_opt_iterations": 200, "tsp_local_search_iterations": 200})
     assert both["best_cost_tsp_ls"] == res["best_cost_tsp_ls"] and "best_cost_2opt" in both
 
 
 def test_tsplib_driver_prints_and_records(tmp_path, capsys):
     import pickle
-    from elg_b200.synth import DEFAULT_MODEL_PARAMS, synthetic_state_dict
-    from elg_b200.tsp import TSPModel
+    from elg_b200.synth import DEFAULT_MODEL_PARAMS
     from elg_b200.tsp.test_tsplib import TSPLib_Tester
     z = np.load(os.path.join(LIB, "tsplib_inputs.npz"))
     d = tmp_path / "TSPLib"
@@ -236,11 +212,8 @@ def test_tsplib_driver_prints_and_records(tmp_path, capsys):
         cfg = {"name": "ELG", "use_cuda": True, "cuda_device_num": 0, "tsplib_path": str(d), "load_checkpoint": None,
                "params": {"aug_factor": 8, "tsp_local_search_iterations": iters},
                "model_params": dict(DEFAULT_MODEL_PARAMS["tsp"])}
-        m = TSPModel(**cfg["model_params"])
-        m.decoder.add_local_policy(DEV)
-        m.load_state_dict(synthetic_state_dict("tsp", seed=3, gain=3.0))
         random.seed(1)
-        results = TSPLib_Tester(cfg, model=m).test_on_tsplib(out_dir=str(tmp_path / ("out%d" % iters)))
+        results = TSPLib_Tester(cfg, model=model("tsp", 3, 3.0)).test_on_tsplib(out_dir=str(tmp_path / ("out%d" % iters)))
         out = capsys.readouterr().out
         recs = [r["record"][0] for r in results]
         if iters:
@@ -251,21 +224,18 @@ def test_tsplib_driver_prints_and_records(tmp_path, capsys):
 
 
 def test_test_py_with_or_opt(capsys):
-    from elg_b200.synth import DEFAULT_MODEL_PARAMS, synthetic_state_dict, synthetic_tsp_batch
-    from elg_b200.tsp import TSPEnv, TSPModel
+    from elg_b200.synth import synthetic_tsp_batch
+    from elg_b200.tsp import TSPEnv
     from elg_b200.tsp.test import test
     batch = synthetic_tsp_batch(4, 20, seed=8).to(DEV)
-    model = TSPModel(**DEFAULT_MODEL_PARAMS["tsp"])
-    model.decoder.add_local_policy(DEV)
-    model.load_state_dict(synthetic_state_dict("tsp", seed=21, gain=3.0))
-    model = model.to(DEV)
+    m = model("tsp", 21, 3.0).to(DEV)
     env = TSPEnv(20, DEV)
     random.seed(5)
-    avg = test([batch], model, env, 8)
+    avg = test([batch], m, env, 8)
     plain = capsys.readouterr().out
     assert "or-opt" not in plain
     random.seed(5)
-    avg2 = test([batch], model, env, 8, two_opt_iterations=100, tsp_local_search_iterations=100)
+    avg2 = test([batch], m, env, 8, two_opt_iterations=100, tsp_local_search_iterations=100)
     out = capsys.readouterr().out
     assert out.startswith(plain.split("Wall-clock")[0]) and float(avg2) == float(avg)
     lines = out.splitlines()

@@ -4,7 +4,6 @@ against the CPU oracle (tests/two_opt_oracle.py).
 Under the rounded library metric every edge is an integer, so gains are exact in fp32 and fp64 alike and the kernel must
 make the oracle's moves exactly.  Under the scaled metric the kernel's fp32 gains can order near-ties differently from the
 oracle's fp64 gains, so there the invariants are exact and the tours only mostly equal."""
-import json
 import os
 import random
 
@@ -13,79 +12,10 @@ import pytest
 import torch
 
 import two_opt_oracle as TO
+from local_search_helpers import DEV, LIB, greedy_rows, lib_rows, model
 from oracle import elg_oracle as O
 
 pytestmark = pytest.mark.gpu
-DEV = "cuda:0"
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "tests", "golden", "lib")
-
-
-def _model(problem, wseed=1234, gain=3.0):
-    from elg_b200.synth import DEFAULT_MODEL_PARAMS, synthetic_state_dict
-    from elg_b200 import engine
-    return engine.ModelHandle(problem, DEFAULT_MODEL_PARAMS[problem], synthetic_state_dict(problem, seed=wseed, gain=gain), DEV)
-
-
-def _greedy_rows(problem, N, n, seed, aug=8):
-    """Greedy rollout of n random instances x aug with the synthetic model -> (xy (B, N1, 2), demand | None,
-    best POMO row of every aug-instance (B, L) int64), all on the GPU."""
-    from elg_b200 import engine
-    from elg_b200.synth import synthetic_cvrp_batch, synthetic_tsp_batch
-    if problem == "cvrp":
-        b = synthetic_cvrp_batch(n, N, seed=seed)
-        xy, dem = engine.load_problems("cvrp", b["loc"].to(DEV), b["depot"].to(DEV), b["demand"].to(DEV), aug=aug)
-    else:
-        xy, dem = engine.load_problems("tsp", synthetic_tsp_batch(n, N, seed=seed).to(DEV), aug=aug)
-    batch = engine.encode(_model(problem), xy, dem)
-    M = N
-    rng = random.Random(seed)
-    tours16, reward, _, n_steps = engine.rollout(batch, M, rng.sample(range(N), M))
-    T = int(n_steps.max()) if problem == "cvrp" else N
-    rows = tours16[torch.arange(xy.shape[0], device=DEV), reward.argmax(1), :T].long()
-    return xy, dem, rows
-
-
-def _lib_rows(kind, name, two_opt_iterations=None):
-    """Greedy rollout of one library instance through its driver -> (unscaled xy (B or 1, N1, 2), best rows (B, L),
-    the driver's record, the optimal cost).  two_opt_iterations: params.two_opt_iterations (None: key absent)."""
-    with open(os.path.join(LIB, kind + "_ref.json")) as f:
-        ref = json.load(f)
-    z = np.load(os.path.join(LIB, kind + "_inputs.npz"))
-    from elg_b200.synth import DEFAULT_MODEL_PARAMS, synthetic_state_dict
-    problem = "cvrp" if kind == "setx" else "tsp"
-    cfg = {"name": "ELG", "use_cuda": True, "cuda_device_num": 0, "vrplib_set": "X", "load_checkpoint": None,
-           "params": {"aug_factor": 8}, "model_params": dict(DEFAULT_MODEL_PARAMS[problem])}
-    if two_opt_iterations is not None:
-        cfg["params"]["two_opt_iterations"] = two_opt_iterations
-    sd = synthetic_state_dict(problem, seed=ref["wseed"], gain=ref["gain"])
-    random.seed(ref["seed"])
-    if problem == "cvrp":
-        from elg_b200.cvrp import CVRPModel as Model
-        from elg_b200.cvrp.test_vrplib import VRPLib_Tester as Tester
-    else:
-        from elg_b200.tsp import TSPModel as Model
-        from elg_b200.tsp.test_tsplib import TSPLib_Tester as Tester
-    m = Model(**cfg["model_params"])
-    m.decoder.add_local_policy(DEV)
-    m.load_state_dict(sd)
-    tester = Tester(cfg, model=m)
-    res = {}
-    if problem == "cvrp":
-        cap, opt = z[name + "/capopt"]
-        inst = {"node_coord": z[name + "/coord"].astype(np.float64), "demand": z[name + "/demand"].astype(np.float64),
-                "capacity": float(cap), "depot": np.array([0])}
-        sols, rewards = tester.test_on_one_ins(name=name, result_dict=res, instance=inst, solution=float(opt))
-        xy = torch.tensor(z[name + "/coord"], dtype=torch.float32)[None]
-        from elg_b200 import engine
-        xy = engine.load_problems("cvrp", xy[:, 1:].to(DEV), xy[:, 0].to(DEV),
-                                  torch.zeros(1, xy.shape[1] - 1, device=DEV), aug=8)[0]   # x8 unscaled, as the driver
-    else:
-        opt = float(z[name + "/opt"])
-        sols, rewards = tester.test_on_one_ins(name, res, [z[name + "/coord"], opt])
-        xy = torch.tensor(z[name + "/coord"], dtype=torch.float32)[None].to(DEV)           # shared by all augmentations
-    B = rewards.shape[0]
-    return xy, sols[torch.arange(B, device=DEV), rewards.argmax(1)], res, float(opt)
 
 
 def _oracle(problem, xy, rows, max_iterations, rounding):
@@ -138,7 +68,7 @@ def _check_invariants(problem, xy, rows, out, length, iters, max_iterations, dem
 def test_rounded_metric_identical_to_oracle(kind, name, cap):
     from elg_b200 import engine
     problem = "cvrp" if kind == "setx" else "tsp"
-    xy, rows, _, _ = _lib_rows(kind, name)
+    xy, rows, _, _ = lib_rows(kind, name)
     out, length, iters = engine.two_opt(problem, xy, rows, max_iterations=cap, rounding=True)
     ref_t, ref_len, ref_it = _oracle(problem, xy, rows, cap, True)
     assert torch.equal(iters.cpu().long(), ref_it)
@@ -154,7 +84,7 @@ def test_random_instances_scaled_metric(problem):
     from elg_b200 import engine
     same, total = 0, 0
     for N in (20, 50, 100, 200, 500):
-        xy, dem, rows = _greedy_rows(problem, N, 4, seed=N)
+        xy, dem, rows = greedy_rows(problem, N, 4, seed=N)
         out, length, iters = engine.two_opt(problem, xy, rows, max_iterations=1000)
         _check_invariants(problem, xy, rows, out, length, iters, 1000, dem)
         k = 32 if N <= 100 else (8 if N == 200 else 3)                       # oracle time grows as N^2 per move
@@ -205,7 +135,7 @@ def test_cvrp_short_routes_padding_and_shared_coordinates():
 
 def test_many_tours_persistent_loop():
     from elg_b200 import engine
-    xy, _, rows = _greedy_rows("tsp", 100, 250, seed=7)                     # 2000 tours, far above the SM count
+    xy, _, rows = greedy_rows("tsp", 100, 250, seed=7)                     # 2000 tours, far above the SM count
     out, length, iters = engine.two_opt("tsp", xy, rows)
     _check_invariants("tsp", xy, rows, out, length, iters, 1000)
     parts = [engine.two_opt("tsp", xy[s:s + 100], rows[s:s + 100]) for s in range(0, 2000, 100)]
@@ -249,7 +179,7 @@ def test_too_many_nodes_fails_loudly():
 @pytest.mark.parametrize("problem", ["tsp", "cvrp"])
 def test_deterministic_and_idempotent(problem):
     from elg_b200 import engine
-    xy, _, rows = _greedy_rows(problem, 100, 16, seed=5)
+    xy, _, rows = greedy_rows(problem, 100, 16, seed=5)
     a = engine.two_opt(problem, xy, rows)
     b = engine.two_opt(problem, xy, rows.to(torch.int16))
     assert all(torch.equal(x, y) for x, y in zip(a, b))
@@ -265,7 +195,7 @@ def test_batched_two_opt_torch(problem):
     from elg_b200 import engine
     from elg_b200.cvrp import batched_two_opt_torch as cvrp_2opt
     from elg_b200.tsp import batched_two_opt_torch as tsp_2opt
-    xy, _, rows = _greedy_rows(problem, 50, 1, seed=9)
+    xy, _, rows = greedy_rows(problem, 50, 1, seed=9)
     pts, rows = xy[0], rows                                           # augmentation 0 = the instance itself
     want, _, it = engine.two_opt(problem, pts[None], rows, max_iterations=500)
     if problem == "tsp":
@@ -288,9 +218,9 @@ def test_batched_two_opt_torch(problem):
 def test_library_drivers_refine_with_2opt():
     for kind, name in (("tsplib", "eil51"), ("tsplib", "berlin52"), ("setx", "X-n101-k25")):
         problem = "cvrp" if kind == "setx" else "tsp"
-        xy, rows, res_off, opt = _lib_rows(kind, name)
+        xy, rows, res_off, opt = lib_rows(kind, name)
         assert not any("2opt" in k or "two_opt" in k for k in res_off)        # key absent: no new fields
-        _, rows_on, res, _ = _lib_rows(kind, name, 200)
+        _, rows_on, res, _ = lib_rows(kind, name, 200)
         assert torch.equal(rows_on, rows) and res["best_cost"] == res_off["best_cost"]
         _, ref_len, ref_it = _oracle(problem, xy, rows, 200, True)
         assert res["best_cost_2opt"] == float(ref_len.min()) <= res["best_cost"]
@@ -311,13 +241,8 @@ def test_tsplib_driver_prints_and_records(tmp_path, capsys):
     for iters in (0, 100):
         cfg = {"name": "ELG", "use_cuda": True, "cuda_device_num": 0, "tsplib_path": str(d), "load_checkpoint": None,
                "params": {"aug_factor": 8, "two_opt_iterations": iters}, "model_params": dict(DEFAULT_MODEL_PARAMS["tsp"])}
-        from elg_b200.tsp import TSPModel
-        m = TSPModel(**cfg["model_params"])
-        m.decoder.add_local_policy(DEV)
-        from elg_b200.synth import synthetic_state_dict
-        m.load_state_dict(synthetic_state_dict("tsp", seed=3, gain=3.0))
         random.seed(1)
-        results = TSPLib_Tester(cfg, model=m).test_on_tsplib(out_dir=str(tmp_path / ("out%d" % iters)))
+        results = TSPLib_Tester(cfg, model=model("tsp", 3, 3.0)).test_on_tsplib(out_dir=str(tmp_path / ("out%d" % iters)))
         out = capsys.readouterr().out
         recs = [r["record"][0] for r in results]
         if iters:
@@ -329,26 +254,23 @@ def test_tsplib_driver_prints_and_records(tmp_path, capsys):
 
 @pytest.mark.parametrize("kind", ["cvrp", "tsp"])
 def test_test_py_with_2opt(kind, capsys):
-    from elg_b200.synth import DEFAULT_MODEL_PARAMS, synthetic_cvrp_batch, synthetic_state_dict, synthetic_tsp_batch
+    from elg_b200.synth import synthetic_cvrp_batch, synthetic_tsp_batch
     if kind == "cvrp":
-        from elg_b200.cvrp import CVRPEnv as Env, CVRPModel as Model
+        from elg_b200.cvrp import CVRPEnv as Env
         from elg_b200.cvrp.test import test
         batch = {k: v.to(DEV) for k, v in synthetic_cvrp_batch(4, 20, seed=8).items()}
     else:
-        from elg_b200.tsp import TSPEnv as Env, TSPModel as Model
+        from elg_b200.tsp import TSPEnv as Env
         from elg_b200.tsp.test import test
         batch = synthetic_tsp_batch(4, 20, seed=8).to(DEV)
-    model = Model(**DEFAULT_MODEL_PARAMS[kind])
-    model.decoder.add_local_policy(DEV)
-    model.load_state_dict(synthetic_state_dict(kind, seed=21, gain=3.0))
-    model = model.to(DEV)
+    m = model(kind, 21, 3.0).to(DEV)
     env = Env(20, DEV)
     random.seed(5)
-    avg = test([batch], model, env, 8)
+    avg = test([batch], m, env, 8)
     plain = capsys.readouterr().out
     assert "2-opt" not in plain
     random.seed(5)
-    avg2 = test([batch], model, env, 8, two_opt_iterations=100)
+    avg2 = test([batch], m, env, 8, two_opt_iterations=100)
     out = capsys.readouterr().out
     assert out.startswith(plain.split("Wall-clock")[0]) and float(avg2) == float(avg)
     line = [l for l in out.splitlines() if l.startswith("2-opt Aug cost: ")]

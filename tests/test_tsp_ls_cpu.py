@@ -282,9 +282,9 @@ def test_cvrp_models_reject_the_key():
     with pytest.raises(ValueError, match="local_search_iterations"):
         drv.load_model(CVRPModel, cfg, "cpu")                   # what VRPLib_Tester calls
     with pytest.raises(ValueError, match="params.local_search_iterations"):
-        drv.reject_tsp_local_search(cfg)                        # cvrp/test.py
-    drv.reject_tsp_local_search({"params": {"tsp_local_search_iterations": 0}})
-    drv.reject_tsp_local_search({"params": {}})
+        drv.reject("cvrp", cfg)                                 # cvrp/test.py
+    drv.reject("cvrp", {"params": {"tsp_local_search_iterations": 0}})
+    drv.reject("cvrp", {"params": {}})
     cfg["params"]["local_search_iterations"] = 10               # the TSP rejection of the CVRP key is unchanged
     with pytest.raises(ValueError, match="two_opt_iterations"):
         drv.load_model(TSPModel, cfg, "cpu")

@@ -161,6 +161,8 @@ def test_engine_and_drop_in_reject_the_cpu():
     xy = torch.rand(1, 10, 2)
     with pytest.raises(_lib.ElgError):
         engine.two_opt("tsp", xy, torch.arange(10)[None])
+    with pytest.raises(ValueError, match="inst"):                                    # Bxy neither 1 nor R, before the
+        engine.two_opt("tsp", xy.expand(3, -1, -1), torch.arange(10).expand(2, -1))  # device check
     from elg_b200.cvrp import batched_two_opt_torch as cvrp_2opt
     from elg_b200.tsp import batched_two_opt_torch as tsp_2opt
     with pytest.raises(_lib.ElgError):
