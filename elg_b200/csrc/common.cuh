@@ -126,18 +126,21 @@ __device__ __forceinline__ float edge_len(const float2* __restrict__ xy, int a, 
   return round_edges ? rintf(d) : d;
 }
 
-// (gain, key) ordered by gain, then by key: torch.argmin's first-index tie-break
-__device__ __forceinline__ bool gain_better(float g, int key, float bg, int bkey) {
+// (gain, key) ordered by gain, then by key: torch.argmin's first-index tie-break.  K is int, or unsigned where the keys
+// can pass 2^31-1 (cvrp_ls.cu with segment moves).
+template <typename K>
+__device__ __forceinline__ bool gain_better(float g, K key, float bg, K bkey) {
   return g < bg || (g == bg && key < bkey);
 }
 
 // CTA-wide minimum of every thread's (bg, bkey) under gain_better, returned to every thread.  red_g / red_k hold one
 // entry per warp; a barrier must separate the reads here from the next writes to them.
-__device__ __forceinline__ void cta_min_gain(float& bg, int& bkey, float* red_g, int* red_k) {
+template <typename K>
+__device__ __forceinline__ void cta_min_gain(float& bg, K& bkey, float* red_g, K* red_k) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
   for (int o = 16; o > 0; o >>= 1) {
     const float g = __shfl_xor_sync(0xffffffffu, bg, o);
-    const int k = __shfl_xor_sync(0xffffffffu, bkey, o);
+    const K k = __shfl_xor_sync(0xffffffffu, bkey, o);
     if (gain_better(g, k, bg, bkey)) { bg = g; bkey = k; }
   }
   if (lane == 0) { red_g[warp] = bg; red_k[warp] = bkey; }

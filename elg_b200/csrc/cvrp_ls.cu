@@ -1,5 +1,6 @@
-// Best-improvement CVRP local search with capacity (elg_cvrp_local_search): 2-opt inside a route, relocate of one
-// customer, swap of two customers of different routes, and 2-opt* (tail exchange) between two routes.
+// Best-improvement CVRP local search with capacity (elg_cvrp_local_search_ex): 2-opt inside a route, relocate of one
+// customer, swap of two customers of different routes, 2-opt* (tail exchange) between two routes, and with
+// max_segment > 1 Or-opt moves of a chain of 2 or 3 customers, forward or reversed, within or between routes.
 //
 // One CTA refines one row at a time and is persistent over the R rows.  The whole solution lives in shared memory and
 // global memory is touched only to load the row and to write the result:
@@ -12,11 +13,16 @@
 //
 // Per move every position i (positions 0..P-1, P = 1 + last customer position) sweeps the positions j in chunks of
 // CVRP_LS_CHUNK; consecutive j share d(t_j, t_i) and d(t_j, t_j+1), so a pair costs two distances plus one to three for
-// the move types that apply to it.  The CTA reduces (gain, type*L^2 + i*L + j) to its minimum.  Every applied move is a
-// composition of reversals of row spans; a route emptied by it leaves two adjacent depot visits, one of which is rotated
-// to the end of the used positions.  The route starts and load prefixes are then rebuilt from the first changed route
-// to the end of the used positions with one segmented scan.
+// the move types that apply to it.  The kernel is instantiated for the longest segment SEG (1, 2, 3): for SEG > 1 the
+// sweep also carries A_1(j) = d(t_j, t_i+1) and, for SEG = 3, A_2(j) = d(t_j, t_i+2) from one j to the next, which
+// cover every insertion term of the segment moves (and the 2-opt and swap terms that used t_i+1), while their removal
+// terms cost four distances per task.  The CTA reduces (gain, type*L^2 + i*L + j) to its minimum; with eight move types
+// the key passes 2^31-1 for L > 16384, so SEG > 1 keys are unsigned.  Every applied move is a composition of reversals
+// of row spans; a route emptied by it leaves two adjacent depot visits, one of which is rotated to the end of the used
+// positions.  The route starts and load prefixes are then rebuilt from the first changed route to the end of the used
+// positions with one segmented scan.
 #include <climits>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -62,6 +68,7 @@ __device__ __forceinline__ void rebuild_routes(const int16_t* row, const int32_t
   __syncthreads();
 }
 
+template <int SEG>
 __global__ void __launch_bounds__(512, 1) cvrp_ls_kernel(const float* __restrict__ xy_g, int Bxy, int N1,
                                                        const int32_t* __restrict__ dem_g, int capacity,
                                                        const int32_t* __restrict__ inst, int16_t* __restrict__ tours,
@@ -77,7 +84,8 @@ __global__ void __launch_bounds__(512, 1) cvrp_ls_kernel(const float* __restrict
   int16_t* row = reinterpret_cast<int16_t*>(dem + N1);
   int16_t* rs = row + L;
   const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, warp = tid >> 5;
-  const int LL = L * L;
+  using Key = typename std::conditional<SEG == 1, int, unsigned>::type;
+  const Key LL = (Key)L * L;
 
   for (int r = blockIdx.x; r < R; r += gridDim.x) {
     const int b = ls_instance(inst, Bxy, r);
@@ -114,7 +122,7 @@ __global__ void __launch_bounds__(512, 1) cvrp_ls_kernel(const float* __restrict
     int moves = 0;
     while (moves < max_iterations) {
       float bg = INFINITY;
-      int bk = INT_MAX;
+      Key bk = SEG == 1 ? (Key)INT_MAX : (Key)UINT_MAX;
       const int nch = (P + CVRP_LS_CHUNK - 1) / CVRP_LS_CHUNK;
       for (int task = tid; task < P * nch; task += nthr) {
         const int i = task / nch, j0 = (task % nch) * CVRP_LS_CHUNK, j1 = min(j0 + CVRP_LS_CHUNK, P);
@@ -122,40 +130,80 @@ __global__ void __launch_bounds__(512, 1) cvrp_ls_kernel(const float* __restrict
         const float e_im1 = edge_len(xy, a, u, round_edges), e_i = edge_len(xy, u, bn, round_edges);
         const float rem = edge_len(xy, a, bn, round_edges) - e_im1 - e_i;        // relocate: u taken out
         const int du = dem[u], load_a = pref[ri], pre_a = u ? pref[i] : 0;
+        // segments t_i..t_i+s-1 (s = 2, 3) taken out: t_i-1 joined to t_i+s; loads from the demands
+        int c2 = 0, load2 = 0, load3 = 0;
+        bool ok2 = false, ok3 = false;
+        float rem2 = 0.f, rem3 = 0.f;
+        if constexpr (SEG >= 2) {
+          c2 = i + 2 < P ? row[i + 2] : 0;
+          ok2 = u != 0 && bn != 0;
+          load2 = du + dem[bn];
+          if (ok2) rem2 = (edge_len(xy, a, c2, round_edges) - e_im1) - edge_len(xy, bn, c2, round_edges);
+        }
+        if constexpr (SEG >= 3) {
+          const int c3 = i + 3 < P ? row[i + 3] : 0;
+          ok3 = ok2 && c2 != 0;
+          load3 = load2 + dem[c2];
+          if (ok3) rem3 = (edge_len(xy, a, c3, round_edges) - e_im1) - edge_len(xy, c2, c3, round_edges);
+        }
         const int t0 = row[j0], tm1 = j0 > 0 ? row[j0 - 1] : 0;
         float dju = edge_len(xy, t0, u, round_edges);                             // d(t_j, u)
         float djm1u = edge_len(xy, tm1, u, round_edges);                          // d(t_j-1, u)
         float ejm1 = edge_len(xy, tm1, t0, round_edges);                          // d(t_j-1, t_j)
+        float dj1 = 0.f, dj2 = 0.f;                                               // d(t_j, t_i+1), d(t_j, t_i+2)
+        if constexpr (SEG >= 2) dj1 = edge_len(xy, t0, bn, round_edges);
+        if constexpr (SEG >= 3) if (ok3) dj2 = edge_len(xy, t0, c2, round_edges);
         for (int j = j0; j < j1; ++j) {
           const int tj = row[j], tj1 = j + 1 < P ? row[j + 1] : 0, rj = rs[j];
           const float dj1u = edge_len(xy, tj1, u, round_edges), ej = edge_len(xy, tj, tj1, round_edges);
+          float dj11 = 0.f, dj12 = 0.f;                                           // the same for t_j+1
+          if constexpr (SEG >= 2) dj11 = edge_len(xy, tj1, bn, round_edges);
+          if constexpr (SEG >= 3) if (ok3) dj12 = edge_len(xy, tj1, c2, round_edges);
           if (j >= i + 2 && rj <= i) {                                            // 0: reverse i+1..j inside a route
-            const float g = (dju - e_i) + (edge_len(xy, bn, tj1, round_edges) - ej);
-            if (gain_better(g, i * L + j, bg, bk)) { bg = g; bk = i * L + j; }
+            const float g = (dju - e_i) + ((SEG >= 2 ? dj11 : edge_len(xy, bn, tj1, round_edges)) - ej);
+            if (gain_better<Key>(g, i * L + j, bg, bk)) { bg = g; bk = i * L + j; }
           }
           if (u != 0 && j != i - 1 && j != i && (rj == ri || pref[rj] + du <= capacity)) {   // 1: u onto (t_j, t_j+1)
             const float g = rem + ((dju + dj1u) - ej);
-            const int key = LL + i * L + j;
+            const Key key = LL + i * L + j;
             if (gain_better(g, key, bg, bk)) { bg = g; bk = key; }
           }
           if (j > i && rj != ri) {
-            const float dvb = edge_len(xy, tj, bn, round_edges);
+            const float dvb = SEG >= 2 ? dj1 : edge_len(xy, tj, bn, round_edges);
             const int dv = dem[tj], load_b = pref[rj], pre_b = tj ? pref[j] : 0;
             if (u != 0 && tj != 0 && load_a - du + dv <= capacity && load_b - dv + du <= capacity) {   // 2: swap
               const float g = ((edge_len(xy, a, tj, round_edges) + dvb) - (e_im1 + e_i)) + ((djm1u + dj1u) - (ejm1 + ej));
-              const int key = 2 * LL + i * L + j;
+              const Key key = 2 * LL + i * L + j;
               if (gain_better(g, key, bg, bk)) { bg = g; bk = key; }
             }
             if (pre_a + load_b - pre_b <= capacity && pre_b + load_a - pre_a <= capacity) {          // 3: 2-opt*
               const float g = (dj1u - e_i) + (dvb - ej);
-              const int key = 3 * LL + i * L + j;
+              const Key key = 3 * LL + i * L + j;
               if (gain_better(g, key, bg, bk)) { bg = g; bk = key; }
             }
+          }
+          if constexpr (SEG >= 2) {                     // 4 / 5: t_i t_i+1 onto (t_j, t_j+1), forward / reversed
+            if (ok2 && (j < i - 1 || j > i + 1) && (rj == ri || pref[rj] + load2 <= capacity)) {
+              const float gf = rem2 + ((dju - ej) + dj11), gr = rem2 + ((dj1 - ej) + dj1u);
+              const Key key = 4 * LL + i * L + j;
+              if (gain_better(gf, key, bg, bk)) { bg = gf; bk = key; }
+              if (gain_better(gr, key + LL, bg, bk)) { bg = gr; bk = key + LL; }
+            }
+            dj1 = dj11;
+          }
+          if constexpr (SEG >= 3) {                     // 6 / 7: t_i t_i+1 t_i+2 onto (t_j, t_j+1), forward / reversed
+            if (ok3 && (j < i - 1 || j > i + 2) && (rj == ri || pref[rj] + load3 <= capacity)) {
+              const float gf = rem3 + ((dju - ej) + dj12), gr = rem3 + ((dj2 - ej) + dj1u);
+              const Key key = 6 * LL + i * L + j;
+              if (gain_better(gf, key, bg, bk)) { bg = gf; bk = key; }
+              if (gain_better(gr, key + LL, bg, bk)) { bg = gr; bk = key + LL; }
+            }
+            dj2 = dj12;
           }
           djm1u = dju; dju = dj1u; ejm1 = ej;
         }
       }
-      cta_min_gain(bg, bk, red_g, red_a);
+      cta_min_gain(bg, bk, red_g, reinterpret_cast<Key*>(red_a));
       if (!(bg < LS_MIN_GAIN)) break;                   // every thread reads the same reduction: uniform exit
       const int type = bk / LL, i = bk % LL / L, j = bk % L;
       const int lo = rs[min(i, j)];                     // first route the move changes
@@ -166,7 +214,7 @@ __global__ void __launch_bounds__(512, 1) cvrp_ls_kernel(const float* __restrict
         else { reverse_span(row, j + 1, i); __syncthreads(); reverse_span(row, j + 2, i); }
       } else if (type == 2) {
         if (tid == 0) { const int16_t t = row[i]; row[i] = row[j]; row[j] = t; }
-      } else {
+      } else if (SEG == 1 || type == 3) {
         // [X Z Y] -> [Y Z X] with X = A after i, Z = the routes between up to B's head, Y = B after j
         if (tid == 0) { s_pos[0] = P; s_pos[1] = P; }
         __syncthreads();
@@ -179,6 +227,14 @@ __global__ void __launch_bounds__(512, 1) cvrp_ls_kernel(const float* __restrict
         reverse_span(row, i + 1, i + ny);
         reverse_span(row, i + 1 + ny, i + ny + nz);
         reverse_span(row, i + 1 + ny + nz, eb);
+      } else {
+        // segment S = i..last and the run T between it and the insertion edge: [S T] -> [T S] (j > i) or
+        // [T S] -> [S T] (j < i) is reverse S, reverse T, reverse both; a reversed insertion skips reversing S
+        const int last = i + type / 2 - 1;
+        if (!(type & 1)) reverse_span(row, i, last);
+        if (j > i) reverse_span(row, last + 1, j); else reverse_span(row, j + 1, i - 1);
+        __syncthreads();
+        if (j > i) reverse_span(row, i, j); else reverse_span(row, j + 1, last);
       }
       __syncthreads();
       if (tid == 0) s_pos[0] = P;                       // an emptied route: two adjacent depot visits
@@ -213,15 +269,24 @@ using namespace elg;
 
 extern "C" {
 
-int elg_cvrp_local_search(const float* xy, int Bxy, int N1, const int32_t* demand, int32_t capacity, const int32_t* inst,
-                          int16_t* tours, int R, int L, int round_edges, int max_iterations, int32_t* iterations,
-                          float* length, void* stream) {
+int elg_cvrp_local_search_ex(const float* xy, int Bxy, int N1, const int32_t* demand, int32_t capacity,
+                             const int32_t* inst, int16_t* tours, int R, int L, int max_segment, int round_edges,
+                             int max_iterations, int32_t* iterations, float* length, void* stream) {
   if (int e = ls_check_args("cvrp local search", xy, Bxy, N1, inst, tours, R, max_iterations, iterations, length)) return e;
   ELG_REQUIRE(L > 0 && L <= 2 * N1 + 2, ELG_EINVAL, "rows need 0 < L <= 2*N1+2 (L=%d, N1=%d)", L, N1);
   ELG_REQUIRE(capacity > 0, ELG_EINVAL, "capacity must be > 0 (got %d)", capacity);
   ELG_REQUIRE(demand, ELG_EINVAL, "NULL pointer");
-  return ls_launch(cvrp_ls_kernel, cvrp_ls_smem_bytes(N1, L), L, R, stream, "cvrp local search", N1, L, xy, Bxy, N1,
-                   demand, capacity, inst, tours, R, L, round_edges, max_iterations, iterations, length);
+  ELG_REQUIRE(max_segment >= 1 && max_segment <= 3, ELG_EINVAL, "max_segment must be 1, 2 or 3 (got %d)", max_segment);
+  auto* kernel = max_segment == 1 ? cvrp_ls_kernel<1> : max_segment == 2 ? cvrp_ls_kernel<2> : cvrp_ls_kernel<3>;
+  return ls_launch(kernel, cvrp_ls_smem_bytes(N1, L), L, R, stream, "cvrp local search", N1, L, xy, Bxy, N1, demand,
+                   capacity, inst, tours, R, L, round_edges, max_iterations, iterations, length);
+}
+
+int elg_cvrp_local_search(const float* xy, int Bxy, int N1, const int32_t* demand, int32_t capacity, const int32_t* inst,
+                          int16_t* tours, int R, int L, int round_edges, int max_iterations, int32_t* iterations,
+                          float* length, void* stream) {
+  return elg_cvrp_local_search_ex(xy, Bxy, N1, demand, capacity, inst, tours, R, L, 1, round_edges, max_iterations,
+                                  iterations, length, stream);
 }
 
 }  // extern "C"

@@ -30,11 +30,13 @@ def solve_batch(model, env, batch, aug_factor):
     return no_aug_cost, aug_cost, solutions, rewards
 
 
-def test(dataloader, model, env, aug_factor, two_opt_iterations=0, local_search_iterations=0, capacity=None):
+def test(dataloader, model, env, aug_factor, two_opt_iterations=0, local_search_iterations=0, capacity=None,
+         local_search_max_segment=1):
     """two_opt_iterations > 0 (config params.two_opt_iterations) also refines the best POMO row of every aug-instance
     with 2-opt in the reward metric and prints the refined cost after the reference's lines.  local_search_iterations > 0
     (params.local_search_iterations) does the same with the capacity-aware local search, independently of the 2-opt
-    stage; it needs the integer vehicle capacity the batches' demands are normalised by."""
+    stage; it needs the integer vehicle capacity the batches' demands are normalised by, and moves chains of up to
+    local_search_max_segment customers (params.local_search_max_segment)."""
     if local_search_iterations and capacity is None:
         raise ValueError("the local search stage needs the capacity the demands are normalised by")
     model.eval()
@@ -50,7 +52,7 @@ def test(dataloader, model, env, aug_factor, two_opt_iterations=0, local_search_
         no_avg_cost_total += no_aug_cost.mean()
         for (stage, iterations), total in zip(stages, totals):
             cost, seconds, moves = drv.refine(stage, "cvrp", env.depot_node_xy, solutions, rewards, aug_factor, iterations,
-                                              False, env.depot_node_demand, capacity)
+                                              False, env.depot_node_demand, capacity, local_search_max_segment)
             total[0] += cost.mean()
             total[1] += seconds
             total[2] += int(moves.sum())
@@ -95,4 +97,5 @@ if __name__ == "__main__":
                for i in range(0, len(data), bs)]
     test(batches, model, env, aug_factor=config['params']['aug_factor'],
          two_opt_iterations=config['params'].get('two_opt_iterations') or 0,
-         local_search_iterations=config['params'].get('local_search_iterations') or 0, capacity=data[0][3])
+         local_search_iterations=config['params'].get('local_search_iterations') or 0, capacity=data[0][3],
+         local_search_max_segment=config['params'].get('local_search_max_segment') or 1)

@@ -93,9 +93,10 @@ def _dropin(name, points, tour, device, search):
     return refined.to(t.device, t.dtype), n_iter
 
 
-def cvrp_local_search(points, demand, capacity, tour, max_iterations=1000, device=None):
-    """Capacity-aware CVRP local search on the GPU (elg_cvrp_local_search): 2-opt inside a route, relocate, swap and
-    2-opt* between routes, best improvement, every tour stopping on its own.
+def cvrp_local_search(points, demand, capacity, tour, max_iterations=1000, device=None, max_segment=1):
+    """Capacity-aware CVRP local search on the GPU (elg_cvrp_local_search_ex): 2-opt inside a route, relocate, swap and
+    2-opt* between routes, and with max_segment 2 or 3 Or-opt moves of chains of up to that many customers, best
+    improvement, every tour stopping on its own.
 
     points (N+1, 2) with the depot at row 0; demand (N+1,) normalised by the capacity as the environments hold it (depot
     0); capacity the integer vehicle capacity; tour (batch, T) rollout rows (depot visits as 0, every customer once, every
@@ -103,7 +104,8 @@ def cvrp_local_search(points, demand, capacity, tour, max_iterations=1000, devic
     in order, each preceded by one 0, zero padding to T).  Returns (tour, iterations), iterations being the largest number
     of moves any tour took.  device=None is the current CUDA device; there is no CPU path."""
     return _dropin("cvrp_local_search", points, tour, device, lambda xy, t: engine.cvrp_local_search(
-        xy, t, torch.as_tensor(demand).to(xy.device, torch.float32)[None], capacity, max_iterations=max_iterations))
+        xy, t, torch.as_tensor(demand).to(xy.device, torch.float32)[None], capacity, max_iterations=max_iterations,
+        max_segment=max_segment))
 
 
 def augment_xy_data_by_8_fold(problems):

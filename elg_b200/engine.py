@@ -394,16 +394,20 @@ def tsp_local_search(xy, tours, inst=None, max_iterations=1000, max_segment=3, r
         stream))
 
 
-def cvrp_local_search(xy, tours, demand, capacity, inst=None, max_iterations=1000, rounding=False):
-    """Capacity-aware best-improvement CVRP local search (elg_cvrp_local_search; semantics in include/elg_b200.h): 2-opt
-    inside a route, relocate, swap and 2-opt* between routes, one launch for all rows.
+def cvrp_local_search(xy, tours, demand, capacity, inst=None, max_iterations=1000, rounding=False, max_segment=1):
+    """Capacity-aware best-improvement CVRP local search (elg_cvrp_local_search_ex; semantics in include/elg_b200.h):
+    2-opt inside a route, relocate, swap and 2-opt* between routes, and with max_segment 2 or 3 Or-opt moves of chains of
+    up to that many customers within and between routes, one launch for all rows.
 
     xy (Bxy, N1, 2) coordinates; tours (R, L) rollout rows, int16 or int64, with every customer exactly once, position 0
     the depot and every route within capacity; demand (Bxy, N1) normalised demands as CVRPEnv holds them (depot 0);
     capacity the integer vehicle capacity: demands in units are rint(demand * capacity) and must lie within 1e-3 of it.
     inst (R,) picks the xy / demand instance of every row (default: row r uses instance r, or 0 when Bxy == 1); rounding
-    rint()s every edge (library metric).  Returns (canonical tours int64 (R, L), length (R,) as tour_length measures it,
-    iterations (R,) moves applied)."""
+    rint()s every edge (library metric); max_segment (1..3) the longest Or-opt chain, 1 being relocate of one customer
+    only.  Returns (canonical tours int64 (R, L), length (R,) as tour_length measures it, iterations (R,) moves
+    applied)."""
+    if max_segment not in (1, 2, 3):
+        raise ValueError("max_segment must be 1, 2 or 3 (got %r)" % (max_segment,))
     s = _LocalSearch(xy, tours, inst, max_iterations, whole_row=True)
     R, L, N1 = s.R, s.L, s.N1
     if demand.shape != xy.shape[:2]:
@@ -428,9 +432,9 @@ def cvrp_local_search(xy, tours, demand, capacity, inst=None, max_iterations=100
                                                                                          s.per_row(units).gather(1, t).long())
         if int(loads.max()) > capacity:
             raise ValueError("an input route exceeds the capacity %d" % capacity)
-    return s.run(lambda xy_p, inst_p, t_p, it_p, len_p, stream: lib.elg_cvrp_local_search(
-        xy_p, s.Bxy, N1, _ptr(units), capacity, inst_p, t_p, R, L, 1 if rounding else 0, int(max_iterations), it_p,
-        len_p, stream), demand=units)
+    return s.run(lambda xy_p, inst_p, t_p, it_p, len_p, stream: lib.elg_cvrp_local_search_ex(
+        xy_p, s.Bxy, N1, _ptr(units), capacity, inst_p, t_p, R, L, int(max_segment), 1 if rounding else 0,
+        int(max_iterations), it_p, len_p, stream), demand=units)
 
 
 # ---------------------------------------------------------------------------------------------- training path

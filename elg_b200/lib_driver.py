@@ -8,7 +8,8 @@ TSP/test_tsplib.py:18-168) but are thin shells around the functions here:
 
 Optional refinement stages (STAGES; a config key absent or 0: nothing changes): 2-opt (params.two_opt_iterations, both
 problems), the capacity-aware CVRP local search (params.local_search_iterations, with the capacity
-CVRPEnv.load_vrplib_problem recorded) and the TSP 2-opt + Or-opt local search (params.tsp_local_search_iterations).
+CVRPEnv.load_vrplib_problem recorded, and its longest Or-opt chain params.local_search_max_segment, 1..3, default 1) and
+the TSP 2-opt + Or-opt local search (params.tsp_local_search_iterations).
 load_model records the settings on the model and rejects a key the problem does not accept; solve_instance then refines
 the best POMO row of every aug-instance with every enabled stage, independently and in the library metric (rounded
 unscaled coordinates), and returns the cost as an InstanceCost carrying each stage's result; fill_record adds the
@@ -47,6 +48,7 @@ def load_model(model_cls, config, device, model=None, needs_local=True):
     model.eval()
     model.requires_grad_(False)
     model._elg_stage_iterations = {stage.key: config.get('params', {}).get(stage.key) or 0 for stage in STAGES}
+    model._elg_local_search_max_segment = config.get('params', {}).get('local_search_max_segment') or 1
     return model
 
 
@@ -58,19 +60,21 @@ class InstanceCost(float):
     tsp_local_search = None
 
 
-def _cvrp_local_search(problem, xy, rows, demand, capacity, iterations, rounding):
+def _cvrp_local_search(problem, xy, rows, demand, capacity, iterations, rounding, max_segment):
     if capacity is None:
         raise ValueError("the local search stage needs the instance's capacity (CVRPEnv.load_vrplib_problem)")
-    return engine.cvrp_local_search(xy, rows, demand, capacity, max_iterations=iterations, rounding=rounding)
+    return engine.cvrp_local_search(xy, rows, demand, capacity, max_iterations=iterations, rounding=rounding,
+                                    max_segment=max_segment)
 
 
 # An optional refinement stage: config key (under params), problems that accept it, InstanceCost attribute, record key
 # suffix and prefix, name in the printouts, rejection message for the other problem, and the engine call
-# run(problem, xy, rows, demand, capacity, iterations, rounding) -> (tours, length, moves).
+# run(problem, xy, rows, demand, capacity, iterations, rounding, max_segment) -> (tours, length, moves); max_segment
+# (params.local_search_max_segment) only concerns the CVRP local search.
 Stage = namedtuple('Stage', 'key problems attr suffix prefix label rejection run')
 STAGES = (
     Stage('two_opt_iterations', ('tsp', 'cvrp'), 'two_opt', '2opt', 'two_opt', '2-opt', None,
-          lambda problem, xy, rows, demand, capacity, iterations, rounding:
+          lambda problem, xy, rows, demand, capacity, iterations, rounding, max_segment:
           engine.two_opt(problem, xy, rows, max_iterations=iterations, rounding=rounding)),
     Stage('local_search_iterations', ('cvrp',), 'local_search', 'ls', 'ls', 'local search',
           "params.local_search_iterations is the capacity-aware CVRP local search; "
@@ -78,16 +82,28 @@ STAGES = (
     Stage('tsp_local_search_iterations', ('tsp',), 'tsp_local_search', 'tsp_ls', 'tsp_ls', '2-opt + or-opt',
           "params.tsp_local_search_iterations is the TSP 2-opt + Or-opt local search; "
           "refine CVRP rows with params.local_search_iterations",
-          lambda problem, xy, rows, demand, capacity, iterations, rounding:
+          lambda problem, xy, rows, demand, capacity, iterations, rounding, max_segment:
           engine.tsp_local_search(xy, rows, max_iterations=iterations, rounding=rounding)),
 )
 
 
 def reject(problem, config):
-    """Raises ValueError for a stage key in config['params'] that the problem ('tsp' / 'cvrp') does not accept."""
+    """Raises ValueError for a stage key in config['params'] that the problem ('tsp' / 'cvrp') does not accept, and for
+    a params.local_search_max_segment that is not 1..3 or has no CVRP local search stage to feed."""
+    params = config.get('params', {})
     for stage in STAGES:
-        if problem not in stage.problems and config.get('params', {}).get(stage.key):
+        if problem not in stage.problems and params.get(stage.key):
             raise ValueError(stage.rejection)
+    max_segment = params.get('local_search_max_segment')
+    if max_segment is None:
+        return
+    if problem != 'cvrp':
+        raise ValueError("params.local_search_max_segment is the longest Or-opt chain of the CVRP local search; the TSP "
+                         "local search (params.tsp_local_search_iterations) always moves chains of up to 3 nodes")
+    if max_segment not in (1, 2, 3):
+        raise ValueError("params.local_search_max_segment must be 1, 2 or 3 (got %r)" % (max_segment,))
+    if not params.get('local_search_iterations'):
+        raise ValueError("params.local_search_max_segment needs the local search stage: set params.local_search_iterations")
 
 
 def enabled_stages(iterations):
@@ -95,16 +111,17 @@ def enabled_stages(iterations):
     return [(stage, iterations[stage.key]) for stage in STAGES if iterations.get(stage.key)]
 
 
-def refine(stage, problem, xy, solutions, rewards, aug_factor, iterations, rounding, demand=None, capacity=None):
+def refine(stage, problem, xy, solutions, rewards, aug_factor, iterations, rounding, demand=None, capacity=None,
+           max_segment=1):
     """One stage (one launch) on the best POMO row of every aug-instance of a greedy rollout.  xy (aug*n or 1, N1, 2) is
     the metric the cost is measured in: library runs pass the unscaled coordinates with rounding, random instances the
-    scaled ones without; the CVRP local search also takes demand (aug*n, N1), normalised as the environment holds it, and
-    the integer capacity.  -> (refined cost per instance, best over its augmentations (n,); seconds; moves applied per
+    scaled ones without; the CVRP local search also takes demand (aug*n, N1), normalised as the environment holds it, the
+    integer capacity and its longest Or-opt chain max_segment.  -> (refined cost per instance, best over its augmentations (n,); seconds; moves applied per
     instance, summed over its augmentations (n,))"""
     rows = solutions[torch.arange(rewards.shape[0], device=solutions.device), rewards.argmax(dim=1)]
     torch.cuda.synchronize()
     t0 = time.time()
-    _, length, iters = stage.run(problem, xy, rows, demand, capacity, iterations, rounding)
+    _, length, iters = stage.run(problem, xy, rows, demand, capacity, iterations, rounding, max_segment)
     torch.cuda.synchronize()
     seconds = time.time() - t0
     B = length.shape[0]
@@ -124,7 +141,8 @@ def solve_instance(model, env, rollout, aug_factor, width):
     for stage, iterations in enabled_stages(getattr(model, '_elg_stage_iterations', {})):
         if cvrp:
             refined, seconds, moves = refine(stage, 'cvrp', env.unscaled_depot_node_xy, solutions, rewards, aug_factor,
-                                             iterations, True, env.depot_node_demand, env.capacity)
+                                             iterations, True, env.depot_node_demand, env.capacity,
+                                             getattr(model, '_elg_local_search_max_segment', 1))
         else:
             refined, seconds, moves = refine(stage, 'tsp', env._unscaled_dev, solutions, rewards, aug_factor, iterations,
                                              True)

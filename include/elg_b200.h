@@ -30,7 +30,8 @@ extern "C" {
 #endif
 
 #define ELG_ABI_VERSION 4   /* 2: training path, data generators; 3: elg_tables.et / .ws (streamed tensor-core decode);
-                               4: elg_two_opt, then elg_cvrp_local_search, then elg_tsp_local_search (purely additive,
+                               4: elg_two_opt, then elg_cvrp_local_search, then elg_tsp_local_search, then
+                                  elg_cvrp_local_search_ex (purely additive,
                                   so the version stays 4: a library without one fails on the missing symbol when the
                                   binding loads) */
 
@@ -277,18 +278,32 @@ int elg_tsp_local_search(const float* xy, int Bxy, int N1, const int32_t* inst, 
  *   tours [R][L]      int16 rollout rows: position 0 the depot, every customer 1..N1-1 exactly once, depot visits as 0,
  *                     trailing zero padding, L <= 2*N1+2.  The output row is canonical even without a move: routes in
  *                     their order, each preceded by one 0, no empty route, zero padding to L.
- * A route is a maximal run of customers.  Positions refer to the current canonical row, P = 1 + last customer position:
+ *   max_segment       1, 2 or 3: the longest chain of customers an Or-opt move (types 4..7) carries; 1 evaluates
+ *                     types 0..3 only.  Any other value is ELG_EINVAL.
+ * A route is a maximal run of customers.  Positions refer to the current canonical row, P = 1 + last customer position,
+ * e_p = d(t_p, t_p+1) with t_P = 0:
  *   type 0, 2-opt inside a route: reverse positions i+1..j (j >= i+2), all customers of one route.
  *   type 1, relocate: move the customer at i onto the edge (t_j, t_j+1), j < P, j not i-1 or i; feasible within its
  *           route, or if the target route's load + its demand <= capacity.  A route emptied by the move disappears.
  *   type 2, swap: exchange the customers at i < j of two different routes; both new loads <= capacity.
  *   type 3, 2-opt*: cut positions i < j (a route's depot position or a customer) of different routes A and B;
  *           A' = A[..i] + B(j..] takes A's slot, B' = B[..j] + A(i..] takes B's; both loads <= capacity; an empty
- *           result disappears, so two routes can merge.  No move opens a route.
- * Gains are added minus removed edges of d (the reward's seglen, rint()-ed when round_edges is set).  Every iteration
- * evaluates every admissible move and applies the smallest gain, ties to the lowest type*L^2 + i*L + j, if it is below
- * -1e-6, at most max_iterations times.  length is the closed length of the returned row as elg_tour_length sums it.
- * N1 <= 8192 (shared memory: 12*N1 + 8*L bytes). */
+ *           result disappears, so two routes can merge.
+ *   types 4 / 5 (s = 2) and 6 / 7 (s = 3), Or-opt: move the segment at positions i..i+s-1, all customers (so one route),
+ *           onto the edge (t_j, t_j+1), forward / reversed; j < P, j not in i-1..i+s-1, s <= max_segment.  Feasible
+ *           within its route, or if the target route's load + the segment's load <= capacity.  Gain
+ *           ((d(t_i-1, t_i+s) - e_i-1) - e_i+s-1) + ((d(t_j, a) - e_j) + d(b, t_j+1)), fp32 in that order, with
+ *           (a, b) = (t_i, t_i+s-1) forward and (t_i+s-1, t_i) reversed.  A segment that is its whole route empties it
+ *           and the route disappears.
+ * No move opens a route.  Gains of types 0..3 are added minus removed edges of d (the reward's seglen, rint()-ed when
+ * round_edges is set).  Every iteration evaluates every admissible move and applies the smallest gain, ties to the
+ * lowest type*L^2 + i*L + j (unsigned: up to 8*L^2 - 1), if it is below -1e-6, at most max_iterations times.  length is
+ * the closed length of the returned row as elg_tour_length sums it.  N1 <= 8192 (shared memory: 12*N1 + 8*L bytes). */
+int elg_cvrp_local_search_ex(const float* xy, int Bxy, int N1, const int32_t* demand, int32_t capacity,
+                             const int32_t* inst, int16_t* tours, int R, int L, int max_segment, int round_edges,
+                             int max_iterations, int32_t* iterations, float* length, void* stream);
+
+/* elg_cvrp_local_search_ex with max_segment = 1 (types 0..3). */
 int elg_cvrp_local_search(const float* xy, int Bxy, int N1, const int32_t* demand, int32_t capacity, const int32_t* inst,
                           int16_t* tours, int R, int L, int round_edges, int max_iterations, int32_t* iterations,
                           float* length, void* stream);

@@ -6,9 +6,10 @@ ABI between two events, after a warm-up call of the same search (2-opt: the same
       TSP100 / CVRP100, the best POMO row of each of 8000 aug-instances (1000 instances x 8), scaled metric; synthetic
       TSP with N = 1000, 4000, 7000 (one instance x 8 augmentations), scaled metric; all 49 TSPLIB and 51 Set-X
       instances of tests/golden/lib, the drivers' greedy tours, rounded unscaled metric.
-  --search cvrp_ls  (elg_cvrp_local_search -> profiles/r04_cvrp_local_search):
+  --search cvrp_ls  (elg_cvrp_local_search_ex, --max-segment 1 -> profiles/r04_cvrp_local_search):
       CVRP100 x 8000 and CVRP1000 x 8 rows, scaled metric; all 51 Set-X instances, rounded unscaled metric, with the gap
-      after 2-opt on the same rows beside it.
+      after 2-opt on the same rows beside it.  With --max-segment 2 or 3 (Or-opt chains of up to that many customers ->
+      profiles/r07_cvrp_or_opt) the same cases, each also run with max_segment 1 on the same rows.
   --search tsp_ls   (elg_tsp_local_search, max_segment 3, with elg_two_opt timed on the same tours beside it
                      -> profiles/r05_tsp_local_search):
       TSP100 x 8000, TSP1000 x 8 and TSP4000 x 8 tours, scaled metric; all 49 TSPLIB instances, rounded unscaled metric.
@@ -18,7 +19,7 @@ moves applied, us per move (call time over the largest per-tour move count: tour
 pair evaluations per second (pairs the kernel sweeps, counted on the host; see each markdown header), cost or gap
 before and after.  --quick runs small sizes only (a rehearsal).
 
-    python tools/local_search_timing.py --search {two_opt,cvrp_ls,tsp_ls} [--quick] [--out PREFIX]"""
+    python tools/local_search_timing.py --search {two_opt,cvrp_ls,tsp_ls} [--max-segment {1,2,3}] [--quick] [--out PREFIX]"""
 import argparse
 import ctypes as C
 import json
@@ -40,14 +41,16 @@ MAX_SEGMENT = 3
 OUT = {"two_opt": "r03_two_opt", "cvrp_ls": "r04_cvrp_local_search", "tsp_ls": "r05_tsp_local_search"}
 
 
-def timed(kernel, xy, rows, max_iterations, rounding, warmup_iterations, dem=None, cap=None):
-    """kernel 'tsp' / 'cvrp' (elg_two_opt), 'tsp_ls' or 'cvrp_ls' -> (ms of the timed launch, tours, length, iterations)"""
+def timed(kernel, xy, rows, max_iterations, rounding, warmup_iterations, dem=None, cap=None, max_segment=1):
+    """kernel 'tsp' / 'cvrp' (elg_two_opt), 'tsp_ls' or 'cvrp_ls' (max_segment) -> (ms of the timed launch, tours,
+    length, iterations)"""
     from elg_b200 import engine
     from elg_b200._lib import ELG_CVRP, ELG_TSP, check, lib
     if kernel == "tsp_ls":                              # warm-up, argument checks
         engine.tsp_local_search(xy, rows, max_iterations=warmup_iterations, max_segment=MAX_SEGMENT, rounding=rounding)
     elif kernel == "cvrp_ls":
-        engine.cvrp_local_search(xy, rows, dem, cap, max_iterations=warmup_iterations, rounding=rounding)
+        engine.cvrp_local_search(xy, rows, dem, cap, max_iterations=warmup_iterations, rounding=rounding,
+                                 max_segment=max_segment)
     else:
         engine.two_opt(kernel, xy, rows, max_iterations=warmup_iterations, rounding=rounding)
     R, L = rows.shape
@@ -67,8 +70,8 @@ def timed(kernel, xy, rows, max_iterations, rounding, warmup_iterations, dem=Non
         check(lib.elg_tsp_local_search(p(xy), B, N1, null, p(t16), R, L, MAX_SEGMENT, int(rounding), max_iterations,
                                        p(iters), p(length), s))
     elif kernel == "cvrp_ls":
-        check(lib.elg_cvrp_local_search(p(xy), B, N1, p(units), int(cap), null, p(t16), R, L, int(rounding),
-                                        max_iterations, p(iters), p(length), s))
+        check(lib.elg_cvrp_local_search_ex(p(xy), B, N1, p(units), int(cap), null, p(t16), R, L, max_segment,
+                                           int(rounding), max_iterations, p(iters), p(length), s))
     else:
         check(lib.elg_two_opt(ELG_CVRP if kernel == "cvrp" else ELG_TSP, p(xy), B, N1, null, p(t16), R, L, int(rounding),
                               max_iterations, p(iters), p(length), s))
@@ -224,9 +227,9 @@ def two_opt_markdown(device, power, cases, library):
 # ------------------------------------------------------------------------------------------------ cvrp_ls
 
 
-def cvrp_ls_summary(case, xy, rows, dem, cap, rounding, before, opt=None):
+def cvrp_ls_summary(case, xy, rows, dem, cap, rounding, before, opt=None, max_segment=1):
     from elg_b200 import engine
-    ms, out, length, iters = timed("cvrp_ls", xy, rows, MAX_IT, rounding, 1, dem, cap)
+    ms, out, length, iters = timed("cvrp_ls", xy, rows, MAX_IT, rounding, 1, dem, cap, max_segment)
     it = iters.cpu().numpy()
     pos = torch.arange(out.shape[1], device=out.device)
     P = (torch.where(out != 0, pos, 0).max(1)[0] + 1).cpu().numpy()      # used positions: up to the last customer
@@ -241,22 +244,72 @@ def cvrp_ls_summary(case, xy, rows, dem, cap, rounding, before, opt=None):
     if opt is not None:
         row["gap_before"] = float(((inst_before - opt) / opt).mean())
         row["gap_after"] = float(((inst_after - opt) / opt).mean())
-        two = engine.two_opt("cvrp", xy, rows, max_iterations=MAX_IT, rounding=rounding)[1]
-        row["gap_after_2opt"] = float(((per_instance(two) - opt) / opt).mean())
+        if max_segment == 1:
+            two = engine.two_opt("cvrp", xy, rows, max_iterations=MAX_IT, rounding=rounding)[1]
+            row["gap_after_2opt"] = float(((per_instance(two) - opt) / opt).mean())
+    if max_segment > 1:
+        row["max_segment"] = max_segment
     return row
 
 
-def cvrp_ls_run(quick):
+def cvrp_ls_run(quick, max_segment=1):
+    """max_segment 1: the r04 cases.  Above 1: each case with max_segment and with 1 on the same rows, as a pair
+    {"case", "or_opt": summary, "relocate": summary}."""
+    def run(case, xy, rows, dem, cap, rounding, before, opt=None):
+        if max_segment == 1:
+            return cvrp_ls_summary(case, xy, rows, dem, cap, rounding, before, opt)
+        return {"case": case, "or_opt": cvrp_ls_summary(case, xy, rows, dem, cap, rounding, before, opt, max_segment),
+                "relocate": cvrp_ls_summary(case, xy, rows, dem, cap, rounding, before, opt, 1)}
     cases = []
     for N, n, cap in ([(100, 16, 50), (1000, 1, 250)] if quick else [(100, 1000, 50), (1000, 1, 250)]):
         xy, dem, rows, before = random_rows("cvrp", N, n, min(N, 100), seed=N, capacity=float(cap))
-        cases.append(cvrp_ls_summary("CVRP%d x %d" % (N, 8 * n), xy, rows, dem, cap, False, before))
+        cases.append(run("CVRP%d x %d" % (N, 8 * n), xy, rows, dem, cap, False, before))
         print(json.dumps(cases[-1]), flush=True)
     setx = []
     for name, xy, dem, cap, rows, before, opt in library_rows("setx", ["X-n101-k25", "X-n200-k36"] if quick else None):
-        setx.append(cvrp_ls_summary(name, xy, rows, dem, cap, True, before, opt=opt))
+        setx.append(run(name, xy, rows, dem, cap, True, before, opt=opt))
         print(json.dumps(setx[-1]), flush=True)
     return {"cases": cases, "setx": setx}
+
+
+def cvrp_or_opt_markdown(device, power, cases, setx):
+    seg = (cases or setx)[0]["or_opt"]["max_segment"]
+    out = ["# Or-opt in the CVRP local search on the GPU (`elg_cvrp_local_search_ex`, max_segment %d)" % seg, "",
+           "Measured on %s, power limit %s, with `tools/local_search_timing.py --search cvrp_ls --max-segment %d` (CUDA "
+           "events around one launch after a one-move warm-up launch).  Rows are the greedy rollouts of the seeded "
+           "synthetic checkpoint (gain 3), best POMO row of every aug-instance, the cases of `r04`.  Every case runs "
+           "max_segment %d (Or-opt chains of up to %d customers) and max_segment 1 (relocate of one customer only, the "
+           "search of `r04`) on the same rows.  max_iterations is %d.  `us/move` is the call time over the largest "
+           "per-row move count.  Cost is the best over the 8 augmentations, averaged over instances; routes are averaged "
+           "over rows." % (device, power, seg, seg, seg, MAX_IT), "",
+           "| case | max_segment | rows | N1 | ms / call | moves (sum) | max moves / row | rows at the cap | us / move | routes before | routes after | cost before | cost after |",
+           "|---|---|---|---|---|---|---|---|---|---|---|---|---|"]
+    for pair in cases:
+        for c, s in ((pair["relocate"], 1), (pair["or_opt"], seg)):
+            out.append("| %s | %d | %d | %d | %.2f | %d | %d | %d | %.1f | %.1f | %.1f | %.4f | %.4f |" % (
+                pair["case"], s, c["rows"], c["N1"], c["ms"], c["moves"], c["max_moves"], c["capped"], c["us_per_move"],
+                c["routes_before"], c["routes_after"], c["cost_before"], c["cost_after"]))
+    if setx:
+        mean = lambda k, key: 100 * np.mean([r[k][key] for r in setx])
+        above = [r["case"] for r in setx if r["or_opt"]["gap_after"] > r["relocate"]["gap_after"]]
+        out += ["", "## Set-X: %d instances, rounded unscaled metric" % len(setx), "",
+                "Total kernel time %.1f ms with max_segment %d (%d moves), %.1f ms with max_segment 1 (%d moves).  Mean gap "
+                "%.2f %% before, %.2f %% after max_segment 1, %.2f %% after max_segment %d.  max_segment %d ends below "
+                "max_segment 1 on %d instances, equal on %d, above on %d%s." % (
+                    sum(r["or_opt"]["ms"] for r in setx), seg, sum(r["or_opt"]["moves"] for r in setx),
+                    sum(r["relocate"]["ms"] for r in setx), sum(r["relocate"]["moves"] for r in setx),
+                    mean("or_opt", "gap_before"), mean("relocate", "gap_after"), mean("or_opt", "gap_after"), seg, seg,
+                    sum(r["or_opt"]["gap_after"] < r["relocate"]["gap_after"] for r in setx),
+                    sum(r["or_opt"]["gap_after"] == r["relocate"]["gap_after"] for r in setx), len(above),
+                    (" (%s)" % ", ".join(above)) if above else ""), "",
+                "| instance | N1 | ms max_segment 1 | ms max_segment %d | moves 1 (8 rows) | moves %d | us / move 1 | us / move %d | routes after 1 | routes after %d | gap before | gap after 1 | gap after %d |" % (seg, seg, seg, seg, seg),
+                "|---|---|---|---|---|---|---|---|---|---|---|---|---|"]
+        for r in setx:
+            a, b = r["relocate"], r["or_opt"]
+            out.append("| %s | %d | %.2f | %.2f | %d | %d | %.1f | %.1f | %.1f | %.1f | %.2f %% | %.2f %% | %.2f %% |" % (
+                r["case"], a["N1"], a["ms"], b["ms"], a["moves"], b["moves"], a["us_per_move"], b["us_per_move"],
+                a["routes_after"], b["routes_after"], 100 * a["gap_before"], 100 * a["gap_after"], 100 * b["gap_after"]))
+    return out
 
 
 def cvrp_ls_markdown(device, power, cases, setx):
@@ -374,9 +427,14 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--search", required=True, choices=sorted(SEARCHES))
     ap.add_argument("--out", help="output prefix for .md / .json (default: profiles/ r03 / r04 / r05 of the search)")
+    ap.add_argument("--max-segment", type=int, choices=(1, 2, 3), default=1,
+                    help="cvrp_ls: longest Or-opt chain; above 1 also runs 1 on the same rows (profiles/r07_cvrp_or_opt)")
     ap.add_argument("--quick", action="store_true", help="small sizes only (rehearsal)")
     args = ap.parse_args()
-    out_prefix = args.out or os.path.join(ROOT, "profiles", OUT[args.search])
+    if args.max_segment > 1 and args.search != "cvrp_ls":
+        ap.error("--max-segment is an option of --search cvrp_ls")
+    or_opt = args.max_segment > 1
+    out_prefix = args.out or os.path.join(ROOT, "profiles", "r07_cvrp_or_opt" if or_opt else OUT[args.search])
     if not torch.cuda.is_available():
         raise SystemExit("no CUDA device: this measurement needs the GPU")
     device = torch.cuda.get_device_name(0)
@@ -386,7 +444,10 @@ def main():
     except OSError:
         power = "not reported"
     run, markdown = SEARCHES[args.search]
-    result = run(args.quick)
+    if or_opt:
+        result, markdown = cvrp_ls_run(args.quick, args.max_segment), cvrp_or_opt_markdown
+    else:
+        result = run(args.quick)
     md = "\n".join(markdown(device, power, *result.values())) + "\n"
     os.makedirs(os.path.dirname(os.path.abspath(out_prefix)), exist_ok=True)
     with open(out_prefix + ".md", "w") as f:
