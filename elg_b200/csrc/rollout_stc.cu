@@ -13,24 +13,22 @@
 //
 // CTA = one (aug-instance, tile of 128 POMO rows); TMEM lane = row; 16 warps as in rollout_tc.cu (lane quadrant q =
 // warp % 4, sub-slot wsub = warp / 4; two softmax groups of 8 warps with their own S/P buffer and mbarrier).
-// The local policy (CVRP/models.py:51-175) is the TMEM-lane formulation of rollout_tc.cu with both contractions on
-// tcgen05; its neighbourhood comes from the uint16 rank-ordered neighbour lists, tested 128 entries at a time until k
-// valid ones are found, and its features (distance, polar angle, demand / load) are computed in the kernel.  The ~k
+// The local policy (CVRP/models.py:51-175) is rollout_tc.cu's, steps (3)-(6) shared through rollout_common.cuh (12
+// sequence positions per thread); its neighbourhood comes from the uint16 rank-ordered neighbour lists, tested 128
+// entries at a time until k valid ones are found, and its features (distance, polar angle, demand / load) are computed
+// in the kernel.  The ~k
 // neighbour nodes of a row get their exact logit per tile: the scores of flagged nodes are parked in an on-chip
 // [128 rows][128 nodes] scratch (the second 64 KB buffer), left out of the running arg-max, and compared with their
 // penalty + local score by the threads that own the local sequence.
 // Per-row bit masks (masked / visited / neighbour, one 32-bit word per 32 nodes) live in global scratch (L2-resident).
 //
-// TMEM columns: [0,128) Q hi|lo, later O hi|lo   [128,256) O accumulators (8 heads x 16)
-//               [256,384) / [384,512) S / P buffers of the two groups, later the two score-tile accumulators
-//   during the local policy (before the first Q K^T): as in rollout_tc.cu
+// TMEM columns: the plan in rollout_common.cuh, with S / P buffers [256,384) / [384,512) of the two groups, later the two
+// score-tile accumulators
 #include "rollout_common.cuh"
 
 namespace elg {
 
 constexpr int SKT = 48, SPT = 12;             // local sequence slots (k + depot <= 48), slots per thread
-constexpr uint32_t SC_Q = 0, SC_O = 128, SC_S = 256, SC_PX = 128, SC_D2 = 128, SC_A2 = 192, SC_A1 = 256, SC_D1 = 448;
-constexpr float SC_P_SCALE_LOG2 = 10.f;
 
 struct StcL {      // shared-memory layout in floats (compile-time)
   static constexpr int buf = 0;                                  // 2 x 64 KB: K' | V^T tile, later two E' tiles
@@ -61,26 +59,7 @@ struct StcL {      // shared-memory layout in floats (compile-time)
 };
 static_assert(StcL::total * 4 <= 227 * 1024, "layout exceeds one SM's shared memory");
 
-__device__ __forceinline__ uint32_t pick4s(const uint32_t (&w)[4], int i) {
-  return i == 0 ? w[0] : (i == 1 ? w[1] : (i == 2 ? w[2] : w[3]));
-}
-__device__ __forceinline__ void pair_sync_s(int id) { asm volatile("bar.sync %0, 64;" ::"r"(id) : "memory"); }
-__device__ __forceinline__ void group_sync_s(int id) { asm volatile("bar.sync %0, 256;" ::"r"(id) : "memory"); }
-__device__ __forceinline__ void quad_sync_s(int id) { asm volatile("bar.sync %0, 128;" ::"r"(id) : "memory"); }
 __device__ __forceinline__ float scr_at(const float* sSc, int row, int jl, int lane) { return sSc[row * 128 + (jl ^ lane)]; }
-__device__ __forceinline__ int select128s(const uint32_t (&r)[4], int n) {
-  const int c0 = __popc(r[0]), c1 = c0 + __popc(r[1]), c2 = c1 + __popc(r[2]);
-  const int w = (n >= c0 ? 1 : 0) + (n >= c1 ? 1 : 0) + (n >= c2 ? 1 : 0);
-  int m = n - (w == 0 ? 0 : (w == 1 ? c0 : (w == 2 ? c1 : c2)));
-  uint32_t x = pick4s(r, w);
-  int pos = 0, t;
-  t = __popc(x & 0xffffu); if (m >= t) { m -= t; pos = 16; x >>= 16; }
-  t = __popc(x & 0xffu);   if (m >= t) { m -= t; pos += 8; x >>= 8; }
-  t = __popc(x & 0xfu);    if (m >= t) { m -= t; pos += 4; x >>= 4; }
-  t = __popc(x & 0x3u);    if (m >= t) { m -= t; pos += 2; x >>= 2; }
-  t = (int)(x & 1u);       if (m >= t) pos += 1;
-  return w * 32 + pos;
-}
 
 // =================================================================================================
 template <int PROBLEM>
@@ -92,7 +71,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
   const int N1 = A.N1;
   const int NT = stc_tiles(N1);
   const int K1 = A.k_local + DEP;
-  const int N2 = (K1 + 4 + 15) & ~15;
+  const int N2 = tc_n2(K1);
   const float* sWL = sm + L::wl;
   const float* sU = sm + L::u;
   const float* sT = sm + L::tt;
@@ -129,19 +108,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
   uint8_t* wsb = reinterpret_cast<uint8_t*>(A.t.ws);
 
   {
-    const float* loc = A.derived + DER_LOC;
-    float* w = sm;
-    for (int i = tid; i < E; i += RT) w[L::wl + i] = A.derived[DER_WL + i];
-    for (int i = tid; i < LH * 4; i += RT) w[L::u + i] = loc[LOC_U + i];
-    for (int i = tid; i < LH * KT_MAX; i += RT) w[L::tt + i] = loc[LOC_T + i];
-    for (int i = tid; i < LE * 4; i += RT) w[L::a + i] = (i & 3) == 3 ? loc[LOC_CV + (i >> 2)] : loc[LOC_A + i];
-    for (int i = tid; i < KT_MAX; i += RT) w[L::pb + i] = loc[LOC_PB + i];
-    for (int i = tid; i < 4; i += RT) w[L::zb + i] = loc[LOC_ZB + i];
-    for (int i = tid; i < LH * SKT * 16; i += RT) {
-      const int h = i / (SKT * 16), r = i % (SKT * 16), part = r / (SKT * 8), x = r % (SKT * 8);
-      w[L::op1 + i] = loc[LOC_OP1 + h * (KT_MAX * 16) + part * (KT_MAX * 8) + x];
-    }
-    for (int i = tid; i < N2 * LE; i += RT) w[L::op2 + i] = loc[LOC_OP2 + i];
+    stage_local_consts<L, SKT>(sm, A.derived, N2, tid);
     if (tid == 0) {
       for (int i = 0; i < 9; ++i) mbar_init(bar_kv + i, 1);
       sCtrl[1] = 0;
@@ -241,8 +208,8 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
 #pragma unroll
             for (int i = 0; i < 16; ++i) hw[i] = lw[i] = 0u;
           }
-          umma::st16s<1>(tl + SC_Q + 16 * wsub, hw);
-          umma::st16s<1>(tl + SC_Q + 64 + 16 * wsub, lw);
+          umma::st16s<1>(tl + TC_COL_Q + 16 * wsub, hw);
+          umma::st16s<1>(tl + TC_COL_Q + 64 + 16 * wsub, lw);
         }
         PHASE_MARK(0);
 
@@ -281,16 +248,16 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
           }
           uint32_t* xr = reinterpret_cast<uint32_t*>(sX4);                 // [4][128] words
           xr[wsub * 128 + row] = rp;
-          quad_sync_s(11 + q);
+          quad_sync(11 + q);
           const uint32_t R[4] = {xr[row], xr[128 + row], xr[256 + row], xr[384 + row]};
           const int cc = __popc(R[0]) + __popc(R[1]) + __popc(R[2]) + __popc(R[3]);
           if (want && cc > 0) {
             const int take = min(cc, kloc - c0);
-            elast = c * 128 + select128s(R, take - 1);
+            elast = c * 128 + select128(R, take - 1);
             // my ranks inside this chunk: [max(ps, c0), min(pe, c0 + cc))
             const int lo = max(ps, c0), hi = min(pe, c0 + cc);
             if (lo < hi) {
-              const int e1 = select128s(R, lo - c0);
+              const int e1 = select128(R, lo - c0);
               unsigned long long ra = ((unsigned long long)R[1] << 32) | R[0], rb = ((unsigned long long)R[3] << 32) | R[2];
               if (e1 < 64) { ra &= ~0ull << e1; } else { ra = 0ull; rb &= ~0ull << (e1 - 64); }
 #pragma unroll
@@ -315,9 +282,10 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
         PHASE_MARK(1);
         const int np = act ? kk + DEP : 0;
         // slot s of this thread is sequence position p0 + s; neighbour rank p0 + s - DEP (the depot heads the cvrp sequence)
-        float f0[SPT], f1[SPT], f2[SPT];
+        LocalSeq<SPT> ls;
+        ls.p0 = p0;
+        ls.cpen = 1.f;
         uint32_t idw[SPT / 2];
-        float cpen = 1.f;
         {
           const float xc = pXY[2 * cur0], yc = pXY[2 * cur0 + 1];
           float dmax = 0.f;
@@ -326,13 +294,13 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
             dmax = dist2(xc - pXY[2 * nl], yc - pXY[2 * nl + 1]);
           }
           const float r0d = CVRP ? (dmax != 0.f ? 1.f / (dmax + 1e-6f) : 1.f) : 1.f / (dmax + 1e-6f);
-          if (CVRP && dmax != 0.f) cpen = (dmax + 1e-6f) / dmax;       // penalty -d / dmax = -f0 (dmax + 1e-6) / dmax
+          if (CVRP && dmax != 0.f) ls.cpen = (dmax + 1e-6f) / dmax;       // penalty -d / dmax = -f0 (dmax + 1e-6) / dmax
           const float rld = 1.f / ld0;
 #pragma unroll
           for (int i = 0; i < SPT / 2; ++i) idw[i] = 0u;
 #pragma unroll
           for (int s = 0; s < SPT; ++s) {
-            f0[s] = f1[s] = f2[s] = 0.f;
+            ls.f0[s] = ls.f1[s] = ls.f2[s] = 0.f;
             const int p = p0 + s;
             // the rank of slot s among my ranks: slots of wsub 0 are shifted by the depot
             const int sr = (DEP && wsub == 0) ? s - 1 : s;
@@ -342,9 +310,9 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
               idw[s >> 1] |= (uint32_t)nd << ((s & 1) * 16);
               const float xn = pXY[2 * nd], yn = pXY[2 * nd + 1];
               const float dd = dist2(xc - xn, yc - yn);
-              f0[s] = dd * r0d;
-              f1[s] = atan2f(yn - yc, xn - xc);
-              if (CVRP) f2[s] = pDem[nd] * rld;
+              ls.f0[s] = dd * r0d;
+              ls.f1[s] = atan2f(yn - yc, xn - xc);
+              if (CVRP) ls.f2[s] = pDem[nd] * rld;
               atomicOr(gnb + (nd >> 5), 1u << (nd & 31));               // flagged: left out of the streamed arg-max
             }
           }
@@ -352,182 +320,60 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
         }
         const bool depot_masked = CVRP && act && (gmask[0] & 1u);
         PHASE_MARK(2);
-        const int nv = np - p0;
-        const bool dep_off = DEP && wsub == 0 && depot_masked;
-        auto load_head = [&](int h, float4& u, float (&tq)[SPT]) {
-          u = *reinterpret_cast<const float4*>(sU + h * 4);
-#pragma unroll
-          for (int i = 0; i < SPT / 4; ++i) {
-            const float4 t4 = *reinterpret_cast<const float4*>(sT + h * KT_MAX + p0 + 4 * i);
-            tq[4 * i] = t4.x; tq[4 * i + 1] = t4.y; tq[4 * i + 2] = t4.z; tq[4 * i + 3] = t4.w;
-          }
-          if (dep_off) tq[0] = -INFINITY;
-        };
-        auto lscore = [&](const float4& u, const float (&tq)[SPT], int s) -> float {
-          const float v = fmaf(u.z, f2[s], fmaf(u.y, f1[s], fmaf(u.x, f0[s], tq[s])));
-          return s < nv ? v : -INFINITY;
-        };
+        // (3) per-head maxima of the row: fp32, combined over the four quarters through shared memory
+        ls.nv = np - p0;
+        ls.dep_off = DEP && wsub == 0 && depot_masked;
         float mh[LH];
         {
-#pragma unroll
-          for (int h = 0; h < LH; ++h) {
-            float4 u;
-            float tq[SPT];
-            load_head(h, u, tq);
-            float m = -INFINITY;
-#pragma unroll
-            for (int s = 0; s < SPT; ++s) m = fmaxf(m, lscore(u, tq, s));
-            mh[h] = m;
-          }
+          lp_head_max(ls, sU, sT, mh);
           sX4[wsub * 128 + row] = make_float4(mh[0], mh[1], mh[2], mh[3]);
-          quad_sync_s(11 + q);
+          quad_sync(11 + q);
           const float4 a0 = sX4[row], a1 = sX4[128 + row], a2 = sX4[256 + row], a3 = sX4[384 + row];
           mh[0] = fmaxf(fmaxf(a0.x, a1.x), fmaxf(a2.x, a3.x)); mh[1] = fmaxf(fmaxf(a0.y, a1.y), fmaxf(a2.y, a3.y));
           mh[2] = fmaxf(fmaxf(a0.z, a1.z), fmaxf(a2.z, a3.z)); mh[3] = fmaxf(fmaxf(a0.w, a1.w), fmaxf(a2.w, a3.w));
         }
-        {
-#pragma unroll
-          for (int h = 0; h < LH; ++h) {
-            const float moff = mh[h] == -INFINITY ? 0.f : mh[h] - SC_P_SCALE_LOG2;
-            float sum = 0.f, g0 = 0.f, g1 = 0.f, g2 = 0.f;
-            uint32_t hw[SPT / 2], lw[SPT / 2];
-            float4 u;
-            float tq[SPT];
-            load_head(h, u, tq);
-#pragma unroll
-            for (int i = 0; i < SPT / 2; ++i) {
-              const float w0 = umma::ex2_raw(lscore(u, tq, 2 * i) - moff);
-              const float w1 = umma::ex2_raw(lscore(u, tq, 2 * i + 1) - moff);
-              sum += w0;
-              g0 = fmaf(w0, f0[2 * i], g0); g1 = fmaf(w0, f1[2 * i], g1); g2 = fmaf(w0, f2[2 * i], g2);
-              sum += w1;
-              g0 = fmaf(w1, f0[2 * i + 1], g0); g1 = fmaf(w1, f1[2 * i + 1], g1); g2 = fmaf(w1, f2[2 * i + 1], g2);
-              umma::split2_f16(w0, w1, hw[i], lw[i]);
-            }
-            const uint32_t ca = tl + SC_A1 + h * SKT + wsub * (SPT / 2);
-            umma::st4(ca, hw); umma::st2(ca + 4, hw + 4);
-            umma::st4(ca + SKT / 2, lw); umma::st2(ca + SKT / 2 + 4, lw + 4);
-            const uint32_t px[4] = {__float_as_uint(sum), __float_as_uint(g0), __float_as_uint(g1), __float_as_uint(g2)};
-            umma::st4(tl + SC_PX + 16 * wsub + 4 * h, px);
-          }
-        }
+        // (4) softmax weights -> TMEM, then the vps contraction
+        lp_weights<SPT, SKT>(ls, sU, sT, mh, tl, wsub);
         umma::wait_st();
         umma::fence_before_sync();
         __syncthreads();
         if (tid == 0) {
           umma::fence_after_sync();
-#pragma unroll
-          for (int h = 0; h < LH; ++h) {
-            const uint32_t d = tm + SC_D1 + 16 * h;
-            const uint32_t aHi = tm + SC_A1 + h * SKT, aLo = aHi + SKT / 2;
-            const uint32_t bHi = op1 + h * (SKT * 64), bLo = bHi + SKT * 32;
-#pragma unroll
-            for (int ks = 0; ks < SKT / 16; ++ks)
-              umma::mma_f16_ts(d, aLo + 8 * ks, umma::make_desc(bHi + ks * 512, 256, 128), idescO, ks > 0);
-#pragma unroll
-            for (int ks = 0; ks < SKT / 16; ++ks)
-              umma::mma_f16_ts(d, aHi + 8 * ks, umma::make_desc(bLo + ks * 512, 256, 128), idescO, true);
-#pragma unroll
-            for (int ks = 0; ks < SKT / 16; ++ks)
-              umma::mma_f16_ts(d, aHi + 8 * ks, umma::make_desc(bHi + ks * 512, 256, 128), idescO, true);
-          }
+          lp_issue_vps<SKT>(tm, op1, idescO);
           umma::commit(bar_loc);
         }
         PHASE_MARK(3);
+        // (5) ol -> A operand of the second contraction
         mbar_wait(bar_loc, 0u);
         umma::fence_after_sync();
-        {
-          uint32_t dv[8], pq[16];
-          umma::ld8_nw(tl + SC_D1 + 16 * wsub, dv);
-          umma::ld4_nw(tl + SC_PX + 4 * wsub, pq);
-          umma::ld4_nw(tl + SC_PX + 16 + 4 * wsub, pq + 4);
-          umma::ld4_nw(tl + SC_PX + 32 + 4 * wsub, pq + 8);
-          umma::ld4_nw(tl + SC_PX + 48 + 4 * wsub, pq + 12);
-          umma::wait_ld();
-          const float sum = (umma::after_wait(pq[0]) + umma::after_wait(pq[4])) + (umma::after_wait(pq[8]) + umma::after_wait(pq[12]));
-          const float inv_s = sum > 0.f ? 1.f / sum : 0.f;
-          const float g0 = ((umma::after_wait(pq[1]) + umma::after_wait(pq[5])) + (umma::after_wait(pq[9]) + umma::after_wait(pq[13]))) * inv_s;
-          const float g1 = ((umma::after_wait(pq[2]) + umma::after_wait(pq[6])) + (umma::after_wait(pq[10]) + umma::after_wait(pq[14]))) * inv_s;
-          const float g2 = ((umma::after_wait(pq[3]) + umma::after_wait(pq[7])) + (umma::after_wait(pq[11]) + umma::after_wait(pq[15]))) * inv_s;
-          float ol[LD];
-#pragma unroll
-          for (int c = 0; c < LD; ++c) {
-            const float4 a4 = *reinterpret_cast<const float4*>(sA + (wsub * LD + c) * 4);
-            ol[c] = fmaf(a4.z, g2, fmaf(a4.y, g1, a4.x * g0)) + a4.w + umma::after_wait(dv[c]) * inv_s;
-          }
-          uint32_t hw[4], lw[4];
-#pragma unroll
-          for (int i = 0; i < 4; ++i) umma::split2_f16(ol[2 * i], ol[2 * i + 1], hw[i], lw[i]);
-          umma::st4(tl + SC_A2 + 4 * wsub, hw);
-          umma::st4(tl + SC_A2 + 16 + 4 * wsub, lw);
-        }
+        lp_ol(tl, wsub, sA);
         umma::wait_st();
         umma::fence_before_sync();
         __syncthreads();
 
         // MMA issue helpers (leaders only): operands of the current key tile sit in the two 64 KB buffers
         auto issue_qk = [&](int head) {
-          const uint32_t d = tm + SC_S + grp * 128;
-          const uint32_t aHi = tm + SC_Q + 8 * head, aLo = aHi + 64;
-          const uint64_t bHi = umma::make_desc(bufA + head * 2 * lboN, lboN, 128);
-          const uint64_t bLo = umma::make_desc(bufA + 32768u + head * 2 * lboN, lboN, 128);
-          umma::mma_f16_ts(d, aLo, bHi, idescS, false);
-          umma::mma_f16_ts(d, aHi, bLo, idescS, true);
-          umma::mma_f16_ts(d, aHi, bHi, idescS, true);
+          const uint32_t aHi = tm + TC_COL_Q + 8 * head, bHi = bufA + head * 2 * lboN;
+          mma_split3(tm + TC_COL_S + grp * 128, aHi, aHi + 64, 0, bHi, bHi + 32768u, 0, lboN, idescS, 1, false);
         };
         auto issue_pv = [&](int head, bool accumulate) {
-          const uint32_t d = tm + SC_O + 16 * head;
-          const uint32_t pHi = tm + SC_S + grp * 128, pLo = pHi + 64;
-          const uint32_t vHi = bufB + head * (128 * 32), vLo = vHi + 32768u;
-          for (int ks = 0; ks < 8; ++ks)
-            umma::mma_f16_ts(d, pLo + 8 * ks, umma::make_desc(vHi + ks * 512, 256, 128), idescO, accumulate || ks > 0);
-          for (int ks = 0; ks < 8; ++ks)
-            umma::mma_f16_ts(d, pHi + 8 * ks, umma::make_desc(vLo + ks * 512, 256, 128), idescO, true);
-          for (int ks = 0; ks < 8; ++ks)
-            umma::mma_f16_ts(d, pHi + 8 * ks, umma::make_desc(vHi + ks * 512, 256, 128), idescO, true);
+          const uint32_t pHi = tm + TC_COL_S + grp * 128, vHi = bufB + head * (128 * 32);
+          mma_split3(tm + TC_COL_O + 16 * head, pHi, pHi + 64, 8, vHi, vHi + 32768u, 512, 256, idescO, 8, accumulate);
         };
         if (tid == 0) {
           umma::fence_after_sync();
-          const uint32_t d = tm + SC_D2, aHi = tm + SC_A2, aLo = aHi + 16;
-          const uint32_t lbo2 = (uint32_t)N2 * 16u, lo2 = (uint32_t)N2 * 64u;
-#pragma unroll
-          for (int ks = 0; ks < 2; ++ks)
-            umma::mma_f16_ts(d, aLo + 8 * ks, umma::make_desc(op2 + ks * 2 * lbo2, lbo2, 128), idescL2, ks > 0);
-#pragma unroll
-          for (int ks = 0; ks < 2; ++ks)
-            umma::mma_f16_ts(d, aHi + 8 * ks, umma::make_desc(op2 + lo2 + ks * 2 * lbo2, lbo2, 128), idescL2, true);
-#pragma unroll
-          for (int ks = 0; ks < 2; ++ks)
-            umma::mma_f16_ts(d, aHi + 8 * ks, umma::make_desc(op2 + ks * 2 * lbo2, lbo2, 128), idescL2, true);
+          lp_issue_pemz(tm, op2, N2, idescL2);
           umma::commit(bar_loc);
         }
         PHASE_MARK(4);
         // (6) penalty + local score per sequence position -> shared memory (with the node ids), read back after the score tiles
         mbar_wait(bar_loc, 1u);
         umma::fence_after_sync();
-        {
-          uint32_t dp[SPT], dz[4];
-          umma::ld8_nw(tl + SC_D2 + p0, dp);
-          umma::ld4_nw(tl + SC_D2 + p0 + 8, dp + 8);
-          umma::ld4_nw(tl + SC_D2 + K1, dz);
-          umma::wait_ld();
-          if (act) {
-            const float z0 = umma::after_wait(dz[0]) + sZB[0], z1 = umma::after_wait(dz[1]) + sZB[1];
-            const float z2 = umma::after_wait(dz[2]) + sZB[2], cz = umma::after_wait(dz[3]) + sZB[3];
-#pragma unroll
-            for (int s = 0; s < SPT; ++s) {
-              const int p = p0 + s;
-              if (p < np) {
-                const float pem = umma::after_wait(dp[s]) + sPB[p];
-                sAdd[row * SKT + p] = (fmaf(f2[s], z2, fmaf(f1[s], z1, f0[s] * z0)) + cz + pem) - f0[s] * cpen;
-                sAddId[row * SKT + p] = (uint16_t)((idw[s >> 1] >> ((s & 1) * 16)) & 0xffffu);
-              }
-            }
-            if (wsub == 0) sNp[row] = np;
-          } else if (wsub == 0) {
-            sNp[row] = 0;
-          }
-        }
+        lp_pen_local(ls, tl, K1, np, act, sZB, sPB, [&](int s, int p, float v) {
+          sAdd[row * SKT + p] = v;
+          sAddId[row * SKT + p] = (uint16_t)((idw[s >> 1] >> ((s & 1) * 16)) & 0xffffu);
+        });
+        if (wsub == 0) sNp[row] = np;          // 0 for an idle row
         umma::fence_before_sync();
         __syncthreads();                       // [pem | z] read by everybody before the first P V reuses the columns
 
@@ -566,7 +412,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
                 bulk_g2s(sm + L::buf, et + (size_t)(kt + 1) * ELG_TILE_BYTES + 65536, 65536u, bar_kv);
               }
             }
-            const uint32_t sb = tl + SC_S + grp * 128;
+            const uint32_t sb = tl + TC_COL_S + grp * 128;
             uint32_t sr[64];
             umma::ld32_nw(sb + kh * 64, sr);
             umma::ld32_nw(sb + kh * 64 + 32, sr + 32);
@@ -582,7 +428,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
             // the row's maximum over this tile: both key halves (shared memory + 64-thread barrier)
             float* xmx = reinterpret_cast<float*>(sX2);
             xmx[wsub * 128 + row] = mloc;
-            pair_sync_s(1 + grp * 4 + q);
+            pair_sync(1 + grp * 4 + q);
             const float mt = fmaxf(mloc, xmx[(wsub ^ 1) * 128 + row]);
             const float mold = rho == 0 ? mr0 : (rho == 1 ? mr1 : (rho == 2 ? mr2 : mr3));
             const float mnew = fmaxf(mold, mt);
@@ -591,14 +437,14 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
             // a higher maximum: rescale the head's accumulator columns (my half of the 16) before P V adds to them
             if (kt > 0 && __any_sync(FULL, fsc != 1.f)) {
               uint32_t oc[8];
-              const uint32_t oa = tl + SC_O + 16 * (4 * grp + rho) + 8 * kh;
+              const uint32_t oa = tl + TC_COL_O + 16 * (4 * grp + rho) + 8 * kh;
               umma::ld8_nw(oa, oc);
               umma::wait_ld();
 #pragma unroll
               for (int i = 0; i < 8; ++i) oc[i] = __float_as_uint(umma::after_wait(oc[i]) * fsc);
               umma::st8(oa, oc);
             }
-            const float moff = mnew == -INFINITY ? 0.f : mnew - SC_P_SCALE_LOG2;
+            const float moff = mnew == -INFINITY ? 0.f : mnew - TC_P_SCALE_LOG2;
             float lloc = 0.f;
 #pragma unroll
             for (int i = 0; i < 32; ++i) {
@@ -622,7 +468,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
             umma::st16s<2>(sb + 64 + kh * 32 + 16, sr + 33);
             umma::wait_st();
             umma::fence_before_sync();
-            group_sync_s(9 + grp);
+            group_sync(9 + grp);
             if (leader) {
               if (rho == 0) mbar_wait(bar_v, ph_v);                   // the tile's V^T (in flight since the end of the previous tile)
               umma::fence_after_sync();
@@ -653,24 +499,12 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
         }
         sX4[wsub * 128 + row] = make_float4(lt0, lt1, lt2, lt3);
         if (tid < 128) sEb[tid] = tid < N1 ? pEb[tid] : 0.f;
-        pair_sync_s(1 + grp * 4 + q);
+        pair_sync(1 + grp * 4 + q);
         {
           const float4 lo4 = sX4[(wsub ^ 1) * 128 + row];
           const float la = kh ? (lt2 + lo4.z) : (lt0 + lo4.x), lb = kh ? (lt3 + lo4.w) : (lt1 + lo4.y);
-          uint32_t orr[32], hw[16], lw[16];
           umma::fence_after_sync();
-          umma::ld32_nw(tl + SC_O + 16 * (4 * grp + 2 * kh), orr);
-          umma::wait_ld();
-#pragma unroll
-          for (int i2 = 0; i2 < 2; ++i2) {
-            const float inv_l = act ? 1.f / (i2 ? lb : la) : 0.f;
-#pragma unroll
-            for (int d2 = 0; d2 < 8; ++d2)
-              umma::split2_f16(act ? umma::after_wait(orr[i2 * 16 + 2 * d2]) * inv_l : 0.f,
-                               act ? umma::after_wait(orr[i2 * 16 + 2 * d2 + 1]) * inv_l : 0.f, hw[i2 * 8 + d2], lw[i2 * 8 + d2]);
-          }
-          umma::st16s<1>(tl + SC_Q + 8 * (4 * grp + 2 * kh), hw);
-          umma::st16s<1>(tl + SC_Q + 64 + 8 * (4 * grp + 2 * kh), lw);
+          store_o_operand(tl, grp, kh, la, lb, act);
           umma::wait_st();
           umma::fence_before_sync();
         }
@@ -682,16 +516,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
         // while its scores are being read); the second buffer is a [128 rows][128 nodes] scratch for the scores of the
         // tile's NEIGHBOUR nodes, which get `penalty + local` instead of xi from the threads that own the local sequence
         auto issue_score = [&](int nt) {
-          const uint32_t d = tm + SC_S + (nt & 1) * 128;
-#pragma unroll
-          for (int ks = 0; ks < 8; ++ks)
-            umma::mma_f16_ts(d, tm + SC_Q + 64 + 8 * ks, umma::make_desc(bufA + ks * 2 * lboN, lboN, 128), idescS, ks > 0);
-#pragma unroll
-          for (int ks = 0; ks < 8; ++ks)
-            umma::mma_f16_ts(d, tm + SC_Q + 8 * ks, umma::make_desc(bufA + 32768u + ks * 2 * lboN, lboN, 128), idescS, true);
-#pragma unroll
-          for (int ks = 0; ks < 8; ++ks)
-            umma::mma_f16_ts(d, tm + SC_Q + 8 * ks, umma::make_desc(bufA + ks * 2 * lboN, lboN, 128), idescS, true);
+          mma_split3(tm + TC_COL_S + (nt & 1) * 128, tm + TC_COL_Q, tm + TC_COL_Q + 64, 8, bufA, bufA + 32768u, 2 * lboN, lboN, idescS, 8, false);
           umma::commit(bar_scm);
         };
         float* sSc = sm + L::buf + 16384;                 // scratch: score of node jl of this tile at [row][jl ^ (row & 31)]
@@ -724,7 +549,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
           }
           {
             uint32_t xr[32];
-            umma::ld32_nw(tl + SC_S + sl2 * 128 + 32 * wsub, xr);
+            umma::ld32_nw(tl + TC_COL_S + sl2 * 128 + 32 * wsub, xr);
             umma::wait_ld();
             if (act) {
               const int jb = nt * 128 + 32 * wsub;
@@ -744,7 +569,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
             }
           }
           umma::fence_before_sync();
-          quad_sync_s(11 + q);      // the scratch row is written and read by the four threads of the row (one lane quadrant);
+          quad_sync(11 + q);      // the scratch row is written and read by the four threads of the row (one lane quadrant);
                                     // the CTA barrier at the end of the iteration still orders the accumulator reads of all
                                     // warps before the MMAs of the tile after next
           // the neighbours of this tile (and the depot) with their own penalty + local score; only the depot can be masked
@@ -770,7 +595,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
         }
         PHASE_MARK(8);
         sX2[wsub * 128 + row] = make_float2(vbest, __int_as_float(ibest));
-        quad_sync_s(11 + q);        // candidates of a row: its lane quadrant only
+        quad_sync(11 + q);        // candidates of a row: its lane quadrant only
         {
           float bv = -INFINITY;
           int bi = 0x7fffffff;
@@ -829,14 +654,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
         live_after = !fin;
         if (wsub == 0) {
           if (t > 0) {
-            float sg;
-            if (A.t.unscaled) {
-              const float* ux = A.t.unscaled + (size_t)b * N1 * 2;
-              sg = rintf(seglen(ux[2 * cur0] - ux[2 * sl], ux[2 * cur0 + 1] - ux[2 * sl + 1]));
-            } else {
-              sg = seglen(pXY[2 * cur0] - pXY[2 * sl], pXY[2 * cur0 + 1] - pXY[2 * sl + 1]);
-            }
-            sTlen[row] += sg;
+            sTlen[row] += seg_cost(A.t, b, N1, pXY, cur0, sl);
           }
           if (!CVRP && t == 0) sFirst[row] = sl;
           sCur[row] = sl;
@@ -857,13 +675,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_stc_kernel(const RolloutArgs A)
     for (int r = tid; r < nrows; r += RT) {
       float len = sTlen[r];
       if (!CVRP) {
-        const int a = sCur[r], f = sFirst[r];
-        if (A.t.unscaled) {
-          const float* ux = A.t.unscaled + (size_t)b * N1 * 2;
-          len += rintf(seglen(ux[2 * a] - ux[2 * f], ux[2 * a + 1] - ux[2 * f + 1]));
-        } else {
-          len += seglen(pXY[2 * a] - pXY[2 * f], pXY[2 * a + 1] - pXY[2 * f + 1]);
-        }
+        len += seg_cost(A.t, b, N1, pXY, sCur[r], sFirst[r]);
       }
       const size_t gg = (size_t)b * A.M + row0 + r;
       A.reward[gg] = -len;

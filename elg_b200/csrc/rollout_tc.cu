@@ -12,15 +12,16 @@
 //   [pem | z] = ol [PW | ZW]  A = local attention output ol, 32 wide (TMEM)   B = (K1 + 4) x 32 (smem, model constant)
 //
 // Split precision (x = hi + lo, fp16 each) with the two small cross terms issued BEFORE hi*hi into the same fp32
-// accumulator keeps every contraction fp32-grade (tests/test_umma_selftest.py).
+// accumulator keeps every contraction fp32-grade (mma_split3 in rollout_common.cuh, tests/test_umma_selftest.py).
 //
 // CTA = one (aug-instance, tile of <= 112 POMO rows); TMEM lane = row.  16 warps: warp w owns TMEM lane quadrant
 // q = w % 4 (rows 32q..32q+31) and sub-slot wsub = w / 4, so a row is served by four threads in four warps that
 // exchange data through the row's TMEM lane or through shared memory + a 128-thread named barrier:
 //   L        local policy, thread = (row, quarter wsub of the local sequence): rank-space validity bits of the
-//            distance-presorted neighbour list, first-k walk by bit scans, features from the pair table, 4-head
-//            scores + softmax weights -> TMEM A operand; the two contractions on the tensor core; thread =
-//            (row, local head wsub) in between; results to shared memory ordered by node id
+//            distance-presorted neighbour list, first-k walk by bit scans, features from the pair table; then the
+//            local policy shared with rollout_stc.cu (rollout_common.cuh): 4-head scores + softmax weights -> TMEM A
+//            operand, the two contractions on the tensor core, thread = (row, local head wsub) in between; results to
+//            shared memory ordered by node id
 //   softmax  two independent groups of 8 warps (grp = wsub / 2): group g walks heads 4g..4g+3 one at a time through
 //            its own S/P buffer, its own mbarrier and a 256-thread named barrier, so one group's tensor-core / TMEM
 //            latency is covered by the other group's arithmetic.  thread = (row, key half kh = wsub & 1); the two
@@ -29,27 +30,18 @@
 //            first-max argmax combined across the 4 quarters through shared memory
 //   C        env step: every thread of a row recomputes the scalar state, owns mask word wsub
 //
-// TMEM columns: [0,128) Q hi|lo, later O hi|lo   [128,256) O accumulators (8 heads x 16)
-//               [256,256+2*N1p) S / P buffers of the two groups, later the score accumulator
-//   during L (before the first Q K^T): [128,192) partial (sum, g) of the four sequence quarters, later [pem | z]
-//               [192,224) ol hi|lo   [224,256) head maxima + neighbour bits of the four quarters   [256,256+4*KT) local softmax weights hi|lo per head   [448,512) vps accumulators
+// TMEM columns: the plan in rollout_common.cuh, with S / P buffers of 2 * N1p columns at [256, 256 + 2 * N1p)
 #include <cstdlib>
 #include "rollout_common.cuh"
 
 namespace elg {
 
 constexpr int TC_MT_MAX = 112;
-constexpr uint32_t TC_COL_Q = 0, TC_COL_O = 128, TC_COL_S = 256;
-constexpr float TC_P_SCALE_LOG2 = 10.f;      // softmax weights are 2^(s - m + 10): keeps small weights out of fp16 subnormals
-
-constexpr uint32_t TC_COL_PX = 128, TC_COL_D2 = 128, TC_COL_A2 = 192, TC_COL_A1 = 256, TC_COL_D1 = 448;
 constexpr int TC_XCH_FLOATS = 2 * 4 * 128 * 4;      // local-policy exchanges (validity words, neighbour bits), alias `add`
 
 // Shared-memory layout in floats.  Every offset is a compile-time constant (sized for the largest resident instance:
 // 112 node slots, 112 rows, KT local positions), so that shared-memory addresses are immediates instead of registers.
 constexpr int TC_NP = 112;                  // node slots (N1 rounded up to 16, at most)
-__host__ __device__ constexpr int tc_r4(int x) { return (x + 3) & ~3; }
-__host__ __device__ constexpr int tc_n2(int K1) { return (K1 + 4 + 15) & ~15; }      // columns of [pem | z]
 template <int KT>
 struct TcL {
   static constexpr int MT = TC_MT_MAX;
@@ -80,28 +72,6 @@ struct TcL {
   static constexpr int total = bar + 12;
 };
 static_assert(TcL<48>::total * 4 <= 227 * 1024 && TcL<32>::total * 4 <= 227 * 1024, "layout exceeds one SM's shared memory");
-
-__device__ __forceinline__ uint32_t pick4(const uint32_t (&w)[4], int i) {
-  return i == 0 ? w[0] : (i == 1 ? w[1] : (i == 2 ? w[2] : (i == 3 ? w[3] : 0u)));
-}
-__device__ __forceinline__ void pair_sync(int id) { asm volatile("bar.sync %0, 64;" ::"r"(id) : "memory"); }
-__device__ __forceinline__ void group_sync(int id) { asm volatile("bar.sync %0, 256;" ::"r"(id) : "memory"); }
-__device__ __forceinline__ void quad_sync(int id) { asm volatile("bar.sync %0, 128;" ::"r"(id) : "memory"); }
-
-// position (0..127) of the n-th (0-based) set bit of the 128-bit value r[3]:r[2]:r[1]:r[0]; n < popc(r)
-__device__ __forceinline__ int select128(const uint32_t (&r)[4], int n) {
-  const int c0 = __popc(r[0]), c1 = c0 + __popc(r[1]), c2 = c1 + __popc(r[2]);
-  const int w = (n >= c0 ? 1 : 0) + (n >= c1 ? 1 : 0) + (n >= c2 ? 1 : 0);
-  int m = n - (w == 0 ? 0 : (w == 1 ? c0 : (w == 2 ? c1 : c2)));
-  uint32_t x = pick4(r, w);
-  int pos = 0, t;
-  t = __popc(x & 0xffffu); if (m >= t) { m -= t; pos = 16; x >>= 16; }
-  t = __popc(x & 0xffu);   if (m >= t) { m -= t; pos += 8; x >>= 8; }
-  t = __popc(x & 0xfu);    if (m >= t) { m -= t; pos += 4; x >>= 4; }
-  t = __popc(x & 0x3u);    if (m >= t) { m -= t; pos += 2; x >>= 2; }
-  t = (int)(x & 1u);       if (m >= t) pos += 1;
-  return w * 32 + pos;
-}
 
 // =================================================================================================
 // NP = 112: the node count rounded up to 16 is known at compile time (the 100-node benchmark shapes); NP = 0: run time
@@ -150,21 +120,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
   const int KH = N1p >> 1, CQ = N1p >> 2;          // keys per softmax thread, node columns per B3 thread
 
   {
-    const float* loc = A.derived + DER_LOC;
-    float* w = sm;
-    for (int i = tid; i < E; i += RT) w[L::wl + i] = A.derived[DER_WL + i];
-    for (int i = tid; i < LH * 4; i += RT) w[L::u + i] = loc[LOC_U + i];
-    for (int i = tid; i < LH * KT_MAX; i += RT) w[L::tt + i] = loc[LOC_T + i];
-    for (int i = tid; i < LE * 4; i += RT) w[L::a + i] = (i & 3) == 3 ? loc[LOC_CV + (i >> 2)] : loc[LOC_A + i];
-    for (int i = tid; i < KT_MAX; i += RT) w[L::pb + i] = loc[LOC_PB + i];
-    for (int i = tid; i < 4; i += RT) w[L::zb + i] = loc[LOC_ZB + i];
-    // local-policy B operands (model constants, written in the tcgen05 layout by elg_prepare_model): per head
-    // [hi | lo] of the first KT sequence positions out of KT_MAX; [PW | ZW] as built for this model's K1
-    for (int i = tid; i < LH * KT * 16; i += RT) {            // 32-bit words: per head 2 x KT * 8
-      const int h = i / (KT * 16), r = i % (KT * 16), part = r / (KT * 8), x = r % (KT * 8);
-      w[L::op1 + i] = loc[LOC_OP1 + h * (KT_MAX * 16) + part * (KT_MAX * 8) + x];
-    }
-    for (int i = tid; i < tc_n2(K1) * LE; i += RT) w[L::op2 + i] = loc[LOC_OP2 + i];
+    stage_local_consts<L, KT>(sm, A.derived, tc_n2(K1), tid);
     if (tid == 0) {
       mbar_init(bar, 1);
       mbar_init(bar + 1, 1);
@@ -364,8 +320,9 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
         const int np = act ? kk + DEP : 0;
         const int p0 = wsub * PT;
         const float4* rec = reinterpret_cast<const float4*>(nrow + ELG_NBR_STRIDE + ELG_NBR_PAIR_BYTES(N1));   // by list rank
-        float f0[PT], f1[PT], f2[PT];
-        float cpen = 1.f;                                                 // distance penalty = -f0 * cpen
+        LocalSeq<PT> ls;
+        ls.p0 = p0;
+        ls.cpen = 1.f;
         uint32_t idw[PT / 4];                                             // this thread's node ids, 4 per word
         uint32_t nbp[4] = {0u, 0u, 0u, 0u};                               // their bits in node space
         {
@@ -403,7 +360,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
           const float dmax = rlast.x;
           const float r0d = dmax != 0.f ? 1.f / (dmax + 1e-6f) : 1.f;      // cvrp: cur_dist / (max + 1e-6); dmax == 0 -> dd itself
           // penalty -d / dmax (no eps, CVRP/models.py:380,403) = -f0 (dmax + 1e-6) / dmax; tsp: -d / (dmax + 1e-6) = -f0
-          if (CVRP && dmax != 0.f) cpen = (dmax + 1e-6f) / dmax;
+          if (CVRP && dmax != 0.f) ls.cpen = (dmax + 1e-6f) / dmax;
           const float rtsp = 1.f / (dmax + 1e-6f);
           const float rld = 1.f / ld0;
 #pragma unroll
@@ -412,17 +369,17 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
 #pragma unroll
           for (int s = 0; s < PT; ++s) {
             const bool mine = (p0 + s) < np && !(DEP && s == 0 && wsub == 0);
-            f0[s] = f1[s] = f2[s] = 0.f;
+            ls.f0[s] = ls.f1[s] = ls.f2[s] = 0.f;
             if (mine) {
               const int nd = __float_as_int(rv[s].w);
               idw[s >> 2] |= (uint32_t)nd << ((s & 3) * 8);
               if (CVRP) {
-                f0[s] = rv[s].x * r0d;
-                f2[s] = rv[s].z * rld;
+                ls.f0[s] = rv[s].x * r0d;
+                ls.f2[s] = rv[s].z * rld;
               } else {
-                f0[s] = rv[s].x * rtsp;
+                ls.f0[s] = rv[s].x * rtsp;
               }
-              f1[s] = rv[s].y;
+              ls.f1[s] = rv[s].y;
               const unsigned long long bit = 1ull << (nd & 63);
               na |= (nd & 64) ? 0ull : bit;
               nb2 |= (nd & 64) ? bit : 0ull;
@@ -434,23 +391,8 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
         PHASE_MARK(1);
         // (3) scores of the constant local query, all four heads for my positions (log2 domain); the row's maximum
         //     per head and the neighbour bits of the row come from the four quarters through shared memory
-        // score of position s under head h given the head's (u0, u1, u2) and table entries t[s]; positions past np and a
-        // masked depot (standing on it) score -inf
-        const int nv = np - p0;                                           // my valid positions are s < nv
-        const bool dep_off = DEP && wsub == 0 && depot_masked;
-        auto load_head = [&](int h, float4& u, float (&tq)[PT]) {
-          u = *reinterpret_cast<const float4*>(sU + h * 4);
-#pragma unroll
-          for (int i = 0; i < PT / 4; ++i) {
-            const float4 t4 = *reinterpret_cast<const float4*>(sT + h * KT_MAX + p0 + 4 * i);
-            tq[4 * i] = t4.x; tq[4 * i + 1] = t4.y; tq[4 * i + 2] = t4.z; tq[4 * i + 3] = t4.w;
-          }
-          if (dep_off) tq[0] = -INFINITY;
-        };
-        auto lscore = [&](const float4& u, const float (&tq)[PT], int s) -> float {
-          const float v = fmaf(u.z, f2[s], fmaf(u.y, f1[s], fmaf(u.x, f0[s], tq[s])));
-          return s < nv ? v : -INFINITY;
-        };
+        ls.nv = np - p0;
+        ls.dep_off = DEP && wsub == 0 && depot_masked;
         float mh[LH];
         {
           uint32_t nbw[4];                                                // neighbour bit mask of the row (node space)
@@ -458,16 +400,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
           uint32_t mp[2];
           {
             float m4[LH];
-#pragma unroll
-            for (int h = 0; h < LH; ++h) {
-              float4 u;
-              float tq[PT];
-              load_head(h, u, tq);
-              float m = -INFINITY;
-#pragma unroll
-              for (int s = 0; s < PT; ++s) m = fmaxf(m, lscore(u, tq, s));
-              m4[h] = m;
-            }
+            lp_head_max(ls, sU, sT, m4);
             mp[0] = umma::pack_h2(__float2half_ru(m4[0]), __float2half_ru(m4[1]));
             mp[1] = umma::pack_h2(__float2half_ru(m4[2]), __float2half_ru(m4[3]));
           }
@@ -491,171 +424,58 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
           if (wsub == 0 && act) *reinterpret_cast<uint4*>(sNb + rc * 4) = make_uint4(nbw[0], nbw[1], nbw[2], nbw[3]);   // read back in (6) and B3
         }
         PHASE_MARK(2);
-        // (4) weights 2^(s - max + 10) -> A operand of head h (TMEM, fp16 hi/lo, slot = sequence position); partial
-        //     (sum, sum w f) of my positions -> TMEM exchange columns
-        {
-#pragma unroll
-          for (int h = 0; h < LH; ++h) {
-            const float moff = mh[h] == -INFINITY ? 0.f : mh[h] - TC_P_SCALE_LOG2;
-            float sum = 0.f, g0 = 0.f, g1 = 0.f, g2 = 0.f;
-            uint32_t hw[PT / 2], lw[PT / 2];
-            float4 u;
-            float tq[PT];
-            load_head(h, u, tq);
-#pragma unroll
-            for (int i = 0; i < PT / 2; ++i) {
-              const float w0 = umma::ex2_raw(lscore(u, tq, 2 * i) - moff); // -inf (masked / beyond np) -> 0
-              const float w1 = umma::ex2_raw(lscore(u, tq, 2 * i + 1) - moff);
-              sum += w0;
-              g0 = fmaf(w0, f0[2 * i], g0); g1 = fmaf(w0, f1[2 * i], g1); g2 = fmaf(w0, f2[2 * i], g2);
-              sum += w1;
-              g0 = fmaf(w1, f0[2 * i + 1], g0); g1 = fmaf(w1, f1[2 * i + 1], g1); g2 = fmaf(w1, f2[2 * i + 1], g2);
-              umma::split2_f16(w0, w1, hw[i], lw[i]);
-            }
-            const uint32_t ca = tl + TC_COL_A1 + h * KT + wsub * (PT / 2);
-            if (PT == 8) {
-              umma::st4(ca, hw);
-              umma::st4(ca + KT / 2, lw);
-            } else {                                                       // PT == 12
-              umma::st4(ca, hw); umma::st2(ca + 4, hw + 4);
-              umma::st4(ca + KT / 2, lw); umma::st2(ca + KT / 2 + 4, lw + 4);
-            }
-            const uint32_t px[4] = {__float_as_uint(sum), __float_as_uint(g0), __float_as_uint(g1), __float_as_uint(g2)};
-            umma::st4(tl + TC_COL_PX + 16 * wsub + 4 * h, px);
-          }
-        }
+        // (4) softmax weights -> TMEM, then the vps contraction
+        lp_weights<PT, KT>(ls, sU, sT, mh, tl, wsub);
         umma::wait_st();                                                   // also the Q operand
         umma::fence_before_sync();
         __syncthreads();
         if (tid == 0) {
-          // vps_h = W_h (Wv PE)_h: per head KT/16 k-steps x (lo*hi, hi*lo, hi*hi)
           umma::fence_after_sync();
-#pragma unroll
-          for (int h = 0; h < LH; ++h) {
-            const uint32_t d = tm + TC_COL_D1 + 16 * h;
-            const uint32_t aHi = tm + TC_COL_A1 + h * KT, aLo = aHi + KT / 2;
-            const uint32_t bHi = op1 + h * (KT * 64), bLo = bHi + KT * 32;
-#pragma unroll
-            for (int ks = 0; ks < KT / 16; ++ks)
-              umma::mma_f16_ts(d, aLo + 8 * ks, umma::make_desc(bHi + ks * 512, 256, 128), idescO, ks > 0);
-#pragma unroll
-            for (int ks = 0; ks < KT / 16; ++ks)
-              umma::mma_f16_ts(d, aHi + 8 * ks, umma::make_desc(bLo + ks * 512, 256, 128), idescO, true);
-#pragma unroll
-            for (int ks = 0; ks < KT / 16; ++ks)
-              umma::mma_f16_ts(d, aHi + 8 * ks, umma::make_desc(bHi + ks * 512, 256, 128), idescO, true);
-          }
+          lp_issue_vps<KT>(tm, op1, idescO);
           umma::commit(bar_loc);
         }
         PHASE_MARK(3);
-        // (5) thread = (row, local head wsub): ol = (Wv We) g + Wv be + vps, normalised -> A operand of the second
-        //     contraction
+        // (5) ol -> A operand of the second contraction
         mbar_wait(bar_loc, 0u);
         umma::fence_after_sync();
-        {
-          uint32_t dv[8], pq[16];
-          umma::ld8_nw(tl + TC_COL_D1 + 16 * wsub, dv);
-          umma::ld4_nw(tl + TC_COL_PX + 4 * wsub, pq);
-          umma::ld4_nw(tl + TC_COL_PX + 16 + 4 * wsub, pq + 4);
-          umma::ld4_nw(tl + TC_COL_PX + 32 + 4 * wsub, pq + 8);
-          umma::ld4_nw(tl + TC_COL_PX + 48 + 4 * wsub, pq + 12);
-          umma::wait_ld();
-          const float sum = (umma::after_wait(pq[0]) + umma::after_wait(pq[4])) + (umma::after_wait(pq[8]) + umma::after_wait(pq[12]));
-          const float inv_s = sum > 0.f ? 1.f / sum : 0.f;
-          const float g0 = ((umma::after_wait(pq[1]) + umma::after_wait(pq[5])) + (umma::after_wait(pq[9]) + umma::after_wait(pq[13]))) * inv_s;
-          const float g1 = ((umma::after_wait(pq[2]) + umma::after_wait(pq[6])) + (umma::after_wait(pq[10]) + umma::after_wait(pq[14]))) * inv_s;
-          const float g2 = ((umma::after_wait(pq[3]) + umma::after_wait(pq[7])) + (umma::after_wait(pq[11]) + umma::after_wait(pq[15]))) * inv_s;
-          float ol[LD];
-#pragma unroll
-          for (int c = 0; c < LD; ++c) {
-            const float4 a4 = *reinterpret_cast<const float4*>(sA + (wsub * LD + c) * 4);
-            ol[c] = fmaf(a4.z, g2, fmaf(a4.y, g1, a4.x * g0)) + a4.w + umma::after_wait(dv[c]) * inv_s;
-          }
-          uint32_t hw[4], lw[4];
-#pragma unroll
-          for (int i = 0; i < 4; ++i) umma::split2_f16(ol[2 * i], ol[2 * i + 1], hw[i], lw[i]);
-          umma::st4(tl + TC_COL_A2 + 4 * wsub, hw);
-          umma::st4(tl + TC_COL_A2 + 16 + 4 * wsub, lw);
-        }
+        lp_ol(tl, wsub, sA);
         umma::wait_st();
         umma::fence_before_sync();
         __syncthreads();
 
-        // MMA issue helpers (leaders only).  Per contraction: lo*hi, hi*lo, then hi*hi into one accumulator.
+        // MMA issue helpers (leaders only)
         auto issue_qk = [&](int head) {
-          const uint32_t d = tm + TC_COL_S + grp * N1p;
-          const uint32_t aHi = tm + TC_COL_Q + 8 * head, aLo = aHi + 64;
-          const uint64_t bHi = umma::make_desc(opK + head * 2 * lboN, lboN, 128);
-          const uint64_t bLo = umma::make_desc(opK + half + head * 2 * lboN, lboN, 128);
-          umma::mma_f16_ts(d, aLo, bHi, idescS, false);
-          umma::mma_f16_ts(d, aHi, bLo, idescS, true);
-          umma::mma_f16_ts(d, aHi, bHi, idescS, true);
+          const uint32_t aHi = tm + TC_COL_Q + 8 * head, bHi = opK + head * 2 * lboN;
+          mma_split3(tm + TC_COL_S + grp * N1p, aHi, aHi + 64, 0, bHi, bHi + half, 0, lboN, idescS, 1, false);
         };
         auto issue_pv = [&](int head) {
-          const uint32_t d = tm + TC_COL_O + 16 * head;
-          const uint32_t pHi = tm + TC_COL_S + grp * N1p, pLo = pHi + (N1p >> 1);
-          const uint32_t vHi = opV + head * (N1p * 32), vLo = vHi + half;
-          for (int ks = 0; ks < nks; ++ks)
-            umma::mma_f16_ts(d, pLo + 8 * ks, umma::make_desc(vHi + ks * 512, 256, 128), idescO, ks > 0);
-          for (int ks = 0; ks < nks; ++ks)
-            umma::mma_f16_ts(d, pHi + 8 * ks, umma::make_desc(vLo + ks * 512, 256, 128), idescO, true);
-          for (int ks = 0; ks < nks; ++ks)
-            umma::mma_f16_ts(d, pHi + 8 * ks, umma::make_desc(vHi + ks * 512, 256, 128), idescO, true);
+          const uint32_t pHi = tm + TC_COL_S + grp * N1p, vHi = opV + head * (N1p * 32);
+          mma_split3(tm + TC_COL_O + 16 * head, pHi, pHi + (N1p >> 1), 8, vHi, vHi + half, 512, 256, idescO, nks, false);
         };
         if (leader) {
           umma::fence_after_sync();
           if (tid == 0) {
-            // [pem | z] = ol [PW | ZW]: 2 k-steps x (lo*hi, hi*lo, hi*hi); the accumulator takes over the exchange columns
-            const uint32_t d = tm + TC_COL_D2, aHi = tm + TC_COL_A2, aLo = aHi + 16;
-            const uint32_t lbo2 = (uint32_t)N2 * 16u, lo2 = (uint32_t)N2 * 64u;
-#pragma unroll
-            for (int ks = 0; ks < 2; ++ks)
-              umma::mma_f16_ts(d, aLo + 8 * ks, umma::make_desc(op2 + ks * 2 * lbo2, lbo2, 128), idescL2, ks > 0);
-#pragma unroll
-            for (int ks = 0; ks < 2; ++ks)
-              umma::mma_f16_ts(d, aHi + 8 * ks, umma::make_desc(op2 + lo2 + ks * 2 * lbo2, lbo2, 128), idescL2, true);
-#pragma unroll
-            for (int ks = 0; ks < 2; ++ks)
-              umma::mma_f16_ts(d, aHi + 8 * ks, umma::make_desc(op2 + ks * 2 * lbo2, lbo2, 128), idescL2, true);
+            lp_issue_pemz(tm, op2, N2, idescL2);
             umma::commit(bar_loc);
           }
           issue_qk(4 * grp);
           umma::commit(bar_grp);
         }
         PHASE_MARK(4);
-        // (6) penalty + local score of my positions: pen + f . z + z3 + pem[p] (tables carry the 1/sqrt(32)), stored
-        //     ordered by node id for phase B3 (runs while the tensor core works on the first Q K^T)
+        // (6) penalty + local score of my positions, stored ordered by node id for phase B3 (runs while the tensor core
+        //     works on the first Q K^T)
         mbar_wait(bar_loc, 1u);
         umma::fence_after_sync();
         {
-          uint32_t dp[PT], dz[4];
-          if (PT == 8) {
-            umma::ld8_nw(tl + TC_COL_D2 + p0, dp);
-          } else {
-            umma::ld8_nw(tl + TC_COL_D2 + p0, dp);
-            umma::ld4_nw(tl + TC_COL_D2 + p0 + 8, dp + 8);
-          }
-          umma::ld4_nw(tl + TC_COL_D2 + K1, dz);
-          umma::wait_ld();
-          if (act) {
-            const float z0 = umma::after_wait(dz[0]) + sZB[0], z1 = umma::after_wait(dz[1]) + sZB[1];
-            const float z2 = umma::after_wait(dz[2]) + sZB[2], c0 = umma::after_wait(dz[3]) + sZB[3];
-            const uint4 n4 = *reinterpret_cast<const uint4*>(sNb + rc * 4);
-            const uint32_t nbw[4] = {n4.x, n4.y, n4.z, n4.w};
-            const int pc1 = __popc(nbw[0]), pc2 = pc1 + __popc(nbw[1]), pc3 = pc2 + __popc(nbw[2]);
-#pragma unroll
-            for (int s = 0; s < PT; ++s) {
-              const int p = p0 + s;
-              if (p < np) {
-                const float pem = umma::after_wait(dp[s]) + sPB[p];
-                const float addv = (fmaf(f2[s], z2, fmaf(f1[s], z1, f0[s] * z0)) + c0 + pem) - f0[s] * cpen;
-                const int nd = (idw[s >> 2] >> ((s & 3) * 8)) & 0xff, wd = nd >> 5;
-                const uint32_t below = pick4(nbw, wd) & ((1u << (nd & 31)) - 1u);
-                const int rank = (wd == 0 ? 0 : (wd == 1 ? pc1 : (wd == 2 ? pc2 : pc3))) + __popc(below);
-                sAdd[rc * KT + rank] = addv;
-              }
-            }
-          }
+          const uint4 n4 = *reinterpret_cast<const uint4*>(sNb + rc * 4);
+          const uint32_t nbw[4] = {n4.x, n4.y, n4.z, n4.w};
+          const int pc1 = __popc(nbw[0]), pc2 = pc1 + __popc(nbw[1]), pc3 = pc2 + __popc(nbw[2]);
+          lp_pen_local(ls, tl, K1, np, act, sZB, sPB, [&](int s, int, float v) {
+            const int nd = (idw[s >> 2] >> ((s & 3) * 8)) & 0xff, wd = nd >> 5;
+            const uint32_t below = pick4(nbw, wd) & ((1u << (nd & 31)) - 1u);
+            const int rank = (wd == 0 ? 0 : (wd == 1 ? pc1 : (wd == 2 ? pc2 : pc3))) + __popc(below);
+            sAdd[rc * KT + rank] = v;
+          });
         }
         PHASE_MARK(5);
 
@@ -756,20 +576,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
           pair_sync(1 + grp * 4 + q);
           const float la = (kh ? lt2 : lt0) + sXm[(wsub ^ 1) * 128 + row];
           const float lb = (kh ? lt3 : lt1) + sXl[(wsub ^ 1) * 128 + row];
-          uint32_t orr[32], hw[16], lw[16];            // heads 4*grp + 2*kh, + 1: 32 consecutive accumulator columns
-          umma::ld32_nw(tl + TC_COL_O + 16 * (4 * grp + 2 * kh), orr);
-          umma::wait_ld();
-#pragma unroll
-          for (int i2 = 0; i2 < 2; ++i2) {
-            const float lsel = i2 ? lb : la;
-            const float inv_l = act ? 1.f / lsel : 0.f;
-#pragma unroll
-            for (int d2 = 0; d2 < 8; ++d2)
-              umma::split2_f16(act ? umma::after_wait(orr[i2 * 16 + 2 * d2]) * inv_l : 0.f,
-                               act ? umma::after_wait(orr[i2 * 16 + 2 * d2 + 1]) * inv_l : 0.f, hw[i2 * 8 + d2], lw[i2 * 8 + d2]);
-          }
-          umma::st16s<1>(tl + TC_COL_Q + 8 * (4 * grp + 2 * kh), hw);
-          umma::st16s<1>(tl + TC_COL_Q + 64 + 8 * (4 * grp + 2 * kh), lw);
+          store_o_operand(tl, grp, kh, la, lb, act);
           umma::wait_st();
           umma::fence_before_sync();
         }
@@ -777,16 +584,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
         if (tid == 0) {
           // scores = O E'^T (the reference's single-head matmul(mh_atten_out, single_head_key), Wo folded into E')
           umma::fence_after_sync();
-          const uint32_t d = tm + TC_COL_S;
-#pragma unroll
-          for (int ks = 0; ks < 8; ++ks)
-            umma::mma_f16_ts(d, tm + TC_COL_Q + 64 + 8 * ks, umma::make_desc(opE + ks * 2 * lboN, lboN, 128), idescS, ks > 0);
-#pragma unroll
-          for (int ks = 0; ks < 8; ++ks)
-            umma::mma_f16_ts(d, tm + TC_COL_Q + 8 * ks, umma::make_desc(opE + half + ks * 2 * lboN, lboN, 128), idescS, true);
-#pragma unroll
-          for (int ks = 0; ks < 8; ++ks)
-            umma::mma_f16_ts(d, tm + TC_COL_Q + 8 * ks, umma::make_desc(opE + ks * 2 * lboN, lboN, 128), idescS, true);
+          mma_split3(tm + TC_COL_S, tm + TC_COL_Q, tm + TC_COL_Q + 64, 8, opE, opE + half, 2 * lboN, lboN, idescS, 8, false);
           umma::commit(bar_sc);
         }
         PHASE_MARK(7);
@@ -953,14 +751,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
         live_after = !fin;
         if (wsub == 0) {
           if (t > 0) {
-            float sg;
-            if (A.t.unscaled) {
-              const float* ux = A.t.unscaled + (size_t)b * N1 * 2;
-              sg = rintf(seglen(ux[2 * cur0] - ux[2 * sl], ux[2 * cur0 + 1] - ux[2 * sl + 1]));
-            } else {
-              sg = seglen(sXY[2 * cur0] - sXY[2 * sl], sXY[2 * cur0 + 1] - sXY[2 * sl + 1]);
-            }
-            sTlen[rc] += sg;
+            sTlen[rc] += seg_cost(A.t, b, N1, sXY, cur0, sl);
           }
           if (!CVRP && t == 0) sFirst[rc] = sl;
           sCur[rc] = sl;
@@ -982,13 +773,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
       for (int r = tid; r < nrows; r += RT) {
         float len = sTlen[r];
         if (!CVRP) {
-          const int a = sCur[r], f = sFirst[r];
-          if (A.t.unscaled) {
-            const float* ux = A.t.unscaled + (size_t)b * N1 * 2;
-            len += rintf(seglen(ux[2 * a] - ux[2 * f], ux[2 * a + 1] - ux[2 * f + 1]));
-          } else {
-            len += seglen(sXY[2 * a] - sXY[2 * f], sXY[2 * a + 1] - sXY[2 * f + 1]);
-          }
+          len += seg_cost(A.t, b, N1, sXY, sCur[r], sFirst[r]);
         }
         const size_t g = (size_t)b * A.M + row0 + r;
         A.reward[g] = -len;
@@ -1017,8 +802,6 @@ static int tc_maxe(const elg_model_desc* d) {
 // Largest row tile (multiple of 4, <= 112) whose layout fits the 227 KB of one SM; 0 = none
 int rollout_tc_max_rows(const elg_model_desc* d, int N1) {
   if (N1 > N_RES_MAX || tc_maxe(d) == 0) return 0;
-  const int K1 = d->local_k + (d->problem == ELG_CVRP ? 1 : 0);
-  (void)K1;
   return TC_MT_MAX;
 }
 
@@ -1036,7 +819,6 @@ int rollout_tc_tiles(const elg_model_desc* d, int B, int M, int N1, int* mt_out)
   int mt = (((M + tiles - 1) / tiles) + 3) & ~3;
   if (mt > cap) { mt = cap; tiles = (M + mt - 1) / mt; }
   if (mt_out) *mt_out = mt;
-  (void)B;
   return tiles;
 }
 
@@ -1048,9 +830,7 @@ int launch_rollout_tc(const elg_model_desc* d, RolloutArgs& a, cudaStream_t st) 
   a.tiles = tiles;
   a.MT = mt;
   const int maxe = tc_maxe(d);
-  const int K1 = d->local_k + (d->problem == ELG_CVRP ? 1 : 0);
   const size_t smem = (size_t)(maxe == 4 ? TcL<32>::total : TcL<48>::total) * sizeof(float);
-  (void)K1;
   int dev = 0, sms = 148;
   ELG_CUDA_OK(cudaGetDevice(&dev));
   ELG_CUDA_OK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
