@@ -73,6 +73,22 @@ struct TcL {
 };
 static_assert(TcL<48>::total * 4 <= 227 * 1024 && TcL<32>::total * 4 <= 227 * 1024, "layout exceeds one SM's shared memory");
 
+#ifdef ELG_PHASE_TIMING
+// The softmax rounds split per group: each group's leader accumulates five sub-phases of its own rounds and counts them
+// (slot 5), so the two groups' waits can be told apart from their arithmetic (tools/phase_timing.py)
+static __device__ unsigned long long g_sm_clk[2][8];
+__device__ __forceinline__ unsigned int sm_clock() {
+  unsigned int c;
+  asm volatile("mov.u32 %0, %%clock;" : "=r"(c)::"memory");
+  return c;
+}
+#define SM_T0() unsigned int sclk_ = sm_clock()
+#define SM_MARK(i) do { if (leader) { const unsigned int n_ = sm_clock(); smclk[i] += n_ - sclk_; sclk_ = n_; } } while (0)
+#else
+#define SM_T0()
+#define SM_MARK(i)
+#endif
+
 // =================================================================================================
 // NP = 112: the node count rounded up to 16 is known at compile time (the 100-node benchmark shapes); NP = 0: run time
 template <int PROBLEM, int MAXE, int NP>
@@ -112,7 +128,10 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
   uint64_t* bar_loc = bar + 4;                                    // tcgen05.commit of the local-policy MMAs
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bar + 5);
 
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  // the warp index through a shuffle: the compiler then knows it is warp-uniform and keeps everything derived from it
+  // (softmax group, TMEM addresses, MMA operands) in uniform registers, so the leader issues each tcgen05.mma without
+  // first moving its operands into uniform registers (R2UR) on the chain of every decode step
+  const int tid = threadIdx.x, warp = __shfl_sync(FULL, tid >> 5, 0), lane = tid & 31;
   const int q = warp & 3, wsub = warp >> 2, grp = wsub >> 1, kh = wsub & 1;     // softmax group (heads 4*grp..), key half
   uint64_t* bar_grp = bar + 2 + grp;                              // tcgen05.commit of this softmax group's MMAs
   const int row = q * 32 + lane;                   // TMEM lane = row of the tile
@@ -159,6 +178,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
   const bool leader = tid == grp * 256;                           // issues this group's MMAs
 #ifdef ELG_PHASE_TIMING
   unsigned long long pclk[16] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+  unsigned int smclk[6] = {0, 0, 0, 0, 0, 0};
 #endif
 
   for (int iter = 0;; ++iter) {
@@ -498,10 +518,12 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
         }
         float lt0 = 0.f, lt1 = 0.f, lt2 = 0.f, lt3 = 0.f;       // softmax denominators of heads 4*grp + rho
 
+        SM_T0();
 #pragma unroll 1
         for (int rho = 0; rho < 4; ++rho) {
           mbar_wait(bar_grp, (step_par + rho) & 1u);
           umma::fence_after_sync();
+          SM_MARK(0);
           const uint32_t sb = tl + TC_COL_S + grp * N1p;
           uint32_t sr[56];
           // KH = 8..56 columns in at most three loads (32 + 16 + 8, register i <-> column i); columns past KH that the
@@ -528,9 +550,11 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
           // the row's maximum over both key halves first (shared memory + 64-thread barrier): both halves then use the same
           // offset, no rescaling of the weights; the two partial denominators meet at the normalisation of O
           sXm[wsub * 128 + row] = mloc;
+          SM_MARK(1);
           pair_sync(1 + grp * 4 + q);
           const float mm = fmaxf(mloc, sXm[(wsub ^ 1) * 128 + row]);
           const float moff = mm == -INFINITY ? 0.f : mm - TC_P_SCALE_LOG2;
+          SM_MARK(2);
           float lloc = 0.f;
           // P (fp16 hi/lo, two keys per 32-bit column) in place of S: hi at [sb, sb + N1p/2), lo behind it
 #pragma unroll
@@ -552,6 +576,7 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
           umma::st_words<2>(sb + (N1p >> 1) + kh * (KH >> 1), sr + 1, KH >> 1);
           umma::wait_st();
           umma::fence_before_sync();
+          SM_MARK(3);
           // round 0 is CTA-wide: the first P V overwrites accumulator columns that held [pem | z], which the other
           // group's threads may still be reading in (6)
           if (rho == 0) __syncthreads(); else group_sync(9 + grp);
@@ -561,6 +586,10 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
             if (rho < 3) issue_qk(4 * grp + rho + 1);
             umma::commit(bar_grp);
           }
+          SM_MARK(4);
+#ifdef ELG_PHASE_TIMING
+          smclk[5] += 1;
+#endif
           PHASE_MARK(6);
 
         }
@@ -789,6 +818,8 @@ __global__ void __launch_bounds__(RT, 1) rollout_tc_kernel(const RolloutArgs A) 
 #ifdef ELG_PHASE_TIMING
   if (tid == 0)
     for (int i = 0; i < 16; ++i) atomicAdd(&g_phase_clk[i], pclk[i]);
+  if (leader)
+    for (int i = 0; i < 6; ++i) atomicAdd(&g_sm_clk[grp][i], (unsigned long long)smclk[i]);
 #endif
 }
 
@@ -860,9 +891,15 @@ int launch_rollout_tc(const elg_model_desc* d, RolloutArgs& a, cudaStream_t st) 
 }  // namespace elg
 
 #ifdef ELG_PHASE_TIMING
-extern "C" int elg_debug_phase_clocks_tc(unsigned long long* out16, int reset) {
-  ELG_CUDA_OK(cudaMemcpyFromSymbol(out16, elg::g_phase_clk, sizeof(unsigned long long) * 16));
-  if (reset) { unsigned long long z[16] = {0}; ELG_CUDA_OK(cudaMemcpyToSymbol(elg::g_phase_clk, z, sizeof(z))); }
+// out32: [0, 16) the phases of a decode step (thread 0), [16, 32) the softmax rounds of group 0 and group 1 (8 each)
+extern "C" int elg_debug_phase_clocks_tc(unsigned long long* out32, int reset) {
+  ELG_CUDA_OK(cudaMemcpyFromSymbol(out32, elg::g_phase_clk, sizeof(unsigned long long) * 16));
+  ELG_CUDA_OK(cudaMemcpyFromSymbol(out32 + 16, elg::g_sm_clk, sizeof(unsigned long long) * 16));
+  if (reset) {
+    unsigned long long z[16] = {0};
+    ELG_CUDA_OK(cudaMemcpyToSymbol(elg::g_phase_clk, z, sizeof(z)));
+    ELG_CUDA_OK(cudaMemcpyToSymbol(elg::g_sm_clk, z, sizeof(z)));
+  }
   return ELG_OK;
 }
 #endif
